@@ -225,6 +225,18 @@ def workload_config(args, method):
     return cfg
 
 
+def dump_outputs(path, table, field, n_local):
+    """Writes what the last timed step computed as <path>/<name>.npy: `table` (float64), the result table the timed call
+    returns (one row per solve, columns COLS of efficiency_map / time_series), and `psi` (float64), the solution fields
+    of a fixed, seeded sample of at most 16 of this process's solves (1 MiB each on the bench grid), with their row
+    numbers in `psi_solves`.  The inputs depend on the arguments only, so two builds can be compared file by file."""
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "table.npy"), np.asarray(table, np.float64))
+    pick = np.sort(np.random.default_rng(0).choice(n_local, size=min(16, n_local), replace=False))
+    np.save(os.path.join(path, "psi_solves.npy"), pick.astype(np.float64))
+    np.save(os.path.join(path, "psi.npy"), np.ascontiguousarray(field("psi")[pick], np.float64))
+
+
 KERNEL_NAMES = {1: "sweep_direct_kernel (v1)", 2: "sweep_tma_kernel (v2)", 3: "solve_resident_kernel (v3)",
                 4: "sweep_tb_kernel (v4, temporal blocking)", 5: "sweep_line_kernel (v5, block-line relaxation, TMA loads + TMA stores)"}
 
@@ -313,6 +325,8 @@ def run_ours(args):
     probe_ms = m.probe_ms() if series else None
     tab = loc if isinstance(loc, np.ndarray) else loc.cpu().numpy()
     clocks = sampler.finish() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out if isinstance(out, np.ndarray) else out.cpu().numpy(), m.field, nloc)
     ms_per_step = ms_total / args.steps
     value = total / (ms_per_step * 1e-3)
     # every rank's solves must have converged (err 0) or stopped on their round-off floor (err 4); sweep range over all ranks
@@ -498,6 +512,8 @@ def main():
     ap.add_argument("--lfl-sweeps", type=int, default=300, help="GPU STRICT Jacobi sweeps timed for like_for_like")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-streaming", action="store_true", help="skip the extra one-level pass that reports the streaming kernel's roofline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's result table and a sample of its solution fields as DIR/<name>.npy")
     args = ap.parse_args()
     if args.method is None:
         args.method = "line2_chebyshev"

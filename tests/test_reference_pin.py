@@ -18,9 +18,9 @@ def test_pin_kit_is_in_place():
 
 def test_oracle_is_pinned_against_the_compiled_reference():
     fc = next((c for c in ("gfortran", "flang", "nvfortran") if shutil.which(c)), None)
-    ref = os.environ.get("REF", "/root/reference")
-    if fc is None or not os.path.exists(os.path.join(ref, "src", "diagnose", "main.f90")):
-        pytest.skip("PARITY UNPINNED: no Fortran compiler (gfortran/flang/nvfortran) or no reference sources here - "
+    ref = os.environ.get("REF")
+    if fc is None or not ref or not os.path.exists(os.path.join(ref, "src", "diagnose", "main.f90")):
+        pytest.skip("PARITY UNPINNED: needs a Fortran compiler (gfortran/flang/nvfortran) and REF=<XLab-EE-fortran checkout> - "
                     "run scripts/pin_against_reference.sh on a machine that has both")
     r = subprocess.run([SCRIPT], capture_output=True, text=True, timeout=3600)
     assert r.returncode == 0, r.stdout + r.stderr
