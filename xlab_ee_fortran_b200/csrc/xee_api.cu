@@ -52,22 +52,14 @@ int xee_plan_apply_dev(xee_plan* p, const void* psi, void* out, void* stream) {
   DeviceGuard g(p->impl->d.device);
   return p->impl->apply(psi, out, (cudaStream_t)stream);
 }
-int xee_sweep_kernel_stats(xee_plan* p, double* ms, long long* launches, int reset) {
-  if (ms) *ms = p->impl->sweep_ms;
-  if (launches) *launches = p->impl->sweep_launches;
-  if (reset) { p->impl->sweep_ms = 0; p->impl->sweep_launches = 0; p->impl->kernel_launches = 0; }
-  return 0;
-}
+int xee_sweep_kernel_stats(xee_plan* p, double* ms, long long* launches, int reset) { return p->impl->kernel_stats(ms, launches, reset); }
 int xee_plan_cheb_params(xee_plan* p, double* rho, double* gamma) {
   if (rho) *rho = p->impl->cheb_rho_used;
   if (gamma) *gamma = p->impl->cheb_gamma_used;
   return 0;
 }
 int xee_plan_kernel_info(xee_plan* p, int* variant, int* sweeps_per_pass, long long* kernel_launches) {
-  if (variant) *variant = p->impl->variant_used;
-  if (sweeps_per_pass) *sweeps_per_pass = p->impl->depth_used;
-  if (kernel_launches) *kernel_launches = p->impl->kernel_launches;
-  return 0;
+  return p->impl->kernel_info(variant, sweeps_per_pass, kernel_launches);
 }
 
 }  // extern "C"

@@ -191,11 +191,8 @@ struct xee_map { MapBase* impl; };
 
 extern "C" {
 int xee_map_create(const xee_map_desc* desc, const float* A, const float* B, const float* C, xee_map** out) {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("xee: no CUDA device available - this library has no CPU fallback");
-  int dev = desc->device;
-  if (dev < 0) XEE_CHECK(cudaGetDevice(&dev));
-  if (dev >= ndev) return fail("xee: device index out of range");
+  int dev = 0;
+  if (resolve_device(desc->device, &dev)) return 1;
   DeviceGuard guard(dev);
   if (desc->nr < 4 || desc->nz < 4 || desc->nheat < 1) return fail("xee_map: nr, nz >= 4 and nheat >= 1 required");
   MapBase* m = nullptr; int rc;
@@ -216,18 +213,8 @@ int xee_map_run_dev(xee_map* m, const double* heat_dev, const xee_solve_params* 
   return m->impl->run(heat_dev, false, prm, table_dev, false, (cudaStream_t)stream);
 }
 int xee_map_get_field(xee_map* m, int which, void* host_out) { DeviceGuard g(m->impl->device()); return m->impl->get_field(which, host_out); }
-int xee_map_sweep_kernel_stats(xee_map* m, double* ms, long long* launches, int reset) {
-  PlanBase* p = m->impl->plan();
-  if (ms) *ms = p->sweep_ms;
-  if (launches) *launches = p->sweep_launches;
-  if (reset) { p->sweep_ms = 0; p->sweep_launches = 0; p->kernel_launches = 0; }
-  return 0;
-}
+int xee_map_sweep_kernel_stats(xee_map* m, double* ms, long long* launches, int reset) { return m->impl->plan()->kernel_stats(ms, launches, reset); }
 int xee_map_kernel_info(xee_map* m, int* variant, int* sweeps_per_pass, long long* kernel_launches) {
-  PlanBase* p = m->impl->plan();
-  if (variant) *variant = p->variant_used;
-  if (sweeps_per_pass) *sweeps_per_pass = p->depth_used;
-  if (kernel_launches) *kernel_launches = p->kernel_launches;
-  return 0;
+  return m->impl->plan()->kernel_info(variant, sweeps_per_pass, kernel_launches);
 }
 }  // extern "C"

@@ -10,6 +10,7 @@
 #include <map>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "xee_kernels.cuh"
@@ -73,6 +74,28 @@ struct DeviceGuard {
 inline int env_int(const char* name, int dflt) {
   const char* v = getenv(name);
   return v && *v ? atoi(v) : dflt;
+}
+
+// Runtime flags to compile-time ones: calls f(std::bool_constant<b0>{}, std::bool_constant<b1>{}, ...), so that a launch
+// site spells its kernel's template arguments once and instantiates one kernel per combination of the flags it passes.
+template <class F> int dispatch(F&& f) { return f(); }
+template <class F, class... B> int dispatch(F&& f, bool b, B... rest) {
+  if (b) return dispatch([&](auto... c) { return f(std::true_type{}, c...); }, rest...);
+  return dispatch([&](auto... c) { return f(std::false_type{}, c...); }, rest...);
+}
+constexpr int arith_of(bool strict) { return strict ? XEE_ARITH_STRICT : XEE_ARITH_FAST; }
+constexpr int mode_of(bool cheb) { return cheb ? MODE_CHEBYSHEV : MODE_JACOBI; }
+
+// The device of a new plan, map or series: `want`, or the current device when want < 0, resolved so that later entry
+// points can return to it.
+inline int resolve_device(int want, int* dev) {
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+    return fail("xee: no CUDA device available - this library has no CPU fallback");
+  *dev = want;
+  if (*dev < 0) XEE_CHECK(cudaGetDevice(dev));
+  if (*dev >= ndev) return fail("xee: device index out of range");
+  return 0;
 }
 
 // Caching device allocator for the large field buffers: cudaFree of GiB-sized blocks costs tens of ms
@@ -157,6 +180,19 @@ struct PlanBase {
   double norm_floor = 0.0;
   int rho_subsample = 0;   // > 1 (one operator per solve): probe every rho_subsample-th operator set only and interpolate the
                            // spectral data in between - for series whose operators vary smoothly with the index (set by the caller)
+  // the *_sweep_kernel_stats and *_kernel_info entry points of plans, maps and series
+  int kernel_stats(double* ms, long long* launches, int reset) {
+    if (ms) *ms = sweep_ms;
+    if (launches) *launches = sweep_launches;
+    if (reset) { sweep_ms = 0; sweep_launches = 0; kernel_launches = 0; }
+    return 0;
+  }
+  int kernel_info(int* variant, int* sweeps_per_pass, long long* launches) const {
+    if (variant) *variant = variant_used;
+    if (sweeps_per_pass) *sweeps_per_pass = depth_used;
+    if (launches) *launches = kernel_launches;
+    return 0;
+  }
 };
 
 template <class T>
@@ -198,7 +234,7 @@ struct Plan : PlanBase {
   // two-level block-line methods (XEE_METHOD_LINE2_*, xee_twolevel.cuh): coarse-grid data of the operator and of a batch
   bool use_two = false;
   tl::Dims tld{};
-  double *tl_ainv = nullptr, *tl_tmp = nullptr;   // [ncp][ncp]: Ac^-1 (and the second Gauss-Jordan buffer)
+  double *tl_ainv = nullptr, *tl_tmp = nullptr;   // [ncp][ncp]: Ac^-1, and Ac for the band factorisation
   double *tl_part = nullptr;                      // [nbatch][ntiles][32] per-tile restriction of the residual
   double *tl_band = nullptr;                      // [nsets][2][nc][ncx + 2] band LU factors of the coarse operators
   double *tl_scale = nullptr;                     // [nbatch] per-solve factor of the coarse correction (one operator per solve)
@@ -244,7 +280,7 @@ struct Plan : PlanBase {
     // Keep the operator in registers across `spb` solves, but leave >= ~4 waves of blocks on 148 SMs.
     spb = 1;
     if (d.shared_coe) {
-      spb = env_int("XEE_SPB", 8);
+      spb = 8;
       while (spb > 1 && (long long)ntiles * ((d.nbatch + spb - 1) / spb) < 148LL * 8 * 4) spb /= 2;
     }
     gz = (d.nbatch + spb - 1) / spb;
@@ -262,21 +298,12 @@ struct Plan : PlanBase {
       tma_tiles_x = (d.nx - 2 + tma::TW - 1) / tma::TW;
       tma_tiles_y = (d.ny - 2 + tma::TH - 1) / tma::TH;
       const int nt = tma_tiles_x * tma_tiles_y;
-      // chunk = solves per work unit (operator registers reused across them).  Pick the chunk in [4,32] that
-      // minimises the makespan of the static round-robin over the persistent CTAs.
-      const int grid_cap = num_sms;
-      long long best = -1; tma_chunk = 1;
-      for (int ch = std::min(32, d.nbatch); ch >= std::min(4, d.nbatch); --ch) {
-        const int nch = (d.nbatch + ch - 1) / ch;
-        const long long units = (long long)nt * nch;
-        const int g = (int)std::min<long long>(grid_cap, units);
-        const long long makespan = ((units + g - 1) / g) * ch + 2;   // +2: operator reload per unit
-        if (best < 0 || makespan < best) { best = makespan; tma_chunk = ch; }
-      }
+      // operator registers reused across the solves of a unit; +2: operator reload per unit
+      tma_chunk = pick_chunk(nt, std::min(4, d.nbatch), std::min(32, d.nbatch), [](long long rounds, int ch) { return rounds * ch + 2; });
       tma_nchunks = (d.nbatch + tma_chunk - 1) / tma_chunk;
-      tma_grid = (int)std::min<long long>(grid_cap, (long long)nt * tma_nchunks);
-      tma_nstage = std::max(2, std::min(env_int("XEE_TMA_STAGES", 6), tma::NSTAGE_MAX));
-      if (!d.shared_coe) tma_nstage = 2;   // the operator tiles travel with every stage: 2 x ~110 KB (fp64)
+      tma_grid = (int)std::min<long long>(num_sms, (long long)nt * tma_nchunks);
+      static_assert(tma::NSTAGE_MAX >= 6, "six pipeline stages for a shared operator");
+      tma_nstage = d.shared_coe ? 6 : 2;   // one operator per solve: its tiles travel with every stage, 2 x ~110 KB (fp64)
       if (nt > ntiles) return fail("xee: internal: partial buffer too small for the TMA tiling");
     }
     // v5: segment-line relaxation is a METHOD, not a variant of the reference iteration: explicit request only.
@@ -290,21 +317,11 @@ struct Plan : PlanBase {
       use_tma = false;
       ln_tiles_x = (d.nx + ln::TW - 1) / ln::TW; ln_tiles_y = (d.ny + ln::TH - 1) / ln::TH;
       const int nt = ln_tiles_x * ln_tiles_y;
-      long long best = -1; ln_chunk = 1;
-      const int chmax = d.shared_coe ? std::min(env_int("XEE_LINE_CHUNK", 32), d.nbatch) : 1, chmin = std::min(4, chmax);
-      for (int ch = chmax; ch >= chmin; --ch) {
-        const int nch = (d.nbatch + ch - 1) / ch;
-        const long long units = (long long)nt * nch;
-        const int g = (int)std::min<long long>(num_sms, units);
-        const long long makespan = ((units + g - 1) / g) * (ch + 1);
-        if (best < 0 || makespan < best) { best = makespan; ln_chunk = ch; }
-      }
+      const int chmax = d.shared_coe ? std::min(32, d.nbatch) : 1;
+      ln_chunk = pick_chunk(nt, std::min(4, chmax), chmax, [](long long rounds, int ch) { return rounds * (ch + 1); });
       ln_nchunks = (d.nbatch + ln_chunk - 1) / ln_chunk;
-      ln_tstore = d.nx % ln::TW == 0 && env_int("XEE_LINE_TSTORE", 1) != 0;
-      if (nt > ntiles) {
-        pool_free(partial); partial = nullptr;
-        XEE_CHECK(pool_alloc(&partial, sizeof(double) * (size_t)nt * nb));
-      }
+      ln_tstore = d.nx % ln::TW == 0;
+      if (grow_partial(nt)) return 1;
       XEE_CHECK(pool_alloc(&linefac, sizeof(T) * kLineFacPlanes * nn * nsets));
       XEE_CHECK(pool_alloc(&linepack, (size_t)nt * line_pack_tile_bytes<T>() * nsets));
       want = 5;
@@ -339,22 +356,12 @@ struct Plan : PlanBase {
       tb_tiles_x = d.nx <= tb::W ? 1 : (d.nx - tb::W + sx - 1) / sx + 1;
       tb_tiles_y = d.ny <= tb::H ? 1 : (d.ny - tb::H + sy - 1) / sy + 1;
       const int nt = tb_tiles_x * tb_tiles_y;
-      // chunk = solves per work unit: the operator registers are reloaded (from L2) once per unit, worth ~2 solves
-      long long best = -1; tb_chunk = 1;
-      const int chmax = std::min(env_int("XEE_TB_CHUNK", 64), d.nbatch), chmin = std::min(8, chmax);
-      for (int ch = chmax; ch >= chmin; --ch) {
-        const int nch = (d.nbatch + ch - 1) / ch;
-        const long long units = (long long)nt * nch;
-        const int g = (int)std::min<long long>(num_sms, units);
-        const long long makespan = ((units + g - 1) / g) * (ch + 2);
-        if (best < 0 || makespan < best) { best = makespan; tb_chunk = ch; }
-      }
+      // the operator registers are reloaded (from L2) once per unit, worth ~2 solves
+      const int chmax = std::min(64, d.nbatch);
+      tb_chunk = pick_chunk(nt, std::min(8, chmax), chmax, [](long long rounds, int ch) { return rounds * (ch + 2); });
       tb_nchunks = (d.nbatch + tb_chunk - 1) / tb_chunk;
       tb_grid = (int)std::min<long long>(num_sms, (long long)nt * tb_nchunks);
-      if (nt > ntiles) {   // the residual partials are per (solve, tile)
-        pool_free(partial); partial = nullptr;
-        XEE_CHECK(pool_alloc(&partial, sizeof(double) * (size_t)nt * nb));
-      }
+      if (grow_partial(nt)) return 1;
       XEE_CHECK(pool_alloc(&x2, sizeof(T) * nn * d.nbatch));
       XEE_CHECK(pool_alloc(&x3, sizeof(T) * nn * d.nbatch));
     }
@@ -362,9 +369,33 @@ struct Plan : PlanBase {
   }
   int sweep_ntiles() const { return use_line ? ln_tiles_x * ln_tiles_y : use_tma ? tma_tiles_x * tma_tiles_y : ntiles; }
   int tb_ntiles() const { return tb_tiles_x * tb_tiles_y; }
+  int check_ntiles() const { return use_tb ? tb_ntiles() : sweep_ntiles(); }   // residual partials per solve
 
-  // cuTensorMapEncodeTiled through the runtime (no link-time dependency on libcuda).
-  static int encode_map(CUtensorMap* m, const void* base, int nx, int ny, int nb, int box_w, int box_h) {
+  // Solves per work unit of a persistent kernel: the chunk in [chmin, chmax] that minimises the makespan
+  // cost(rounds, chunk) of the static round-robin of the units over at most num_sms CTAs (ties: the largest chunk).
+  template <class Cost>
+  int pick_chunk(int nt, int chmin, int chmax, Cost cost) const {
+    long long best = -1; int chunk = 1;
+    for (int ch = chmax; ch >= chmin; --ch) {
+      const long long units = (long long)nt * ((d.nbatch + ch - 1) / ch);
+      const long long g = std::min<long long>(num_sms, units);
+      const long long makespan = cost((units + g - 1) / g, ch);
+      if (best < 0 || makespan < best) { best = makespan; chunk = ch; }
+    }
+    return chunk;
+  }
+  // the residual partials are per (solve, tile): room for a tiling with more tiles than the direct kernel's
+  int grow_partial(int nt) {
+    if (nt <= ntiles) return 0;
+    pool_free(partial); partial = nullptr;
+    XEE_CHECK(pool_alloc(&partial, sizeof(double) * (size_t)nt * d.nbatch));
+    return 0;
+  }
+
+  // cuTensorMapEncodeTiled through the runtime (no link-time dependency on libcuda): elements of type T, no interleave, no
+  // swizzle, 128-byte L2 promotion, no out-of-bounds fill.  dims and box have `rank` entries, byte_strides rank - 1.
+  static int encode_tiled(CUtensorMap* m, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* byte_strides,
+                          const cuuint32_t* box) {
     typedef CUresult (*Fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                            const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                            CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -375,15 +406,19 @@ struct Plan : PlanBase {
       if (!p) return fail("xee: cuTensorMapEncodeTiled not available from the driver");
       fn = (Fn)p;
     }
+    const cuuint32_t es[4] = {1, 1, 1, 1};
+    const CUresult r = fn(m, sizeof(T) == 8 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, rank,
+                          const_cast<void*>(base), dims, byte_strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { char b[128]; snprintf(b, sizeof b, "xee: cuTensorMapEncodeTiled (rank %d) failed (%d)", rank, (int)r); return fail(b); }
+    return 0;
+  }
+  // a batch of nb fields [nb][ny][nx] in boxes of box_w x box_h
+  static int encode_map(CUtensorMap* m, const void* base, int nx, int ny, int nb, int box_w, int box_h) {
     const cuuint64_t dims[3] = {(cuuint64_t)nx, (cuuint64_t)ny, (cuuint64_t)nb};
     const cuuint64_t strides[2] = {(cuuint64_t)nx * sizeof(T), (cuuint64_t)nx * ny * sizeof(T)};
     const cuuint32_t box[3] = {(cuuint32_t)box_w, (cuuint32_t)box_h, 1};
-    const cuuint32_t es[3] = {1, 1, 1};
-    const CUresult r = fn(m, sizeof(T) == 8 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3,
-                          const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { char b[128]; snprintf(b, sizeof b, "xee: cuTensorMapEncodeTiled failed (%d)", (int)r); return fail(b); }
-    return 0;
+    return encode_tiled(m, base, 3, dims, strides, box);
   }
   // (Re)build the tensor maps when the buffers of this call differ from the cached ones.
   int prepare_maps(const T* x0, const T* x1buf, const T* f, int nb) {
@@ -396,46 +431,13 @@ struct Plan : PlanBase {
         encode_map(&map_f, f, d.nx, d.ny, nb, hw, tma::TH))
       return 1;
     map_ptrs[0] = x0; map_ptrs[1] = x1buf; map_ptrs[2] = f;
-    if (!d.shared_coe && !map_coe_ready) {
-      if (encode_map4(&map_coe, coe, d.nx, d.ny, kPlanes, nsets, hw, tma::TH, kPlanes)) return 1;
+    if (!d.shared_coe && !map_coe_ready) {   // the operator planes of every set, kPlanes of them per box
+      const cuuint64_t dims[4] = {(cuuint64_t)d.nx, (cuuint64_t)d.ny, (cuuint64_t)kPlanes, (cuuint64_t)nsets};
+      const cuuint64_t strides[3] = {(cuuint64_t)d.nx * sizeof(T), (cuuint64_t)nn * sizeof(T), (cuuint64_t)nn * kPlanes * sizeof(T)};
+      const cuuint32_t box[4] = {(cuuint32_t)hw, (cuuint32_t)tma::TH, (cuuint32_t)kPlanes, 1};
+      if (encode_tiled(&map_coe, coe, 4, dims, strides, box)) return 1;
       map_coe_ready = true;
     }
-    return 0;
-  }
-  static int encode_map4(CUtensorMap* m, const void* base, int nx, int ny, int np, int ns, int box_w, int box_h, int box_p) {
-    typedef CUresult (*Fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                           const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                           CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    void* p = nullptr; cudaDriverEntryPointQueryResult q;
-    XEE_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q));
-    if (!p) return fail("xee: cuTensorMapEncodeTiled not available from the driver");
-    const cuuint64_t dims[4] = {(cuuint64_t)nx, (cuuint64_t)ny, (cuuint64_t)np, (cuuint64_t)ns};
-    const cuuint64_t strides[3] = {(cuuint64_t)nx * sizeof(T), (cuuint64_t)nx * ny * sizeof(T), (cuuint64_t)nx * ny * np * sizeof(T)};
-    const cuuint32_t box[4] = {(cuuint32_t)box_w, (cuuint32_t)box_h, (cuuint32_t)box_p, 1};
-    const cuuint32_t es[4] = {1, 1, 1, 1};
-    const CUresult r = ((Fn)p)(m, sizeof(T) == 8 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4,
-                               const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { char b[128]; snprintf(b, sizeof b, "xee: cuTensorMapEncodeTiled(4D) failed (%d)", (int)r); return fail(b); }
-    return 0;
-  }
-  // 4-D view of a field batch for the TMA stores of the v5 kernel: (column within a TW-wide tile column, tile column, row,
-  // solve).  A [TH][FW] staging box stored at column 0 loses its FW - TW pad columns as out-of-bounds elements.
-  int encode_map_out(CUtensorMap* m, const void* base, int nb) {
-    typedef CUresult (*Fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                           const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                           CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    void* p = nullptr; cudaDriverEntryPointQueryResult q;
-    XEE_CHECK(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q));
-    if (!p) return fail("xee: cuTensorMapEncodeTiled not available from the driver");
-    const cuuint64_t dims[4] = {(cuuint64_t)ln::TW, (cuuint64_t)(d.nx / ln::TW), (cuuint64_t)d.ny, (cuuint64_t)nb};
-    const cuuint64_t strides[3] = {(cuuint64_t)ln::TW * sizeof(T), (cuuint64_t)d.nx * sizeof(T), (cuuint64_t)d.nx * d.ny * sizeof(T)};
-    const cuuint32_t box[4] = {(cuuint32_t)ln::Cfg<T>::FW, 1, (cuuint32_t)ln::TH, 1};
-    const cuuint32_t es[4] = {1, 1, 1, 1};
-    const CUresult r = ((Fn)p)(m, sizeof(T) == 8 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4,
-                               const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { char b[128]; snprintf(b, sizeof b, "xee: cuTensorMapEncodeTiled(store view) failed (%d)", (int)r); return fail(b); }
     return 0;
   }
   ~Plan() override {
@@ -497,8 +499,7 @@ struct Plan : PlanBase {
     linefac_ready = true;
     return use_two ? two_setup() : 0;
   }
-  // Two-level methods, once per operator: Galerkin coarse operator Ac = P^T L P and its inverse (Gauss-Jordan on the device,
-  // one launch per pivot between two buffers).
+  // Two-level methods, once per operator: Galerkin coarse operator Ac = P^T L P and its inverse (band LU on the device).
   int two_setup() {
     TraceTimer tt("two-level setup");
     const int nc = tld.nc, ncp = tld.ncp;
@@ -561,9 +562,8 @@ struct Plan : PlanBase {
     return 0;
   }
   // c = 0 for both iterates: the stored fields ARE the iterates (start of a solve / of a probe)
-  int two_reset(int nb, cudaStream_t s) {
+  int two_reset(cudaStream_t s) {
     XEE_CHECK(cudaMemsetAsync(tl_cv, 0, sizeof(double) * 2 * (size_t)d.nbatch * tld.pz * tld.px, s));
-    (void)nb;
     return 0;
   }
   // psi = y + P c made explicit in both buffers (b0 owns slot 0, b1 slot 1), then c = 0: the same state, stored plainly
@@ -573,7 +573,7 @@ struct Plan : PlanBase {
     XEE_LAUNCH_OK();
     tl::prolong_add_kernel<T><<<g, 256, 0, s>>>(b1, two_cv(1, nb), nullptr, d.nx, d.ny, tld.px, tld.pz * tld.px);
     XEE_LAUNCH_OK();
-    return two_reset(nb, s);
+    return two_reset(s);
   }
   int coe_to_aos_host(void* coe_host) override {  // set 0 only (Fortran-facing cal_coe)
     T* tmp = nullptr;
@@ -604,12 +604,6 @@ struct Plan : PlanBase {
     return a;
   }
 
-  template <int ARITH, int MODE>
-  void launch_mode(const SweepArgs<T>& a, bool check, cudaStream_t s) {
-    dim3 blk(kDirBX, kDirBY), g(gx, gy, gz);
-    if (check) sweep_direct_kernel<T, ARITH, MODE, true><<<g, blk, 0, s>>>(a);
-    else sweep_direct_kernel<T, ARITH, MODE, false><<<g, blk, 0, s>>>(a);
-  }
   template <int ARITH, int MODE, bool CHECK, bool PERSOLVE>
   int launch_tma_inst(const TmaSweepArgs<T>& P, const CUtensorMap& ms, const CUtensorMap& mp, cudaStream_t s) {
     constexpr int coe_off = tma::Cfg<T>::PSI_BYTES + tma::Cfg<T>::FLD_BYTES + (MODE == MODE_CHEBYSHEV ? tma::Cfg<T>::FLD_BYTES : 0);
@@ -620,21 +614,15 @@ struct Plan : PlanBase {
     sweep_tma_kernel<T, ARITH, MODE, CHECK, PERSOLVE><<<tma_grid, tma::NTHREADS, smem, s>>>(P, ms, mp, map_f, map_coe);
     return 0;
   }
-  template <int ARITH, int MODE>
-  int launch_tma_mode(const TmaSweepArgs<T>& P, const CUtensorMap& ms, const CUtensorMap& mp, bool check, cudaStream_t s) {
-    if (d.shared_coe) return check ? launch_tma_inst<ARITH, MODE, true, false>(P, ms, mp, s) : launch_tma_inst<ARITH, MODE, false, false>(P, ms, mp, s);
-    return check ? launch_tma_inst<ARITH, MODE, true, true>(P, ms, mp, s) : launch_tma_inst<ARITH, MODE, false, true>(P, ms, mp, s);
-  }
   int launch_sweep_tma(const SweepArgs<T>& a, int mode, bool check, cudaStream_t s) {
     TmaSweepArgs<T> P{};
     P.a = a; P.tiles_x = tma_tiles_x; P.tiles_y = tma_tiles_y; P.nchunks = tma_nchunks; P.chunk = tma_chunk; P.nstage = tma_nstage;
     const int si = (a.src == (const T*)map_ptrs[0]) ? 0 : 1;      // which ping-pong buffer is the source
     const CUtensorMap& ms = map_halo[si];
     const CUtensorMap& mp = map_plain[si ^ 1];
-    const bool strict = d.arith == XEE_ARITH_STRICT;
-    int rc;
-    if (mode == MODE_JACOBI) rc = strict ? launch_tma_mode<XEE_ARITH_STRICT, MODE_JACOBI>(P, ms, mp, check, s) : launch_tma_mode<XEE_ARITH_FAST, MODE_JACOBI>(P, ms, mp, check, s);
-    else rc = strict ? launch_tma_mode<XEE_ARITH_STRICT, MODE_CHEBYSHEV>(P, ms, mp, check, s) : launch_tma_mode<XEE_ARITH_FAST, MODE_CHEBYSHEV>(P, ms, mp, check, s);
+    const int rc = dispatch([&](auto strict, auto cheb, auto chk, auto persolve) {
+      return launch_tma_inst<arith_of(strict), mode_of(cheb), chk, persolve>(P, ms, mp, s);
+    }, d.arith == XEE_ARITH_STRICT, mode == MODE_CHEBYSHEV, check, !d.shared_coe);
     if (rc) return rc;
     XEE_LAUNCH_OK();
     return 0;
@@ -645,23 +633,26 @@ struct Plan : PlanBase {
     if ((uintptr_t)ptr & 15) return fail("xee: TMA path needs 16-byte aligned field buffers");
     if (line_maps.size() >= 24) line_maps.erase(line_maps.begin());
     LineMap lm{ptr, nb, kind, {}};
-    if (kind == 0 ? encode_map(&lm.map, ptr, d.nx, d.ny, nb, ln::Cfg<T>::XW, ln::TH + 2)
-        : kind == 1 ? encode_map(&lm.map, ptr, d.nx, d.ny, nb, ln::Cfg<T>::FW, ln::TH) : encode_map_out(&lm.map, ptr, nb)) return 1;
+    if (kind < 2) {
+      if (encode_map(&lm.map, ptr, d.nx, d.ny, nb, kind == 0 ? ln::Cfg<T>::XW : ln::Cfg<T>::FW, kind == 0 ? ln::TH + 2 : ln::TH)) return 1;
+    } else {   // (column within a TW-wide tile column, tile column, row, solve): a [TH][FW] staging box stored at column 0
+               // loses its FW - TW pad columns as out-of-bounds elements
+      const cuuint64_t dims[4] = {(cuuint64_t)ln::TW, (cuuint64_t)(d.nx / ln::TW), (cuuint64_t)d.ny, (cuuint64_t)nb};
+      const cuuint64_t strides[3] = {(cuuint64_t)ln::TW * sizeof(T), (cuuint64_t)d.nx * sizeof(T), (cuuint64_t)d.nx * d.ny * sizeof(T)};
+      const cuuint32_t box[4] = {(cuuint32_t)ln::Cfg<T>::FW, 1, (cuuint32_t)ln::TH, 1};
+      if (encode_tiled(&lm.map, ptr, 4, dims, strides, box)) return 1;
+    }
     line_maps.push_back(lm);
     *out = lm.map;
     return 0;
   }
   template <bool CHEB, bool CHECK, bool TWO>
-  int launch_line_inst2(const LineArgs<T>& A, int grid, const CUtensorMap& mx, const CUtensorMap& mxm, const CUtensorMap& mf, const CUtensorMap& mo, cudaStream_t s) {
+  int launch_line_inst(const LineArgs<T>& A, int grid, const CUtensorMap& mx, const CUtensorMap& mxm, const CUtensorMap& mf, const CUtensorMap& mo, cudaStream_t s) {
     constexpr int smem = TWO ? ln::Cfg<T>::SMEM_BYTES_TWO : ln::Cfg<T>::SMEM_BYTES;
     static std::atomic<unsigned long long> attr_done{0};
     if (opt_in_smem(sweep_line_kernel<T, CHEB, CHECK, TWO>, smem, attr_done)) return 1;
     sweep_line_kernel<T, CHEB, CHECK, TWO><<<grid, ln::NT, smem, s>>>(A, mx, mxm, mf, mo, TWO ? map_cv : mf);
     return 0;
-  }
-  template <bool CHEB, bool CHECK>
-  int launch_line_inst(const LineArgs<T>& A, int grid, const CUtensorMap& mx, const CUtensorMap& mxm, const CUtensorMap& mf, const CUtensorMap& mo, cudaStream_t s) {
-    return use_two ? launch_line_inst2<CHEB, CHECK, true>(A, grid, mx, mxm, mf, mo, s) : launch_line_inst2<CHEB, CHECK, false>(A, grid, mx, mxm, mf, mo, s);
   }
   int launch_sweep_line(const SweepArgs<T>& a, int mode, bool check, cudaStream_t s) {
     if (!linefac_ready) return fail("xee: line relaxation: the operator has not been set");
@@ -682,9 +673,8 @@ struct Plan : PlanBase {
     A.cv_cur_z = a.two_slot * d.nbatch; A.cv_prev_z = (1 - a.two_slot) * d.nbatch;
     if (use_two && !tl_ready) return fail("xee: two-level method: the operator has not been set");
     const int grid = (int)std::min<long long>((long long)num_sms * ln::CTAS_PER_SM, (long long)ln_tiles_x * ln_tiles_y * A.nchunks);
-    int rc;
-    if (mode == MODE_CHEBYSHEV) rc = check ? launch_line_inst<true, true>(A, grid, cx, cxm, cf, co, s) : launch_line_inst<true, false>(A, grid, cx, cxm, cf, co, s);
-    else rc = check ? launch_line_inst<false, true>(A, grid, cx, cxm, cf, co, s) : launch_line_inst<false, false>(A, grid, cx, cxm, cf, co, s);
+    const int rc = dispatch([&](auto cheb, auto chk, auto two) { return launch_line_inst<cheb, chk, two>(A, grid, cx, cxm, cf, co, s); },
+                            mode == MODE_CHEBYSHEV, check, use_two);
     if (rc) return rc;
     XEE_LAUNCH_OK();
     if (use_two) {   // psi' = psi - alpha (z + P E) (Jacobi) / y - omega gamma P E (Chebyshev; omega from the per-launch value)
@@ -697,10 +687,11 @@ struct Plan : PlanBase {
     if (use_line && mode != MODE_APPLY) return launch_sweep_line(a, mode, check, s);
     if (use_tma && mode != MODE_APPLY && a.nbatch == d.nbatch && (a.src == map_ptrs[0] || a.src == map_ptrs[1]))
       return launch_sweep_tma(a, mode, check, s);
-    const bool strict = d.arith == XEE_ARITH_STRICT;
-    if (mode == MODE_JACOBI) strict ? launch_mode<XEE_ARITH_STRICT, MODE_JACOBI>(a, check, s) : launch_mode<XEE_ARITH_FAST, MODE_JACOBI>(a, check, s);
-    else if (mode == MODE_CHEBYSHEV) strict ? launch_mode<XEE_ARITH_STRICT, MODE_CHEBYSHEV>(a, check, s) : launch_mode<XEE_ARITH_FAST, MODE_CHEBYSHEV>(a, check, s);
-    else strict ? launch_mode<XEE_ARITH_STRICT, MODE_APPLY>(a, false, s) : launch_mode<XEE_ARITH_FAST, MODE_APPLY>(a, false, s);
+    const dim3 blk(kDirBX, kDirBY), g(gx, gy, gz);
+    dispatch([&](auto strict, auto cheb, auto apply, auto chk) {
+      sweep_direct_kernel<T, arith_of(strict), apply ? MODE_APPLY : mode_of(cheb), chk><<<g, blk, 0, s>>>(a);
+      return 0;
+    }, d.arith == XEE_ARITH_STRICT, mode == MODE_CHEBYSHEV, mode == MODE_APPLY, check);
     XEE_LAUNCH_OK();
     return 0;
   }
@@ -724,10 +715,6 @@ struct Plan : PlanBase {
     sweep_tb_kernel<T, ARITH, MODE, CHECK><<<tb_grid, tb::NT, tb::Cfg<T>::SMEM_BYTES, s>>>(A, mx, mxm, map_tb_f);
     return 0;
   }
-  template <int ARITH, int MODE>
-  int launch_tb_mode(const TbArgs<T>& A, const CUtensorMap& mx, const CUtensorMap& mxm, bool check, cudaStream_t s) {
-    return check ? launch_tb_inst<ARITH, MODE, true>(A, mx, mxm, s) : launch_tb_inst<ARITH, MODE, false>(A, mx, mxm, s);
-  }
   // One pass: sweeps first_cnt .. first_cnt+t-1 (1-based sweep numbers) of every solve that is not done.
   int launch_tb_pass(T* x0, int pass_idx, int first_cnt, int t, bool check, T alpha, int mode, const int* done, cudaStream_t s) {
     T* bufs[4] = {x0, x1, x2, x3};
@@ -741,21 +728,48 @@ struct Plan : PlanBase {
     A.tiles_x = tb_tiles_x; A.tiles_y = tb_tiles_y; A.nchunks = tb_nchunks; A.chunk = tb_chunk;
     const CUtensorMap& mx = map_tb[2 * pin];
     const CUtensorMap& mxm = map_tb[2 * pin + 1];
-    const bool strict = d.arith == XEE_ARITH_STRICT;
-    int rc;
-    if (mode == MODE_JACOBI) rc = strict ? launch_tb_mode<XEE_ARITH_STRICT, MODE_JACOBI>(A, mx, mxm, check, s) : launch_tb_mode<XEE_ARITH_FAST, MODE_JACOBI>(A, mx, mxm, check, s);
-    else rc = strict ? launch_tb_mode<XEE_ARITH_STRICT, MODE_CHEBYSHEV>(A, mx, mxm, check, s) : launch_tb_mode<XEE_ARITH_FAST, MODE_CHEBYSHEV>(A, mx, mxm, check, s);
+    const int rc = dispatch([&](auto strict, auto cheb, auto chk) { return launch_tb_inst<arith_of(strict), mode_of(cheb), chk>(A, mx, mxm, s); },
+                            d.arith == XEE_ARITH_STRICT, mode == MODE_CHEBYSHEV, check);
     if (rc) return rc;
     XEE_LAUNCH_OK();
     ++kernel_launches;
     return 0;
   }
-  // Boundary values and the first guess in every buffer (elliptic_tools.f90:166-171: workspace = dat).
-  int tb_seed_buffers(const T* x0, cudaStream_t s) {
+  // Boundary values and the first guess in every iterate buffer (elliptic_tools.f90:166-171: workspace = dat), and the tensor
+  // maps of this call's buffers.
+  int seed_buffers(T* x0, const T* f, cudaStream_t s) {
     const size_t fbytes = sizeof(T) * nn * d.nbatch;
     XEE_CHECK(cudaMemcpyAsync(x1, x0, fbytes, cudaMemcpyDeviceToDevice, s));
+    if (!use_tb) return prepare_maps(x0, x1, f, d.nbatch);
     XEE_CHECK(cudaMemcpyAsync(x2, x0, fbytes, cudaMemcpyDeviceToDevice, s));
     XEE_CHECK(cudaMemcpyAsync(x3, x0, fbytes, cudaMemcpyDeviceToDevice, s));
+    return prepare_tb_maps(x0, f, d.nbatch);
+  }
+  // Sweeps cnt+1 .. cnt+k (1-based sweep numbers) of every solve that is not done, with the residual partials of the last
+  // one when `check`.  v4 runs them in passes of up to tb_depth sweeps (tb_pass counts the passes of the call); the other
+  // kernels ping-pong: sweep c reads x0 when c is odd, x1 when it is even.
+  int run_sweeps(T* x0, const T* f, T alpha, int mode, int cnt, int k, bool check, const int* done, int& tb_pass, cudaStream_t s) {
+    const int end = cnt + k;
+    if (use_tb) {
+      for (; cnt < end; ++tb_pass) {
+        const int t = std::min(tb_depth, end - cnt);
+        if (launch_tb_pass(x0, tb_pass, cnt + 1, t, check && cnt + t == end, alpha, mode, done, s)) return 1;
+        cnt += t;
+      }
+    } else {
+      while (cnt < end) {
+        ++cnt;
+        const T* src = (cnt & 1) ? x0 : x1;
+        T* dst = (cnt & 1) ? x1 : x0;
+        const double om = mode == MODE_CHEBYSHEV ? cheb_omega_host(cnt, cheb_rho) : 1.0;
+        SweepArgs<T> a = args(src, dst, f, alpha, (T)om, done);
+        a.two_slot = (cnt & 1) ? 0 : 1;      // x0 owns coarse slot 0, x1 slot 1
+        if (mode == MODE_CHEBYSHEV && !d.shared_coe) { a.rho_ps = rho_dev; a.cheb_k = cnt; }
+        if (launch_sweep(a, mode, check && cnt == end, s)) return 1;
+      }
+      kernel_launches += k;
+    }
+    sweep_launches += k;
     return 0;
   }
 
@@ -780,8 +794,6 @@ struct Plan : PlanBase {
     return launch_sweep(a, MODE_APPLY, false, s);
   }
 
-  // Power iteration on the Jacobi iteration matrix G = I - D^-1 L (homogeneous problem, zero
-  // boundary): rho ~ ||G^{k+1} e|| / ||G^k e||.  Uses x1 and a scratch batch of size 1.
   // v3 resident solver (one cooperative launch per solve_elliptic call); see xee_resident.cuh
   int res_G = 0, res_P = 0;          // strips per solve, points per thread (0 = does not fit)
   T *res_final = nullptr, *res_prev = nullptr, *res_halo = nullptr;
@@ -814,22 +826,35 @@ struct Plan : PlanBase {
     XEE_LAUNCH_OK();
     return 0;
   }
-  template <int ARITH, int MODE>
-  int launch_resident_p(res::ResArgs<T>& ra, cudaStream_t s) {
-    return res_P == 1 ? launch_resident<ARITH, MODE, 1, 512>(ra, s) : res_P == 2 ? launch_resident<ARITH, MODE, 2, 512>(ra, s) : launch_resident<ARITH, MODE, 3, 512>(ra, s);
-  }
   int solve_resident(T* x0, const T* fd, const xee_solve_params* prm, int check_step, int converge_time, int lost_rate, int mode, cudaStream_t s);
   int estimate_rho(cudaStream_t s);
   int estimate_rho_subsampled(cudaStream_t s);
   std::vector<double> lmin_ps;       // two-level: per-set smallest eigenvalue of M^-1 L (host copy, for the subsampled estimate)
   std::vector<double> radius_ps;     // per-set spectral radius rho (rho_ps holds the focal distance the weights are computed from)
+  // Per-set Chebyshev parameters to rho_dev; h receives them in T, the values the device computes with.
+  int upload_rho(const std::vector<double>& v, std::vector<T>& h, cudaStream_t s) {
+    if (!rho_dev) XEE_CHECK(pool_alloc(&rho_dev, sizeof(T) * nsets));
+    h.resize(nsets);
+    for (int n = 0; n < nsets; ++n) h[n] = (T)v[n];
+    XEE_CHECK(cudaMemcpyAsync(rho_dev, h.data(), sizeof(T) * nsets, cudaMemcpyHostToDevice, s));
+    return 0;
+  }
+  // Two-level step length from the smallest eigenvalues lmin[n] of M^-1 L and the common largest one tl_lmax: one step from
+  // the mean lmin, with which the spectrum of solve n lies in [1 - gamma lmax, 1 - gamma lmin_n]; rho[n] its radius.
+  void two_step(const std::vector<double>& lmin, std::vector<double>& rho) {
+    double mean = 0.0;
+    for (int n = 0; n < nsets; ++n) mean += lmin[n] / nsets;
+    lmin_ps = lmin;
+    tl_lmin = mean;
+    tl_gamma = 2.0 / (tl_lmax + tl_lmin);
+    for (int n = 0; n < nsets; ++n) rho[n] = std::max(tl_gamma * tl_lmax - 1.0, 1.0 - tl_gamma * lmin[n]);
+  }
   // Make the Chebyshev parameters of this call available: explicit value, cached estimate, or a fresh estimate.
   int prepare_cheb(double rho_given, cudaStream_t s) {
     if (rho_given > 0 && !use_two) {   // (the two-level methods also need the step length: they always estimate)
       cheb_rho = rho_given; rho_ps.assign(nsets, rho_given);
-      if (!rho_dev) XEE_CHECK(pool_alloc(&rho_dev, sizeof(T) * nsets));
-      std::vector<T> h(nsets, (T)rho_given);
-      XEE_CHECK(cudaMemcpyAsync(rho_dev, h.data(), sizeof(T) * nsets, cudaMemcpyHostToDevice, s));
+      std::vector<T> h;
+      if (upload_rho(rho_ps, h, s)) return 1;
       XEE_CHECK(cudaStreamSynchronize(s));
       return 0;
     }
@@ -845,59 +870,23 @@ struct Plan : PlanBase {
   int sweeps(void* psi, const void* f, double alpha, int nsw, double* rms, cudaStream_t s) override {
     T* x0 = (T*)psi;
     const int mode = method_is_cheb() ? MODE_CHEBYSHEV : MODE_JACOBI;
-    if (use_tb) {
-      if (mode == MODE_CHEBYSHEV && prepare_cheb(0.0, s)) return 1;
-      if (tb_seed_buffers(x0, s) || prepare_tb_maps(x0, (const T*)f, d.nbatch)) return 1;
-      cudaEvent_t e0 = next_event(), e1 = next_event();
-      XEE_CHECK(cudaEventRecord(e0, s));
-      int cnt = 0, pass = 0;
-      while (cnt < nsw) {
-        const int t = std::min(tb_depth, nsw - cnt);
-        if (launch_tb_pass(x0, pass, cnt + 1, t, rms && cnt + t == nsw, (T)alpha, mode, nullptr, s)) return 1;
-        cnt += t; ++pass;
-      }
-      sweep_launches += nsw; variant_used = 4; depth_used = tb_depth;
-      XEE_CHECK(cudaEventRecord(e1, s));
-      if (pass & 1) XEE_CHECK(cudaMemcpyAsync(x0, x2, sizeof(T) * nn * d.nbatch, cudaMemcpyDeviceToDevice, s));
-      XEE_CHECK(cudaStreamSynchronize(s));
-      harvest_events();
-      if (rms && nsw > 0) {
-        const int nt = tb_ntiles();
-        std::vector<double> h((size_t)nt * d.nbatch);
-        XEE_CHECK(cudaMemcpy(h.data(), partial, sizeof(double) * h.size(), cudaMemcpyDeviceToHost));
-        const double N = (double)(d.nx - 2) * (d.ny - 2);
-        for (int n = 0; n < d.nbatch; ++n) {
-          double t = 0;
-          for (int q = 0; q < nt; ++q) t += h[(size_t)n * nt + q];
-          rms[n] = std::sqrt(t / N);
-        }
-      }
-      return 0;
-    }
-    XEE_CHECK(cudaMemcpyAsync(x1, x0, sizeof(T) * nn * d.nbatch, cudaMemcpyDeviceToDevice, s));
-    if (prepare_maps(x0, x1, (const T*)f, d.nbatch)) return 1;
     if (mode == MODE_CHEBYSHEV && prepare_cheb(0.0, s)) return 1;   // before the start event: the spectral probe is not sweep time
+    if (seed_buffers(x0, (const T*)f, s)) return 1;
     cheb_rho_used = cheb_rho; cheb_gamma_used = use_two ? tl_gamma : 1.0;
     cudaEvent_t e0 = next_event(), e1 = next_event();
     XEE_CHECK(cudaEventRecord(e0, s));
-    if (use_two && two_reset(d.nbatch, s)) return 1;
-    for (int cnt = 1; cnt <= nsw; ++cnt) {
-      const T* src = (cnt & 1) ? x0 : x1;
-      T* dst = (cnt & 1) ? x1 : x0;
-      const double om = mode == MODE_CHEBYSHEV ? cheb_omega_host(cnt, cheb_rho) : 1.0;
-      SweepArgs<T> a = args(src, dst, (const T*)f, (T)alpha, (T)om, nullptr);
-      a.two_slot = (cnt & 1) ? 0 : 1;      // x0 owns coarse slot 0, x1 slot 1
-      if (mode == MODE_CHEBYSHEV && !d.shared_coe) { a.rho_ps = rho_dev; a.cheb_k = cnt; }
-      if (launch_sweep(a, mode, rms && cnt == nsw, s)) return 1;
-    }
-    sweep_launches += nsw; kernel_launches += nsw; variant_used = use_line ? 5 : use_tma ? 2 : 1; depth_used = 1;
+    if (use_two && two_reset(s)) return 1;
+    int tb_pass = 0;
+    if (run_sweeps(x0, (const T*)f, (T)alpha, mode, 0, nsw, rms != nullptr, nullptr, tb_pass, s)) return 1;
+    variant_used = use_line ? 5 : use_tb ? 4 : use_tma ? 2 : 1; depth_used = use_tb ? tb_depth : 1;
     if (use_two && two_flush(x0, x1, d.nbatch, s)) return 1;
     XEE_CHECK(cudaEventRecord(e1, s));
-    if (nsw & 1) XEE_CHECK(cudaMemcpyAsync(x0, x1, sizeof(T) * nn * d.nbatch, cudaMemcpyDeviceToDevice, s));
+    // the last iterate: v4 leaves it in the pair (x2, x3) after an odd number of passes, the others in x1 after an odd sweep count
+    if (use_tb ? (tb_pass & 1) : (nsw & 1)) XEE_CHECK(cudaMemcpyAsync(x0, use_tb ? x2 : x1, sizeof(T) * nn * d.nbatch, cudaMemcpyDeviceToDevice, s));
     XEE_CHECK(cudaStreamSynchronize(s));
     harvest_events();
     if (rms && nsw > 0) {
-      const int nt = sweep_ntiles();
+      const int nt = check_ntiles();
       std::vector<double> h((size_t)nt * d.nbatch);
       XEE_CHECK(cudaMemcpy(h.data(), partial, sizeof(double) * h.size(), cudaMemcpyDeviceToHost));
       const double N = (double)(d.nx - 2) * (d.ny - 2);
@@ -979,7 +968,18 @@ int Plan<T>::estimate_rho(cudaStream_t s) {
   };
   // two-level: the probe vectors are (stored field, coarse vector) pairs; norms and differences need them made explicit
   auto flush = [&]() -> int { return use_two ? two_flush(e0, e1, ns, s) : 0; };
-  if (use_two && two_reset(ns, s)) return 1;
+  // one probe round: 2p Chebyshev sweeps from the current iterate, norms after p (nA) and after 2p (nB)
+  auto cheb_round = [&](int p) -> int {
+    int r = 0;
+    for (int k = 1; k <= 2 * p && !r; ++k) {
+      r = sweep(MODE_CHEBYSHEV, k);
+      if (k == p || k == 2 * p) r = r || flush();
+      if (k == p) r = r || norms(parity ? e1 : e0, nA);
+      if (k == 2 * p) r = r || norms(parity ? e1 : e0, nB);
+    }
+    return r;
+  };
+  if (use_two && two_reset(s)) return 1;
   if (use_two) {
     // ---- two-level: the spectrum of M^-1 L (M^-1 = block lines + coarse space) is [lmin, lmax] with lmax around 2, possibly
     // above it, so the step length gamma is part of the method:  G = I - gamma M^-1 L,  gamma = 2 / (lmax + lmin),
@@ -994,7 +994,7 @@ int Plan<T>::estimate_rho(cudaStream_t s) {
     TraceTimer t1("  probe: largest eigenvalue");
     if (start_vector(1)) return 1;
     tl_gamma = 1.0;
-    const int itL = env_int("XEE_LMAX_ITERS", ns > 1 ? 24 : 60);
+    const int itL = ns > 1 ? 24 : 60;
     for (int k = 1; k <= itL && !rc; ++k) {
       const T* cur = parity ? e1 : e0;
       if (k == itL) rc = rc || norms(cur, nA);
@@ -1021,7 +1021,7 @@ int Plan<T>::estimate_rho(cudaStream_t s) {
   // ---- stage A
   // probe lengths: the block-line splitting has a ~20x larger spectral gap than point Jacobi, so its modes separate in
   // proportionally fewer sweeps (64/64 measured: same sweep counts to tolerance as 200/200; 32/32 costs 2-3 % more sweeps)
-  const int itA = env_int("XEE_RHO_ITERS", use_two ? 32 : use_line ? 64 : 200);
+  const int itA = use_two ? 32 : use_line ? 64 : 200;
   { TraceTimer t2("  probe: stage A");
   for (int k = 1; k <= itA && !rc; ++k) {
     rc = sweep(MODE_JACOBI, 1);
@@ -1040,21 +1040,15 @@ int Plan<T>::estimate_rho(cudaStream_t s) {
     }
   }
   // ---- stage B
-  const int rounds = env_int("XEE_RHO_ROUNDS", 4), p = env_int("XEE_RHO_PROBE", use_two ? 32 : use_line ? 64 : 200);
+  const int rounds = 4, p = itA;
   std::vector<char> settled(ns, 0);
   auto lncosh = [](double x) { return x + std::log1p(std::exp(-2.0 * x)) - M_LN2; };
   for (int r = 0; r < rounds && !rc; ++r) {
     TraceTimer t3("  probe: stage B round");
-    for (int n = 0; n < ns; ++n) rho_h[n] = (T)rho[n];
-    XEE_CHECK(cudaMemcpyAsync(rho_dev, rho_h.data(), sizeof(T) * ns, cudaMemcpyHostToDevice, s));
+    if (upload_rho(rho, rho_h, s)) return 1;
     // restart the Chebyshev sequence from the current iterate: x_{-1} := x_0
     XEE_CHECK(cudaMemcpyAsync(parity ? e0 : e1, parity ? e1 : e0, sizeof(T) * nn * ns, cudaMemcpyDeviceToDevice, s));
-    for (int k = 1; k <= 2 * p && !rc; ++k) {
-      rc = sweep(MODE_CHEBYSHEV, k);
-      if (k == p || k == 2 * p) rc = rc || flush();
-      if (k == p) rc = rc || norms(parity ? e1 : e0, nA);
-      if (k == 2 * p) rc = rc || norms(parity ? e1 : e0, nB);
-    }
+    rc = cheb_round(p);
     if (rc) break;
     bool all_settled = true;
     for (int n = 0; n < ns; ++n) {
@@ -1082,14 +1076,9 @@ int Plan<T>::estimate_rho(cudaStream_t s) {
   }
   if (rc) return 1;
   if (use_two) {   // rho[n] is the spectral radius of I - gamma0 M^-1 L_n: lmin_n = (1 - rho_n) / gamma0, then the final step and radii
-    // (one common step from the mean lmin; with it the spectrum of solve n lies in [1 - gamma lmax, 1 - gamma lmin_n])
     std::vector<double> lmin(ns);
-    double mean = 0.0;
-    for (int n = 0; n < ns; ++n) { lmin[n] = (1.0 - rho[n]) / tl_gamma; mean += lmin[n] / ns; }
-    lmin_ps = lmin;
-    tl_lmin = mean;
-    tl_gamma = 2.0 / (tl_lmax + tl_lmin);
-    for (int n = 0; n < ns; ++n) rho[n] = std::max(tl_gamma * tl_lmax - 1.0, 1.0 - tl_gamma * lmin[n]);
+    for (int n = 0; n < ns; ++n) lmin[n] = (1.0 - rho[n]) / tl_gamma;
+    two_step(lmin, rho);
     if (env_int("XEE_TRACE", 0)) fprintf(stderr, "xee: two-level spectrum of M^-1 L: [%.4e, %.4f], gamma %.4f\n", tl_lmin, tl_lmax, tl_gamma);
   }
   // ---- stage C (line methods): complex eigenvalues.  With a strongly varying B the operator is not symmetric and the
@@ -1102,8 +1091,8 @@ int Plan<T>::estimate_rho(cudaStream_t s) {
   // decay 1/T_k(1/c) that every mode inside the ellipse shows; repeated with the new c until the excess is gone.
   std::vector<double> foci(rho);
   radius_ps = rho;
-  if (use_line && env_int("XEE_RHO_ELLIPSE", 1)) {
-    const int pc = env_int("XEE_RHO_PROBE_C", 64), roundsC = 3;
+  if (use_line) {
+    const int pc = 64, roundsC = 3;
     uint32_t lcg = 12345u;
     std::vector<T> h(nn, T(0));
     for (int j = 1; j < d.ny - 1; ++j)
@@ -1111,19 +1100,13 @@ int Plan<T>::estimate_rho(cudaStream_t s) {
     std::vector<char> doneC(ns, 0);
     for (int r = 0; r < roundsC && !rc; ++r) {
       TraceTimer t4("  probe: stage C round");
-      for (int n = 0; n < ns; ++n) rho_h[n] = (T)foci[n];
-      XEE_CHECK(cudaMemcpyAsync(rho_dev, rho_h.data(), sizeof(T) * ns, cudaMemcpyHostToDevice, s));
+      if (upload_rho(foci, rho_h, s)) return 1;
       XEE_CHECK(cudaMemcpyAsync(e0, h.data(), sizeof(T) * nn, cudaMemcpyHostToDevice, s));      // one upload, replicated on the device
       if (ns > 1) { probe_replicate_kernel<T><<<dim3((unsigned)((nn + 255) / 256), ns - 1), 256, 0, s>>>(e0, (long long)nn); XEE_LAUNCH_OK(); }
       XEE_CHECK(cudaMemcpyAsync(e1, e0, sizeof(T) * nn * ns, cudaMemcpyDeviceToDevice, s));
-      if (use_two && two_reset(ns, s)) return 1;
+      if (use_two && two_reset(s)) return 1;
       parity = 0;
-      for (int k = 1; k <= 2 * pc && !rc; ++k) {
-        rc = sweep(MODE_CHEBYSHEV, k);
-        if (k == pc || k == 2 * pc) rc = rc || flush();
-        if (k == pc) rc = rc || norms(parity ? e1 : e0, nA);
-        if (k == 2 * pc) rc = rc || norms(parity ? e1 : e0, nB);
-      }
+      rc = cheb_round(pc);
       if (rc) break;
       bool all = true;
       for (int n = 0; n < ns; ++n) {
@@ -1150,8 +1133,7 @@ int Plan<T>::estimate_rho(cudaStream_t s) {
     }
   }
   rho_ps = foci;   // what the Chebyshev weights are computed from
-  for (int n = 0; n < ns; ++n) rho_h[n] = (T)foci[n];
-  XEE_CHECK(cudaMemcpyAsync(rho_dev, rho_h.data(), sizeof(T) * ns, cudaMemcpyHostToDevice, s));
+  if (upload_rho(foci, rho_h, s)) return 1;
   XEE_CHECK(cudaStreamSynchronize(s));
   cheb_rho = foci[0];
   if (env_int("XEE_TRACE", 0)) fprintf(stderr, "xee: Jacobi spectral radius estimate rho[0] = 1 - %.4e (%d operator set%s)\n", 1.0 - rho[0], ns, ns > 1 ? "s" : "");
@@ -1189,28 +1171,22 @@ int Plan<T>::estimate_rho_subsampled(cudaStream_t s) {
   for (int q = 0; q < nq; ++q)
     if (!(v[q] > 0.0)) return fail("xee: subsampled spectral estimate: non-positive gap");
   std::vector<double> rho(nsets), lmin(nsets), bim(nsets);
-  double mean = 0.0;
   for (int n = 0, q = 0; n < nsets; ++n) {
     while (q + 1 < nq - 1 && idx[q + 1] <= n) ++q;
     const double t = idx[q + 1] > idx[q] ? (double)(n - idx[q]) / (idx[q + 1] - idx[q]) : 0.0;
     lmin[n] = std::exp((1.0 - t) * std::log(v[q]) + t * std::log(v[q + 1]));
     bim[n] = std::max(bq[q], bq[q + 1]);        // the larger neighbour: an over-estimate costs sweeps, an under-estimate convergence
-    mean += lmin[n] / nsets;
   }
   if (use_two) {
-    tl_lmax = sub.tl_lmax; tl_lmin = mean;
-    tl_gamma = 2.0 / (tl_lmax + tl_lmin);
-    for (int n = 0; n < nsets; ++n) rho[n] = std::max(tl_gamma * tl_lmax - 1.0, 1.0 - tl_gamma * lmin[n]);
-    lmin_ps = lmin;
+    tl_lmax = sub.tl_lmax;
+    two_step(lmin, rho);
   } else {
     for (int n = 0; n < nsets; ++n) rho[n] = 1.0 - lmin[n];
   }
   radius_ps = rho;
   for (int n = 0; n < nsets; ++n) rho[n] = std::sqrt(std::max(rho[n] * rho[n] - bim[n] * bim[n], 1e-4));   // focal distances
-  if (!rho_dev) XEE_CHECK(pool_alloc(&rho_dev, sizeof(T) * nsets));
-  std::vector<T> rho_h(nsets);
-  for (int n = 0; n < nsets; ++n) rho_h[n] = (T)rho[n];
-  XEE_CHECK(cudaMemcpyAsync(rho_dev, rho_h.data(), sizeof(T) * nsets, cudaMemcpyHostToDevice, s));
+  std::vector<T> rho_h;
+  if (upload_rho(rho, rho_h, s)) return 1;
   XEE_CHECK(cudaStreamSynchronize(s));
   rho_ps = rho; cheb_rho = rho[0];
   if (env_int("XEE_TRACE", 0)) fprintf(stderr, "xee: subsampled spectral estimate: %d of %d operator sets probed, gap[0] = %.4e, gap[last] = %.4e\n", nq, nsets, lmin[0], lmin[nsets - 1]);
@@ -1248,14 +1224,13 @@ int Plan<T>::solve_resident(T* x0, const T* fd, const xee_solve_params* prm, int
     XEE_CHECK(cudaStreamSynchronize(s));
   }
   ra.omega_tab = res_omega;
-  ra.dbg = env_int("XEE_RES_DEBUG", 0);
   ra.r1 = st.r1; ra.r2 = st.r2; ra.detect_explode = prm->detect_explode; ra.stall_checks = prm->stall_checks;
   ra.iters = st.iters; ra.errb = st.errb; ra.err_now = st.err_now; ra.ratio = st.ratio;
   ra.trace_err = st.trace_err; ra.trace_ratio = st.trace_ratio; ra.trace_cap = st.trace_cap;
-  const bool strict = d.arith == XEE_ARITH_STRICT;
-  int rc;
-  if (mode == MODE_JACOBI) rc = strict ? launch_resident_p<XEE_ARITH_STRICT, MODE_JACOBI>(ra, s) : launch_resident_p<XEE_ARITH_FAST, MODE_JACOBI>(ra, s);
-  else rc = strict ? launch_resident_p<XEE_ARITH_STRICT, MODE_CHEBYSHEV>(ra, s) : launch_resident_p<XEE_ARITH_FAST, MODE_CHEBYSHEV>(ra, s);
+  const int rc = dispatch([&](auto strict, auto cheb) {
+    constexpr int A = arith_of(strict), M = mode_of(cheb);
+    return res_P == 1 ? launch_resident<A, M, 1, 512>(ra, s) : res_P == 2 ? launch_resident<A, M, 2, 512>(ra, s) : launch_resident<A, M, 3, 512>(ra, s);
+  }, d.arith == XEE_ARITH_STRICT, mode == MODE_CHEBYSHEV);
   if (rc) return rc;
   // dat <- last iterate; the other buffer as the reference leaves `workspace` (penultimate iterate when the
   // sweep count is even, a copy of the result when it is odd: elliptic_tools.f90:259-264)
@@ -1298,33 +1273,31 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   if (norm_max && !partial_max) XEE_CHECK(pool_alloc(&partial_max, sizeof(double) * nb * kResmaxBlocks));
   const bool resident_ok = !norm_max && !use_line && (d.shared_coe || nb == 1) && max_iter >= 1 && resident_fits();
   if (want_kernel == 3 && !resident_ok) return fail("xee: kernel=3 (resident) needs a problem that fits: nbatch*strips <= SMs, <= 1536 points per strip");
-  if (want_kernel == 3 || (want_kernel == 0 && resident_ok && nb <= 2)) {
-    cudaEvent_t e0 = next_event(), e1 = next_event();
-    XEE_CHECK(cudaEventRecord(e0, s));
-    if (solve_resident(x0, fd, prm, check_step, converge_time, lost_rate, mode, s)) return 1;
-    ++kernel_launches; variant_used = 3; depth_used = 1;
-    XEE_CHECK(cudaEventRecord(e1, s));
+  // the results: fields back to the host (host entry points), iters, err, r1 and r2 of every solve
+  auto finish = [&](bool resident) -> int {
+    if (host_io) {
+      XEE_CHECK(cudaMemcpyAsync(psi, x0, fbytes, cudaMemcpyDeviceToHost, s));
+      if (workspace_host) XEE_CHECK(cudaMemcpyAsync(workspace_host, x1, fbytes, cudaMemcpyDeviceToHost, s));
+    }
     std::vector<int> hi(nb), he(nb);
     std::vector<T> h1(nb), h2(nb);
     XEE_CHECK(cudaMemcpyAsync(hi.data(), st.iters, sizeof(int) * nb, cudaMemcpyDeviceToHost, s));
     XEE_CHECK(cudaMemcpyAsync(he.data(), st.errb, sizeof(int) * nb, cudaMemcpyDeviceToHost, s));
     XEE_CHECK(cudaMemcpyAsync(h1.data(), st.err_now, sizeof(T) * nb, cudaMemcpyDeviceToHost, s));
     XEE_CHECK(cudaMemcpyAsync(h2.data(), st.ratio, sizeof(T) * nb, cudaMemcpyDeviceToHost, s));
-    if (host_io) {
-      XEE_CHECK(cudaMemcpyAsync(psi, x0, fbytes, cudaMemcpyDeviceToHost, s));
-      if (workspace_host) XEE_CHECK(cudaMemcpyAsync(workspace_host, x1, fbytes, cudaMemcpyDeviceToHost, s));
-    }
     XEE_CHECK(cudaStreamSynchronize(s));
     harvest_events();
     for (int n = 0; n < nb; ++n) {
-      if (he[n] & 0x100) return fail("xee: resident solver watchdog tripped (a CTA waited too long for its neighbour)");
-      sweep_launches += hi[n];
+      if (resident) {   // one launch ran every sweep of the solve
+        if (he[n] & 0x100) return fail("xee: resident solver watchdog tripped (a CTA waited too long for its neighbour)");
+        sweep_launches += hi[n];
+      }
       if (iters) iters[n] = hi[n];
       if (err) err[n] = he[n];
       if (r1o) r1o[n] = (double)h1[n];
       if (r2o) r2o[n] = (double)h2[n];
     }
-    if (debug == 2) {
+    if (resident && debug == 2) {   // the per-check lines of solve 0 (the loop below prints them as it goes)
       const int nchk = std::min(hi[0] / check_step, st.trace_cap);
       std::vector<T> te(nchk), tr(nchk);
       if (nchk > 0) {
@@ -1334,14 +1307,17 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
       for (int q = 0; q < nchk; ++q) printf("Iter: %8d, err_now: %12.3E, ratio: %12.3E\n", (q + 1) * check_step, (double)te[q], (double)tr[q]);
     }
     return 0;
+  };
+  if (want_kernel == 3 || (want_kernel == 0 && resident_ok && nb <= 2)) {
+    cudaEvent_t e0 = next_event(), e1 = next_event();
+    XEE_CHECK(cudaEventRecord(e0, s));
+    if (solve_resident(x0, fd, prm, check_step, converge_time, lost_rate, mode, s)) return 1;
+    ++kernel_launches; variant_used = 3; depth_used = 1;
+    XEE_CHECK(cudaEventRecord(e1, s));
+    return finish(true);
   }
-  // workspace = dat: both ping-pong buffers start as boundary + first guess (:166-171)
-  if (use_tb) { if (tb_seed_buffers(x0, s) || prepare_tb_maps(x0, fd, nb)) return 1; }
-  else {
-    XEE_CHECK(cudaMemcpyAsync(x1, x0, fbytes, cudaMemcpyDeviceToDevice, s));
-    if (prepare_maps(x0, x1, fd, nb)) return 1;
-  }
-  if (use_two && two_reset(nb, s)) return 1;
+  if (seed_buffers(x0, fd, s)) return 1;
+  if (use_two && two_reset(s)) return 1;
   int tb_pass = 0;
   variant_used = use_line ? 5 : use_tb ? 4 : use_tma ? 2 : 1; depth_used = use_tb ? tb_depth : 1;
   const int ninterior = (d.nx - 2) * (d.ny - 2);
@@ -1355,38 +1331,22 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
     const int chunk = std::min(to_check, max_iter - cnt);
     cudaEvent_t e0 = next_event(), e1 = next_event();
     XEE_CHECK(cudaEventRecord(e0, s));
-    for (int rem = use_tb ? chunk : 0; rem > 0;) {   // v4: passes of up to tb_depth sweeps, a check closes a pass
-      const int t = std::min(tb_depth, rem);
-      const bool check = ((cnt + t) % check_step) == 0;
-      if (launch_tb_pass(x0, tb_pass, cnt + 1, t, check, (T)prm->alpha, mode, st.done, s)) return 1;
-      cnt += t; rem -= t; ++tb_pass;
-    }
-    for (int k = 0; k < chunk && !use_tb; ++k) {
-      ++cnt;
-      const T* src = (cnt & 1) ? x0 : x1;   // sweep cnt reads the buffer written by sweep cnt-1
-      T* dst = (cnt & 1) ? x1 : x0;
-      const bool check = (cnt % check_step) == 0;                                // :179-183
-      const double om = mode == MODE_CHEBYSHEV ? cheb_omega_host(cnt, cheb_rho) : 1.0;
-      SweepArgs<T> a = args(src, dst, fd, (T)prm->alpha, (T)om, st.done);
-      a.two_slot = (cnt & 1) ? 0 : 1;      // x0 owns coarse slot 0, x1 slot 1
-      if (mode == MODE_CHEBYSHEV && !d.shared_coe) { a.rho_ps = rho_dev; a.cheb_k = cnt; }
-      if (launch_sweep(a, mode, check, s)) return 1;
-    }
-    sweep_launches += chunk;
-    if (!use_tb) kernel_launches += chunk;
+    const bool check = ((cnt + chunk) % check_step) == 0;                        // :179-183
+    if (run_sweeps(x0, fd, (T)prm->alpha, mode, cnt, chunk, check, st.done, tb_pass, s)) return 1;
+    cnt += chunk;
     XEE_CHECK(cudaEventRecord(e1, s));
-    if ((cnt % check_step) == 0) {
+    if (check) {
       // an accelerated iteration with a wrong spectral estimate diverges: a non-finite residual always stops it (err bit 1)
       if (norm_max) {   // the residual of the iterate this check sweep read (it is still in its buffer), in the max norm
         const T* src = (cnt & 1) ? x0 : x1;
-        const dim3 g(kResmaxBlocks, nb);
-        if (d.arith == XEE_ARITH_STRICT)
-          resmax_kernel<T, XEE_ARITH_STRICT><<<g, 256, 0, s>>>(src, fd, coe, d.shared_coe ? 0 : (long long)kPlanes * nn, (long long)nn, d.nx, d.ny, st.done, partial_max);
-        else
-          resmax_kernel<T, XEE_ARITH_FAST><<<g, 256, 0, s>>>(src, fd, coe, d.shared_coe ? 0 : (long long)kPlanes * nn, (long long)nn, d.nx, d.ny, st.done, partial_max);
+        dispatch([&](auto strict) {
+          resmax_kernel<T, arith_of(strict)><<<dim3(kResmaxBlocks, nb), 256, 0, s>>>(src, fd, coe, d.shared_coe ? 0 : (long long)kPlanes * nn,
+                                                                                    (long long)nn, d.nx, d.ny, st.done, partial_max);
+          return 0;
+        }, d.arith == XEE_ARITH_STRICT);
         XEE_LAUNCH_OK();
       }
-      finalize_check_kernel<T><<<nb, 128, 0, s>>>(st, norm_max ? partial_max : partial, norm_max ? kResmaxBlocks : use_tb ? tb_ntiles() : sweep_ntiles(),
+      finalize_check_kernel<T><<<nb, 128, 0, s>>>(st, norm_max ? partial_max : partial, norm_max ? kResmaxBlocks : check_ntiles(),
                                                   ninterior, cnt, check_idx, converge_time, lost_rate, max_iter,
                                                   prm->detect_explode || mode == MODE_CHEBYSHEV, prm->stall_checks, norm_max, norm_floor);
       XEE_LAUNCH_OK();
@@ -1423,35 +1383,13 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   if (use_tb) select_result_tb_kernel<T><<<g, 256, 0, s>>>(x0, x1, x2, x3, st.iters, (long long)nn, check_step, tb_depth);
   else select_result_kernel<T><<<g, 256, 0, s>>>(x0, x1, st.iters, (long long)nn, 1);
   XEE_LAUNCH_OK();
-  if (host_io) {
-    XEE_CHECK(cudaMemcpyAsync(psi, x0, fbytes, cudaMemcpyDeviceToHost, s));
-    if (workspace_host) XEE_CHECK(cudaMemcpyAsync(workspace_host, x1, fbytes, cudaMemcpyDeviceToHost, s));
-  }
-  std::vector<int> hi(nb), he(nb);
-  std::vector<T> h1(nb), h2(nb);
-  XEE_CHECK(cudaMemcpyAsync(hi.data(), st.iters, sizeof(int) * nb, cudaMemcpyDeviceToHost, s));
-  XEE_CHECK(cudaMemcpyAsync(he.data(), st.errb, sizeof(int) * nb, cudaMemcpyDeviceToHost, s));
-  XEE_CHECK(cudaMemcpyAsync(h1.data(), st.err_now, sizeof(T) * nb, cudaMemcpyDeviceToHost, s));
-  XEE_CHECK(cudaMemcpyAsync(h2.data(), st.ratio, sizeof(T) * nb, cudaMemcpyDeviceToHost, s));
-  XEE_CHECK(cudaStreamSynchronize(s));
-  harvest_events();
-  for (int n = 0; n < nb; ++n) {
-    if (iters) iters[n] = hi[n];
-    if (err) err[n] = he[n];
-    if (r1o) r1o[n] = (double)h1[n];
-    if (r2o) r2o[n] = (double)h2[n];
-  }
-  return 0;
+  return finish(false);
 }
 
 inline int make_plan(const xee_plan_desc* desc, PlanBase** out) {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-    return fail("xee: no CUDA device available - this library has no CPU fallback");
+  int dev = 0;
+  if (resolve_device(desc->device, &dev)) return 1;
   if (desc->nx < 3 || desc->ny < 3 || desc->nbatch < 1) return fail("xee: nx, ny >= 3 and nbatch >= 1 required");
-  int dev = desc->device;
-  if (dev < 0) XEE_CHECK(cudaGetDevice(&dev));      // "current device", resolved so that later entry points can return to it
-  if (dev >= ndev) return fail("xee: device index out of range");
   DeviceGuard guard(dev);
   PlanBase* p = nullptr;
   int rc;

@@ -56,7 +56,6 @@ struct ResArgs {
   int max_iter, check_step, converge_time, lost_rate;
   T alpha; double rho;  // rho: Jacobi spectral radius (Chebyshev)
   const T* omega_tab;   // [kChebClamp] host-computed Chebyshev weights
-  int dbg;              // timing experiments only (XEE_RES_DEBUG): 1 skip neighbour wait, 2 skip halo pull, 4 skip release
   const T* r1; const T* r2;   // [nb] thresholds (HUGE when disabled)
   int detect_explode, stall_checks;
   // results
@@ -163,14 +162,14 @@ __global__ void __launch_bounds__(NT, 1) solve_resident_kernel(const ResArgs<T> 
     __syncthreads();                                // strip updated; exchange rows and partial issued by the CTA
     if (tid == 0) {
       // release (cumulative over the CTA's writes ordered before it by the barrier): publish sweep `cnt`
-      if (!(a.dbg & 4)) st_release(&flags[(size_t)g * FLAG_PAD], cnt);
+      st_release(&flags[(size_t)g * FLAG_PAD], cnt);
       if (check) atomicAdd(&a.check_cnt[(size_t)n * 64], 1);
     }
     // ---- wait for the two neighbours to have finished sweep cnt, then pull their rows into the halo rows.
     // Only the two polling threads ever touch the flags; the shared abort word is read only while spinning long.
     if (tid < 2) {
       const int nb = (tid == 0) ? g - 1 : g + 1;
-      if (nb >= 0 && nb < G && !(a.dbg & 1)) {
+      if (nb >= 0 && nb < G) {
         long long spins = 0;
         while (ld_acquire(&flags[(size_t)nb * FLAG_PAD]) < cnt) {
           if ((++spins & 0xfff) == 0 && (spins > SPIN_LIMIT || ld_acquire(a.abort_flag))) { atomicExch(a.abort_flag, 1); sh_abort = 1; break; }
@@ -179,7 +178,7 @@ __global__ void __launch_bounds__(NT, 1) solve_resident_kernel(const ResArgs<T> 
     }
     __syncthreads();
     if (sh_abort) { aborted = true; break; }
-    if (!(a.dbg & 2)) {   // both neighbour rows: issue every load before the first shared-memory store
+    {   // both neighbour rows: issue every load before the first shared-memory store
       const T* lo = halo + ((size_t)par * G + (g > 0 ? g - 1 : 0)) * 2 * nx + nx;       // last row of CTA g-1
       const T* hi = halo + ((size_t)par * G + (g < G - 1 ? g + 1 : g)) * 2 * nx;        // first row of CTA g+1
       for (int i = 1 + tid; i <= w; i += NT) {

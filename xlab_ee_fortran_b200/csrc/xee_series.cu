@@ -282,11 +282,8 @@ struct xee_series { SeriesBase* impl; };
 
 extern "C" {
 int xee_series_create(const xee_series_desc* desc, xee_series** out) {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail("xee: no CUDA device available - this library has no CPU fallback");
-  int dev = desc->device;
-  if (dev < 0) XEE_CHECK(cudaGetDevice(&dev));
-  if (dev >= ndev) return fail("xee: device index out of range");
+  int dev = 0;
+  if (resolve_device(desc->device, &dev)) return 1;
   DeviceGuard guard(dev);
   if (desc->nr < 4 || desc->nz < 5 || desc->nsnap < 1) return fail("xee_series: nr >= 4, nz >= 5 and nsnap >= 1 required");
   SeriesBase* m = nullptr; int rc;
@@ -300,13 +297,7 @@ int xee_series_create(const xee_series_desc* desc, xee_series** out) {
 int xee_series_destroy(xee_series* m) { if (m) { DeviceGuard g(m->impl->device()); delete m->impl; delete m; } return 0; }
 int xee_series_run_host(xee_series* m, const double* params, const xee_solve_params* prm, double* table) { DeviceGuard g(m->impl->device()); return m->impl->run(params, prm, table); }
 int xee_series_get_field(xee_series* m, int which, void* out) { DeviceGuard g(m->impl->device()); return m->impl->get_field(which, out); }
-int xee_series_sweep_kernel_stats(xee_series* m, double* ms, long long* launches, int reset) {
-  PlanBase* p = m->impl->plan();
-  if (ms) *ms = p->sweep_ms;
-  if (launches) *launches = p->sweep_launches;
-  if (reset) { p->sweep_ms = 0; p->sweep_launches = 0; p->kernel_launches = 0; }
-  return 0;
-}
+int xee_series_sweep_kernel_stats(xee_series* m, double* ms, long long* launches, int reset) { return m->impl->plan()->kernel_stats(ms, launches, reset); }
 int xee_series_probe_stats(xee_series* m, double* ms, int reset) {
   PlanBase* p = m->impl->plan();
   if (ms) *ms = p->probe_ms;
@@ -314,10 +305,6 @@ int xee_series_probe_stats(xee_series* m, double* ms, int reset) {
   return 0;
 }
 int xee_series_kernel_info(xee_series* m, int* variant, int* sweeps_per_pass, long long* kernel_launches) {
-  PlanBase* p = m->impl->plan();
-  if (variant) *variant = p->variant_used;
-  if (sweeps_per_pass) *sweeps_per_pass = p->depth_used;
-  if (kernel_launches) *kernel_launches = p->kernel_launches;
-  return 0;
+  return m->impl->plan()->kernel_info(variant, sweeps_per_pass, kernel_launches);
 }
 }  // extern "C"
