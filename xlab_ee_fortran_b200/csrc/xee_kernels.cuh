@@ -330,6 +330,43 @@ __global__ void __launch_bounds__(256) resmax_kernel(const T* __restrict__ src, 
   }
 }
 
+// The stop rule of one solve at one check (elliptic_tools.f90:201-233) and its two extensions: the explode rules
+// (detect_explode) and the stall detector (stall_checks > 0).  The one copy of the rule: the per-launch sweep loop
+// (finalize_check_kernel) and the resident solver call it.  Returns whether the solve stops here; `ratio` receives the
+// signed relative change (err_before - err_now) / err_before of :201.
+template <class T>
+struct StopRule {
+  T err_before, best;          // residual of the previous check (HUGE before the first one) and the best one seen
+  int ccnt, lcnt, errb, stall;
+};
+
+template <class T>
+__device__ __forceinline__ bool stop_rule_check(StopRule<T>& s, T err_now, T r1, T r2, int converge_time, int lost_rate,
+                                                int detect_explode, int stall_checks, T& ratio) {
+  using R = Rn<T>;
+  ratio = R::div(R::sub(s.err_before, err_now), s.err_before);                   // :201
+  const T aratio = R::abs(ratio);                                                 // :205
+  bool stop = false;
+  if (s.err_before == T(0)) {                                                     // :206
+    stop = true;
+  } else if ((err_now < r1) && (aratio < r2)) {                                   // :211
+    s.ccnt += 1; s.lcnt = 0;
+    if (s.ccnt >= converge_time) stop = true;
+  } else if (s.ccnt > 0) {                                                        // :221
+    s.lcnt += 1;
+    if (s.lcnt >= lost_rate) { s.ccnt -= 1; s.lcnt = 0; }
+  }
+  if (detect_explode && !(err_now == err_now && R::abs(err_now) <= R::huge())) { stop = true; s.errb |= XEE_ERR_EXPLODE; }
+  // (accelerated methods pass detect_explode = 1) a residual 10^6 above the best one seen is a divergent iteration too
+  if (detect_explode && stall_checks > 0 && err_now > s.best * T(1e6)) { stop = true; s.errb |= XEE_ERR_EXPLODE; }
+  if (stall_checks > 0 && !stop) {   // opt-in: the residual sits on its round-off floor above r1
+    if (err_now < s.best * T(0.999)) { s.best = err_now; s.stall = 0; }
+    else if (++s.stall >= stall_checks) { stop = true; s.errb |= XEE_ERR_STALLED; }
+  }
+  s.err_before = err_now;                                                         // :233
+  return stop;
+}
+
 // One block per solve: deterministic sum of the tile partials, then the stop-rule state machine.
 // norm_max != 0 (legacy strategies 3/4): the partials are maxima of |r| and err_now = max(they, floor_max), floor_max = the
 // largest |boundary value| (the legacy maxval runs over the whole array, whose rim holds the Dirichlet values).
@@ -359,32 +396,15 @@ __global__ void __launch_bounds__(128) finalize_check_kernel(SolveState<T> st, c
   }
   if (threadIdx.x != 0) return;
   const T err_now = norm_max ? (T)nanmax(tot, floor_max) : R::sqrt(R::div((T)tot, (T)ninterior));   // :199 / legacy :204
-  const T err_before = st.err_before[n];
-  T ratio = R::div(R::sub(err_before, err_now), err_before);                      // :201
+  StopRule<T> r{st.err_before[n], st.best_err[n], st.ccnt[n], st.lcnt[n], st.errb[n], st.stall[n]};
+  T ratio;
+  bool stop = stop_rule_check(r, err_now, st.r1[n], st.r2[n], converge_time, lost_rate, detect_explode, stall_checks, ratio);
   if (n == 0 && check_idx < st.trace_cap) { st.trace_err[check_idx] = err_now; st.trace_ratio[check_idx] = ratio; }
-  ratio = R::abs(ratio);                                                          // :205
-  bool stop = false;
-  int ccnt = st.ccnt[n], lcnt = st.lcnt[n], errb = st.errb[n];
-  if (err_before == T(0)) {                                                       // :206
-    stop = true;
-  } else if ((err_now < st.r1[n]) && (ratio < st.r2[n])) {                        // :211
-    ccnt += 1; lcnt = 0;
-    if (ccnt >= converge_time) stop = true;
-  } else if (ccnt > 0) {                                                          // :221
-    lcnt += 1;
-    if (lcnt >= lost_rate) { ccnt -= 1; lcnt = 0; }
-  }
-  if (detect_explode && !(err_now == err_now && R::abs(err_now) <= R::huge())) { stop = true; errb |= XEE_ERR_EXPLODE; }
-  // (accelerated methods pass detect_explode = 1) a residual 10^6 above the best one seen is a divergent iteration too
-  if (detect_explode && stall_checks > 0 && err_now > st.best_err[n] * T(1e6)) { stop = true; errb |= XEE_ERR_EXPLODE; }
-  if (stall_checks > 0 && !stop) {   // opt-in: the residual sits on its round-off floor above r1
-    if (err_now < st.best_err[n] * T(0.999)) { st.best_err[n] = err_now; st.stall[n] = 0; }
-    else if (++st.stall[n] >= stall_checks) { stop = true; errb |= XEE_ERR_STALLED; }
-  }
-  st.err_before[n] = err_now;                                                     // :233
-  st.err_now[n] = err_now; st.ratio[n] = ratio;
+  st.err_before[n] = r.err_before; st.best_err[n] = r.best; st.stall[n] = r.stall;
+  st.err_now[n] = err_now; st.ratio[n] = R::abs(ratio);
+  int errb = r.errb;
   if (cnt == max_iter) { stop = true; errb |= XEE_ERR_OVER_MAX_ITERATION; }       // :242-244
-  st.ccnt[n] = ccnt; st.lcnt[n] = lcnt; st.errb[n] = errb;
+  st.ccnt[n] = r.ccnt; st.lcnt[n] = r.lcnt; st.errb[n] = errb;
   if (stop) { st.done[n] = 1; st.iters[n] = cnt; atomicSub(st.active, 1); }
 }
 

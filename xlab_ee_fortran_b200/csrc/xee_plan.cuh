@@ -214,6 +214,7 @@ struct Plan : PlanBase {
   cudaEvent_t poll_ev[4]{};
   double cheb_rho = 0.0;             // shared operator: one spectral radius
   std::vector<double> rho_ps;        // one operator per solve: per-solve spectral radii (host copy)
+  std::vector<double> est_rho_ps;    // the spectral estimate of the current operator (rho_ps of the calls that estimate)
   T* rho_dev = nullptr;              //   ... and on the device
   // v2 (TMA) sweep kernel: launch geometry + tensor maps of the buffers of the current call
   bool use_tma = false;
@@ -472,7 +473,7 @@ struct Plan : PlanBase {
     XEE_LAUNCH_OK();
     XEE_CHECK(cudaStreamSynchronize(own_stream));
     if (tmp) pool_free(tmp);
-    cheb_rho = 0.0; rho_ps.clear();
+    cheb_rho = 0.0; rho_ps.clear(); est_rho_ps.clear();
     return line_factors();
   }
   int set_abc(const void* a, const void* b, const void* c, double dx, double dy) override {
@@ -484,7 +485,7 @@ struct Plan : PlanBase {
                                                  d.ny, sa, sb, sc, (long long)kPlanes * nn);
     XEE_LAUNCH_OK();
     XEE_CHECK(cudaStreamSynchronize(own_stream));
-    cheb_rho = 0.0; rho_ps.clear();
+    cheb_rho = 0.0; rho_ps.clear(); est_rho_ps.clear();
     return line_factors();
   }
   int line_factors() {   // Thomas factors of the radial segments (v5), once per operator
@@ -826,7 +827,8 @@ struct Plan : PlanBase {
     XEE_LAUNCH_OK();
     return 0;
   }
-  int solve_resident(T* x0, const T* fd, const xee_solve_params* prm, int check_step, int converge_time, int lost_rate, int mode, cudaStream_t s);
+  int solve_resident(T* x0, const T* fd, const xee_solve_params* prm, int check_step, int converge_time, int lost_rate, int mode,
+                     int detect_explode, cudaStream_t s);
   int estimate_rho(cudaStream_t s);
   int estimate_rho_subsampled(cudaStream_t s);
   std::vector<double> lmin_ps;       // two-level: per-set smallest eigenvalue of M^-1 L (host copy, for the subsampled estimate)
@@ -849,22 +851,28 @@ struct Plan : PlanBase {
     tl_gamma = 2.0 / (tl_lmax + tl_lmin);
     for (int n = 0; n < nsets; ++n) rho[n] = std::max(tl_gamma * tl_lmax - 1.0, 1.0 - tl_gamma * lmin[n]);
   }
-  // Make the Chebyshev parameters of this call available: explicit value, cached estimate, or a fresh estimate.
+  // Make the Chebyshev parameters of this call available: an explicit value for this call only, else the estimate of the
+  // current operator, computed once and uploaded again when an earlier call replaced it with an explicit value.
   int prepare_cheb(double rho_given, cudaStream_t s) {
     if (rho_given > 0 && !use_two) {   // (the two-level methods also need the step length: they always estimate)
-      cheb_rho = rho_given; rho_ps.assign(nsets, rho_given);
-      std::vector<T> h;
-      if (upload_rho(rho_ps, h, s)) return 1;
+      rho_ps.assign(nsets, rho_given);
+    } else if (!est_rho_ps.empty()) {
+      if (rho_ps == est_rho_ps) return 0;
+      rho_ps = est_rho_ps;
+    } else {
       XEE_CHECK(cudaStreamSynchronize(s));
-      return 0;
+      const double t0 = TraceTimer::now();
+      const bool sub = !d.shared_coe && rho_subsample > 1 && nsets >= 4 * rho_subsample;
+      const int rc = sub ? estimate_rho_subsampled(s) : estimate_rho(s);      // synchronises the stream before it returns
+      probe_ms += (TraceTimer::now() - t0) * 1e3;
+      if (rc == 0) est_rho_ps = rho_ps;
+      return rc;
     }
-    if (cheb_rho > 0 && (int)rho_ps.size() == nsets) return 0;
+    cheb_rho = rho_ps[0];
+    std::vector<T> h;
+    if (upload_rho(rho_ps, h, s)) return 1;
     XEE_CHECK(cudaStreamSynchronize(s));
-    const double t0 = TraceTimer::now();
-    const bool sub = !d.shared_coe && rho_subsample > 1 && nsets >= 4 * rho_subsample;
-    const int rc = sub ? estimate_rho_subsampled(s) : estimate_rho(s);      // synchronises the stream before it returns
-    probe_ms += (TraceTimer::now() - t0) * 1e3;
-    return rc;
+    return 0;
   }
 
   int sweeps(void* psi, const void* f, double alpha, int nsw, double* rms, cudaStream_t s) override {
@@ -1195,7 +1203,7 @@ int Plan<T>::estimate_rho_subsampled(cudaStream_t s) {
 
 template <class T>
 int Plan<T>::solve_resident(T* x0, const T* fd, const xee_solve_params* prm, int check_step, int converge_time,
-                            int lost_rate, int mode, cudaStream_t s) {
+                            int lost_rate, int mode, int detect_explode, cudaStream_t s) {
   const int nb = d.nbatch, G = res_G;
   const size_t fbytes = sizeof(T) * nn * nb;
   if (!res_final) {
@@ -1224,7 +1232,7 @@ int Plan<T>::solve_resident(T* x0, const T* fd, const xee_solve_params* prm, int
     XEE_CHECK(cudaStreamSynchronize(s));
   }
   ra.omega_tab = res_omega;
-  ra.r1 = st.r1; ra.r2 = st.r2; ra.detect_explode = prm->detect_explode; ra.stall_checks = prm->stall_checks;
+  ra.r1 = st.r1; ra.r2 = st.r2; ra.detect_explode = detect_explode; ra.stall_checks = prm->stall_checks;
   ra.iters = st.iters; ra.errb = st.errb; ra.err_now = st.err_now; ra.ratio = st.ratio;
   ra.trace_err = st.trace_err; ra.trace_ratio = st.trace_ratio; ra.trace_cap = st.trace_cap;
   const int rc = dispatch([&](auto strict, auto cheb) {
@@ -1261,6 +1269,8 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   const int lost_rate = prm->lost_rate > 0 ? prm->lost_rate : 5;               // :141-144
   const int max_iter = prm->max_iter;
   const int mode = method_is_cheb() ? MODE_CHEBYSHEV : MODE_JACOBI;
+  // an accelerated iteration with a wrong spectral estimate diverges: the explode rules always apply to it (err bit 1)
+  const int detect_explode = prm->detect_explode || mode == MODE_CHEBYSHEV;
   if (mode == MODE_CHEBYSHEV) {
     if (prepare_cheb(prm->rho_jacobi, s)) return 1;
     cheb_rho_used = cheb_rho; cheb_gamma_used = use_two ? tl_gamma : 1.0;
@@ -1311,7 +1321,7 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   if (want_kernel == 3 || (want_kernel == 0 && resident_ok && nb <= 2)) {
     cudaEvent_t e0 = next_event(), e1 = next_event();
     XEE_CHECK(cudaEventRecord(e0, s));
-    if (solve_resident(x0, fd, prm, check_step, converge_time, lost_rate, mode, s)) return 1;
+    if (solve_resident(x0, fd, prm, check_step, converge_time, lost_rate, mode, detect_explode, s)) return 1;
     ++kernel_launches; variant_used = 3; depth_used = 1;
     XEE_CHECK(cudaEventRecord(e1, s));
     return finish(true);
@@ -1336,7 +1346,6 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
     cnt += chunk;
     XEE_CHECK(cudaEventRecord(e1, s));
     if (check) {
-      // an accelerated iteration with a wrong spectral estimate diverges: a non-finite residual always stops it (err bit 1)
       if (norm_max) {   // the residual of the iterate this check sweep read (it is still in its buffer), in the max norm
         const T* src = (cnt & 1) ? x0 : x1;
         dispatch([&](auto strict) {
@@ -1348,7 +1357,7 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
       }
       finalize_check_kernel<T><<<nb, 128, 0, s>>>(st, norm_max ? partial_max : partial, norm_max ? kResmaxBlocks : check_ntiles(),
                                                   ninterior, cnt, check_idx, converge_time, lost_rate, max_iter,
-                                                  prm->detect_explode || mode == MODE_CHEBYSHEV, prm->stall_checks, norm_max, norm_floor);
+                                                  detect_explode, prm->stall_checks, norm_max, norm_floor);
       XEE_LAUNCH_OK();
       const int slot = check_idx & 3;
       XEE_CHECK(cudaMemcpyAsync(&h_active[slot], st.active, sizeof(int), cudaMemcpyDeviceToHost, s));

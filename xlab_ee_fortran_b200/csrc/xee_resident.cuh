@@ -115,8 +115,9 @@ __global__ void __launch_bounds__(NT, 1) solve_resident_kernel(const ResArgs<T> 
   __syncthreads();
 
   // ---- replicated control state (elliptic_tools.f90:160-164)
-  int converge_cnt = 0, lose_cnt = 0, errb = 0, stall = 0, used = 0, check_idx = 0;
-  T err_before = R::huge(), err_now = T(0), ratio = T(0), best = R::huge();
+  StopRule<T> rule{R::huge(), R::huge(), 0, 0, 0, 0};
+  int used = 0, check_idx = 0;
+  T err_now = T(0), ratio = T(0);
   const T r1v = a.r1[n], r2v = a.r2[n];
   bool stop = false, aborted = false;
 
@@ -203,21 +204,12 @@ __global__ void __launch_bounds__(NT, 1) solve_resident_kernel(const ResArgs<T> 
       if (sh_abort) { aborted = true; break; }
       const double tot = sh_tot;
       err_now = R::sqrt(R::div((T)tot, (T)((nx - 2) * (ny - 2))));                 // :199
-      ratio = R::div(R::sub(err_before, err_now), err_before);                     // :201
+      stop = stop_rule_check(rule, err_now, r1v, r2v, a.converge_time, a.lost_rate, a.detect_explode, a.stall_checks, ratio);
       if (g == 0 && tid == 0 && check_idx < a.trace_cap && n == 0) { a.trace_err[check_idx] = err_now; a.trace_ratio[check_idx] = ratio; }
       ratio = R::abs(ratio);
-      if (err_before == T(0)) stop = true;                                         // :206
-      else if ((err_now < r1v) && (ratio < r2v)) { converge_cnt += 1; lose_cnt = 0; if (converge_cnt >= a.converge_time) stop = true; }
-      else if (converge_cnt > 0) { lose_cnt += 1; if (lose_cnt >= a.lost_rate) { converge_cnt -= 1; lose_cnt = 0; } }
-      if (a.detect_explode && !(err_now == err_now && R::abs(err_now) <= R::huge())) { stop = true; errb |= XEE_ERR_EXPLODE; }
-      if (a.stall_checks > 0 && !stop) {
-        if (err_now < best * T(0.999)) { best = err_now; stall = 0; }
-        else if (++stall >= a.stall_checks) { stop = true; errb |= XEE_ERR_STALLED; }
-      }
-      err_before = err_now;                                                        // :233
       ++check_idx;
     }
-    if (cnt == a.max_iter) { stop = true; errb |= XEE_ERR_OVER_MAX_ITERATION; }    // :242-244
+    if (cnt == a.max_iter) { stop = true; rule.errb |= XEE_ERR_OVER_MAX_ITERATION; }    // :242-244
     used = cnt;
     __syncthreads();                                // halo rows in place before the next sweep reads them
   }
@@ -232,7 +224,7 @@ __global__ void __launch_bounds__(NT, 1) solve_resident_kernel(const ResArgs<T> 
       of[o] = x[p]; op[o] = xprev[p];
     }
   if (g == 0 && tid == 0) {
-    a.iters[n] = used; a.errb[n] = errb | (aborted ? 0x100 : 0); a.err_now[n] = err_now; a.ratio[n] = ratio;
+    a.iters[n] = used; a.errb[n] = rule.errb | (aborted ? 0x100 : 0); a.err_now[n] = err_now; a.ratio[n] = ratio;
   }
 }
 
