@@ -56,8 +56,8 @@ void xee_do_elliptic_f64(const double* psi, const double* coe, double* outdat, c
  * hit).  Both criteria non-positive: prints the reference's message and stops the
  * process like Fortran STOP (exit status 0), elliptic_tools.f90:126-129.
  * Environment: XEE_ARITH=strict|fast (default strict: no FMA contraction, true division,
- * iterates bit-identical to the reference's operation order); XEE_METHOD=jacobi|chebyshev|line_jacobi|line_chebyshev
- * (default jacobi, the reference's iteration). */
+ * iterates bit-identical to the reference's operation order); XEE_METHOD=jacobi|chebyshev|line_jacobi|line_chebyshev|
+ * line2_jacobi|line2_chebyshev|line_bicgstab|line2_bicgstab (default jacobi, the reference's iteration). */
 void xee_solve_elliptic_f32(int* max_iter, const int* check_step, const int* converge_time, const int* lost_rate,
                             float* strategy_r1, float* strategy_r2, const float* alpha, float* dat,
                             const float* coe, const float* f, float* workspace, const int* nx, const int* ny,
@@ -124,6 +124,14 @@ void xee_cal_uw_f64(const double* rpsi, double* u, double* w, const double* ra, 
  * same discrete problem, residual and stop rule.  Shared operator, FAST arithmetic, grids of at least 34 x 34 points. */
 #define XEE_METHOD_LINE2_JACOBI 4
 #define XEE_METHOD_LINE2_CHEBYSHEV 5
+/* Right-preconditioned BiCGStab on L (not in the reference) with the block-line (LINE_) or the two-level (LINE2_)
+ * preconditioner: no spectral estimate, no assumption of a real spectrum.  iters, max_iter and check_step count iterations
+ * (two preconditioner sweeps and two operator applications each); a check computes the true residual L psi - f, feeds the
+ * unchanged stop rule and replaces the recurrence residual; a breakdown restarts the solve from its current iterate.
+ * alpha and rho_jacobi are ignored, detect_explode is always on.  Configurations as the Chebyshev counterparts: shared
+ * operator or one per solve, FAST arithmetic, sweep kernel 5; LINE2_BICGSTAB needs fp64 fields. */
+#define XEE_METHOD_LINE_BICGSTAB 6
+#define XEE_METHOD_LINE2_BICGSTAB 7
 
 typedef struct xee_plan xee_plan;
 
@@ -171,6 +179,11 @@ int xee_plan_solve_host(xee_plan* p, void* psi_host, const void* f_host, const x
  * the last sweep, or NULL.  Result left in psi_dev. */
 int xee_plan_sweeps_dev(xee_plan* p, void* psi_dev, const void* f_dev, double alpha, int sweeps, double* rms_out,
                         void* stream);
+/* Same; the BiCGStab methods run `sweeps` iterations with the residual replacements of a solve with this check_step
+ * (xee_plan_sweeps_dev: check_step 100), so that a solve stopping at iters = n returns the field of sweeps = n.  rms_out:
+ * the true residual after them.  The other methods ignore check_step. */
+int xee_plan_sweeps_checked_dev(xee_plan* p, void* psi_dev, const void* f_dev, double alpha, int sweeps, int check_step,
+                                double* rms_out, void* stream);
 /* out = L psi (interior; boundary 0) for the whole batch. */
 int xee_plan_apply_dev(xee_plan* p, const void* psi_dev, void* out_dev, void* stream);
 /* The library keeps freed field buffers (>= 1 MiB) for reuse (cap: XEE_CACHE_MB, default 16 GiB); this returns them. */

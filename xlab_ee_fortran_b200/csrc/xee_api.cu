@@ -46,7 +46,12 @@ int xee_plan_solve_host(xee_plan* p, void* psi, const void* f, const xee_solve_p
 }
 int xee_plan_sweeps_dev(xee_plan* p, void* psi, const void* f, double alpha, int sweeps, double* rms, void* stream) {
   DeviceGuard g(p->impl->d.device);
-  return p->impl->sweeps(psi, f, alpha, sweeps, rms, (cudaStream_t)stream);
+  return p->impl->sweeps(psi, f, alpha, sweeps, 0, rms, (cudaStream_t)stream);
+}
+int xee_plan_sweeps_checked_dev(xee_plan* p, void* psi, const void* f, double alpha, int sweeps, int check_step, double* rms,
+                                void* stream) {
+  DeviceGuard g(p->impl->d.device);
+  return p->impl->sweeps(psi, f, alpha, sweeps, check_step, rms, (cudaStream_t)stream);
 }
 int xee_plan_apply_dev(xee_plan* p, const void* psi, void* out, void* stream) {
   DeviceGuard g(p->impl->d.device);
@@ -95,7 +100,8 @@ PlanBase* new_plan_or_die(int dtype, int nx, int ny, int nbatch, int shared) {
   const char* me = getenv("XEE_METHOD");
   d.method = !me ? XEE_METHOD_JACOBI : !strcmp(me, "chebyshev") ? XEE_METHOD_CHEBYSHEV : !strcmp(me, "line_jacobi") ? XEE_METHOD_LINE_JACOBI
              : !strcmp(me, "line_chebyshev") ? XEE_METHOD_LINE_CHEBYSHEV : !strcmp(me, "line2_jacobi") ? XEE_METHOD_LINE2_JACOBI
-             : !strcmp(me, "line2_chebyshev") ? XEE_METHOD_LINE2_CHEBYSHEV : XEE_METHOD_JACOBI;
+             : !strcmp(me, "line2_chebyshev") ? XEE_METHOD_LINE2_CHEBYSHEV : !strcmp(me, "line_bicgstab") ? XEE_METHOD_LINE_BICGSTAB
+             : !strcmp(me, "line2_bicgstab") ? XEE_METHOD_LINE2_BICGSTAB : XEE_METHOD_JACOBI;
   PlanBase* p = nullptr;
   if (make_plan(&d, &p)) die("plan create");
   return p;

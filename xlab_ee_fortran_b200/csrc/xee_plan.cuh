@@ -19,6 +19,7 @@
 #include "xee_sweep_line.cuh"
 #include "xee_twolevel.cuh"
 #include "xee_resident.cuh"
+#include "xee_krylov.cuh"
 
 namespace xee {
 
@@ -165,7 +166,9 @@ struct PlanBase {
   virtual int set_abc(const void* a, const void* b, const void* c, double dx, double dy) = 0;
   virtual int solve(void* psi, const void* f, const xee_solve_params* prm, int* iters, double* r1o, double* r2o,
                     int* err, cudaStream_t s, bool host_io, void* workspace_host, int debug) = 0;
-  virtual int sweeps(void* psi, const void* f, double alpha, int sweeps, double* rms, cudaStream_t s) = 0;
+  // check_step: the BiCGStab methods replace the recurrence residual every check_step iterations, as a solve does (the
+  // other methods ignore it)
+  virtual int sweeps(void* psi, const void* f, double alpha, int sweeps, int check_step, double* rms, cudaStream_t s) = 0;
   virtual int apply(const void* psi, void* out, cudaStream_t s) = 0;
   virtual int coe_to_aos_host(void* coe_host) = 0;
   double sweep_ms = 0.0;
@@ -250,6 +253,13 @@ struct Plan : PlanBase {
   T *x2 = nullptr, *x3 = nullptr;
   CUtensorMap map_tb[4]{}, map_tb_f{};
   const void* map_tb_ptrs[3] = {nullptr, nullptr, nullptr};
+  // BiCGStab (XEE_METHOD_LINE*_BICGSTAB, xee_krylov.cuh): the Krylov vectors, per-(solve, tile) dot-product partials and
+  // the per-solve recurrence scalars; x1 serves as the zero field the preconditioner sweeps start from
+  bool use_krylov = false;
+  kr::Vecs<T> kv{};
+  kr::Scal ksc{};
+  double* kpart = nullptr;
+  int kcheck = 100;                  // iterations between residual replacements in the current call (its check_step)
 
   int init() {
     TraceTimer tt("plan init");
@@ -308,9 +318,10 @@ struct Plan : PlanBase {
       if (nt > ntiles) return fail("xee: internal: partial buffer too small for the TMA tiling");
     }
     // v5: segment-line relaxation is a METHOD, not a variant of the reference iteration: explicit request only.
-    use_two = d.method == XEE_METHOD_LINE2_JACOBI || d.method == XEE_METHOD_LINE2_CHEBYSHEV;
-    use_line = use_two || d.method == XEE_METHOD_LINE_JACOBI || d.method == XEE_METHOD_LINE_CHEBYSHEV;
-    if (d.method < 0 || d.method > XEE_METHOD_LINE2_CHEBYSHEV) return fail("xee: unknown method");
+    use_krylov = d.method == XEE_METHOD_LINE_BICGSTAB || d.method == XEE_METHOD_LINE2_BICGSTAB;
+    use_two = d.method == XEE_METHOD_LINE2_JACOBI || d.method == XEE_METHOD_LINE2_CHEBYSHEV || d.method == XEE_METHOD_LINE2_BICGSTAB;
+    use_line = use_two || use_krylov || d.method == XEE_METHOD_LINE_JACOBI || d.method == XEE_METHOD_LINE_CHEBYSHEV;
+    if (d.method < 0 || d.method > XEE_METHOD_LINE2_BICGSTAB) return fail("xee: unknown method");
     if (use_line) {
       if (d.arith != XEE_ARITH_FAST || !tma_ok)
         return fail("xee: the line-relaxation methods need FAST arithmetic and nx*sizeof(real) % 16 == 0");
@@ -343,6 +354,14 @@ struct Plan : PlanBase {
         XEE_CHECK(cudaMemsetAsync(tl_cv, 0, sizeof(double) * 2 * (size_t)nb * tld.pz * tld.px, own_stream));     // rim stays 0
         if (encode_map(&map_cv, tl_cv, tld.px, tld.pz, 2 * nb, 8, 3)) return 1;
       }
+      if (use_krylov) {
+        T** vecs[7] = {&kv.r, &kv.r0, &kv.p, &kv.ph, &kv.s, &kv.v, &kv.t};
+        for (T** v : vecs) XEE_CHECK(pool_alloc(v, sizeof(T) * nn * nb));
+        XEE_CHECK(pool_alloc(&kpart, sizeof(double) * kr::NP * (size_t)ntiles * nb));
+        double** sc[5] = {&ksc.rho, &ksc.alpha, &ksc.omega, &ksc.beta, &ksc.r0n};
+        for (double** v : sc) XEE_CHECK(pool_alloc(v, sizeof(double) * nb));
+        XEE_CHECK(pool_alloc(&ksc.restart, sizeof(int) * nb));
+      }
     } else if (want == 5) return fail("xee: kernel=5 is the line-relaxation kernel: select it with method = XEE_METHOD_LINE_*");
     // v4: temporal blocking.  auto: large shared-operator batches in FAST arithmetic (STRICT is bound by its true
     // divisions, where the redundant halo work of overlapping tiles costs more than the saved traffic).
@@ -370,7 +389,7 @@ struct Plan : PlanBase {
   }
   int sweep_ntiles() const { return use_line ? ln_tiles_x * ln_tiles_y : use_tma ? tma_tiles_x * tma_tiles_y : ntiles; }
   int tb_ntiles() const { return tb_tiles_x * tb_tiles_y; }
-  int check_ntiles() const { return use_tb ? tb_ntiles() : sweep_ntiles(); }   // residual partials per solve
+  int check_ntiles() const { return use_krylov ? ntiles : use_tb ? tb_ntiles() : sweep_ntiles(); }   // residual partials per solve
 
   // Solves per work unit of a persistent kernel: the chunk in [chmin, chmax] that minimises the makespan
   // cost(rounds, chunk) of the static round-robin of the units over at most num_sms CTAs (ties: the largest chunk).
@@ -446,12 +465,15 @@ struct Plan : PlanBase {
     // its buffers: apply / eta / uw return without synchronising) still touches them before they go back on the free list.
     cudaDeviceSynchronize();
     { TraceTimer t("  ~Plan: field buffers"); pool_free(coe); pool_free(linefac); pool_free(linepack); pool_free(tl_ainv); pool_free(tl_tmp); pool_free(tl_part); pool_free(tl_rc); pool_free(tl_ck); pool_free(tl_cv); pool_free(tl_scale); pool_free(tl_band); pool_free(x1); pool_free(x2); pool_free(x3); pool_free(io_psi); pool_free(io_f); pool_free(rho_dev);
-      pool_free(res_omega); pool_free(res_final); pool_free(res_prev); pool_free(res_halo); pool_free(res_ints); pool_free(res_partial); }
+      pool_free(res_omega); pool_free(res_final); pool_free(res_prev); pool_free(res_halo); pool_free(res_ints); pool_free(res_partial);
+      T* const kvecs[7] = {kv.r, kv.r0, kv.p, kv.ph, kv.s, kv.v, kv.t};
+      for (T* v : kvecs) pool_free(v); }
     { TraceTimer t("  ~Plan: small cudaFree");
       pool_free(partial); pool_free(partial_max);
       pool_free(st.done); pool_free(st.iters); pool_free(st.ccnt); pool_free(st.lcnt); pool_free(st.errb);
       pool_free(st.err_before); pool_free(st.err_now); pool_free(st.ratio); pool_free(st.r1); pool_free(st.r2);
-      pool_free(st.active); pool_free(st.trace_err); pool_free(st.trace_ratio); pool_free(st.best_err); pool_free(st.stall); }
+      pool_free(st.active); pool_free(st.trace_err); pool_free(st.trace_ratio); pool_free(st.best_err); pool_free(st.stall);
+      pool_free(kpart); pool_free(ksc.rho); pool_free(ksc.alpha); pool_free(ksc.omega); pool_free(ksc.beta); pool_free(ksc.r0n); pool_free(ksc.restart); }
     { TraceTimer t("  ~Plan: cudaFreeHost"); if (h_active) cudaFreeHost(h_active); }
     { TraceTimer t("  ~Plan: events+stream");
       for (auto& e : poll_ev) if (e) cudaEventDestroy(e);
@@ -751,6 +773,12 @@ struct Plan : PlanBase {
   // kernels ping-pong: sweep c reads x0 when c is odd, x1 when it is even.
   int run_sweeps(T* x0, const T* f, T alpha, int mode, int cnt, int k, bool check, const int* done, int& tb_pass, cudaStream_t s) {
     const int end = cnt + k;
+    if (use_krylov) {   // iterations, two preconditioner sweeps each; the residual replacements leave the check partials
+      while (cnt < end)
+        if (krylov_iteration(x0, f, ++cnt % kcheck == 0, done, s)) return 1;
+      kernel_launches += 2LL * k; sweep_launches += 2LL * k;
+      return 0;
+    }
     if (use_tb) {
       for (; cnt < end; ++tb_pass) {
         const int t = std::min(tb_depth, end - cnt);
@@ -771,6 +799,71 @@ struct Plan : PlanBase {
       kernel_launches += k;
     }
     sweep_launches += k;
+    return 0;
+  }
+
+  // ---- BiCGStab (xee_krylov.cuh)
+  kr::Args<T> krylov_args(const int* done) const {
+    kr::Args<T> a{};
+    a.coe = coe; a.coe_set_stride = d.shared_coe ? 0 : (long long)kPlanes * nn; a.nn = (long long)nn;
+    a.nx = d.nx; a.ny = d.ny; a.done = done; a.part = kpart; a.partial = partial; a.v = kv;
+    return a;
+  }
+  // ph = K^-1 v: one Jacobi-mode v5 sweep with alpha 1 from the zero field x1 (its coarse slot 0 stays zero), f = v, plus
+  // the coarse correction it leaves in slot 1
+  int krylov_precond(const T* v, const int* done, cudaStream_t s) {
+    SweepArgs<T> a = args(x1, kv.ph, v, T(1), T(1), done);
+    a.two_slot = 0;
+    if (launch_sweep_line(a, MODE_JACOBI, false, s)) return 1;
+    if (use_two) {
+      const dim3 g((((d.nx + 7) / 8) * d.ny + 255) / 256, 1, d.nbatch);
+      tl::prolong_add_kernel<T><<<g, 256, 0, s>>>(kv.ph, two_cv(1, d.nbatch), done, d.nx, d.ny, tld.px, tld.pz * tld.px);
+      XEE_LAUNCH_OK();
+    }
+    return 0;
+  }
+  int krylov_finish(int stage, const int* done, cudaStream_t s) {
+    kr::finish_kernel<<<d.nbatch, 128, 0, s>>>(ksc, kpart, ntiles, done, stage);
+    XEE_LAUNCH_OK();
+    return 0;
+  }
+  // r = f - L x; the start of a solve also sets r0 = p = r
+  int krylov_residual(const T* x, const T* f, const int* done, bool start, cudaStream_t s) {
+    kr::residual_kernel<T><<<dim3(gx, gy, d.nbatch), dim3(kr::BX, kr::BY), 0, s>>>(krylov_args(done), x, f);
+    XEE_LAUNCH_OK();
+    if (!start) return 0;
+    if (krylov_finish(kr::STAGE_START, done, s)) return 1;
+    kr::p_kernel<T><<<dim3(gx, gy, d.nbatch), dim3(kr::BX, kr::BY), 0, s>>>(krylov_args(done), ksc);
+    XEE_LAUNCH_OK();
+    return 0;
+  }
+  // Start of a solve or of sweeps(): the vectors' rims and the zero field the preconditioner starts from, then r0 = p = r.
+  int krylov_begin(const T* x, const T* f, const int* done, cudaStream_t s) {
+    T* const bufs[8] = {x1, kv.r, kv.r0, kv.p, kv.ph, kv.s, kv.v, kv.t};
+    for (T* v : bufs) XEE_CHECK(cudaMemsetAsync(v, 0, sizeof(T) * nn * d.nbatch, s));
+    if (use_two && two_reset(s)) return 1;
+    return krylov_residual(x, f, done, true, s);
+  }
+  // One iteration of every solve that is not done; `replace`: a check iteration (true residual, check partials)
+  int krylov_iteration(T* x, const T* f, bool replace, const int* done, cudaStream_t s) {
+    const dim3 g(gx, gy, d.nbatch), b(kr::BX, kr::BY);
+    const kr::Args<T> A = krylov_args(done);
+    if (krylov_precond(kv.p, done, s)) return 1;
+    kr::apply_dot_kernel<T><<<g, b, 0, s>>>(A);
+    XEE_LAUNCH_OK();
+    if (krylov_finish(kr::STAGE_ALPHA, done, s)) return 1;
+    kr::s_kernel<T><<<g, b, 0, s>>>(A, ksc, x);
+    XEE_LAUNCH_OK();
+    if (krylov_precond(kv.s, done, s)) return 1;
+    kr::t_kernel<T><<<g, b, 0, s>>>(A);
+    XEE_LAUNCH_OK();
+    if (krylov_finish(kr::STAGE_OMEGA, done, s)) return 1;
+    kr::update_kernel<T><<<g, b, 0, s>>>(A, ksc, x);
+    XEE_LAUNCH_OK();
+    if (replace && krylov_residual(x, f, done, false, s)) return 1;
+    if (krylov_finish(kr::STAGE_RHO, done, s)) return 1;
+    kr::p_kernel<T><<<g, b, 0, s>>>(A, ksc);
+    XEE_LAUNCH_OK();
     return 0;
   }
 
@@ -875,8 +968,9 @@ struct Plan : PlanBase {
     return 0;
   }
 
-  int sweeps(void* psi, const void* f, double alpha, int nsw, double* rms, cudaStream_t s) override {
+  int sweeps(void* psi, const void* f, double alpha, int nsw, int check_step, double* rms, cudaStream_t s) override {
     T* x0 = (T*)psi;
+    kcheck = check_step > 0 ? check_step : 100;
     const int mode = method_is_cheb() ? MODE_CHEBYSHEV : MODE_JACOBI;
     if (mode == MODE_CHEBYSHEV && prepare_cheb(0.0, s)) return 1;   // before the start event: the spectral probe is not sweep time
     if (seed_buffers(x0, (const T*)f, s)) return 1;
@@ -884,13 +978,19 @@ struct Plan : PlanBase {
     cudaEvent_t e0 = next_event(), e1 = next_event();
     XEE_CHECK(cudaEventRecord(e0, s));
     if (use_two && two_reset(s)) return 1;
+    if (use_krylov && krylov_begin(x0, (const T*)f, nullptr, s)) return 1;
     int tb_pass = 0;
     if (run_sweeps(x0, (const T*)f, (T)alpha, mode, 0, nsw, rms != nullptr, nullptr, tb_pass, s)) return 1;
     variant_used = use_line ? 5 : use_tb ? 4 : use_tma ? 2 : 1; depth_used = use_tb ? tb_depth : 1;
-    if (use_two && two_flush(x0, x1, d.nbatch, s)) return 1;
-    XEE_CHECK(cudaEventRecord(e1, s));
-    // the last iterate: v4 leaves it in the pair (x2, x3) after an odd number of passes, the others in x1 after an odd sweep count
-    if (use_tb ? (tb_pass & 1) : (nsw & 1)) XEE_CHECK(cudaMemcpyAsync(x0, use_tb ? x2 : x1, sizeof(T) * nn * d.nbatch, cudaMemcpyDeviceToDevice, s));
+    if (use_krylov) {   // the iterate is x0 itself; rms: the true residual after the last iteration
+      if (rms && krylov_residual(x0, (const T*)f, nullptr, false, s)) return 1;
+      XEE_CHECK(cudaEventRecord(e1, s));
+    } else {
+      if (use_two && two_flush(x0, x1, d.nbatch, s)) return 1;
+      XEE_CHECK(cudaEventRecord(e1, s));
+      // the last iterate: v4 leaves it in the pair (x2, x3) after an odd number of passes, the others in x1 after an odd sweep count
+      if (use_tb ? (tb_pass & 1) : (nsw & 1)) XEE_CHECK(cudaMemcpyAsync(x0, use_tb ? x2 : x1, sizeof(T) * nn * d.nbatch, cudaMemcpyDeviceToDevice, s));
+    }
     XEE_CHECK(cudaStreamSynchronize(s));
     harvest_events();
     if (rms && nsw > 0) {
@@ -1270,7 +1370,7 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   const int max_iter = prm->max_iter;
   const int mode = method_is_cheb() ? MODE_CHEBYSHEV : MODE_JACOBI;
   // an accelerated iteration with a wrong spectral estimate diverges: the explode rules always apply to it (err bit 1)
-  const int detect_explode = prm->detect_explode || mode == MODE_CHEBYSHEV;
+  const int detect_explode = prm->detect_explode || mode == MODE_CHEBYSHEV || use_krylov;
   if (mode == MODE_CHEBYSHEV) {
     if (prepare_cheb(prm->rho_jacobi, s)) return 1;
     cheb_rho_used = cheb_rho; cheb_gamma_used = use_two ? tl_gamma : 1.0;
@@ -1328,6 +1428,8 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   }
   if (seed_buffers(x0, fd, s)) return 1;
   if (use_two && two_reset(s)) return 1;
+  kcheck = check_step;
+  if (use_krylov && krylov_begin(x0, fd, st.done, s)) return 1;
   int tb_pass = 0;
   variant_used = use_line ? 5 : use_tb ? 4 : use_tma ? 2 : 1; depth_used = use_tb ? tb_depth : 1;
   const int ninterior = (d.nx - 2) * (d.ny - 2);
@@ -1386,6 +1488,10 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   if (!all_done) {  // max_iter exhausted (possibly on a non-check sweep)
     finalize_maxiter_kernel<T><<<(nb + 127) / 128, 128, 0, s>>>(st, nb, max_iter);
     XEE_LAUNCH_OK();
+  }
+  if (use_krylov) {   // the result is x0 itself; `workspace` receives a copy of it
+    XEE_CHECK(cudaMemcpyAsync(x1, x0, fbytes, cudaMemcpyDeviceToDevice, s));
+    return finish(false);
   }
   if (use_two && two_flush(x0, x1, nb, s)) return 1;    // psi = y + P c in both buffers (final and penultimate iterate of every solve)
   dim3 g((unsigned)std::min<size_t>((nn + 255) / 256, 64), nb);

@@ -15,8 +15,10 @@ from . import _lib
 F32, F64 = 0, 1
 ARITH_STRICT, ARITH_FAST = 0, 1
 JACOBI, CHEBYSHEV, LINE_JACOBI, LINE_CHEBYSHEV, LINE2_JACOBI, LINE2_CHEBYSHEV = 0, 1, 2, 3, 4, 5
+LINE_BICGSTAB, LINE2_BICGSTAB = 6, 7
 METHODS = {"jacobi": JACOBI, "chebyshev": CHEBYSHEV, "line_jacobi": LINE_JACOBI, "line_chebyshev": LINE_CHEBYSHEV,
-           "line2_jacobi": LINE2_JACOBI, "line2_chebyshev": LINE2_CHEBYSHEV}
+           "line2_jacobi": LINE2_JACOBI, "line2_chebyshev": LINE2_CHEBYSHEV, "line_bicgstab": LINE_BICGSTAB,
+           "line2_bicgstab": LINE2_BICGSTAB}
 
 
 class _PlanDesc(C.Structure):
@@ -145,13 +147,16 @@ class Plan:
             err.ctypes.data_as(C.c_void_p)), "solve_host")
         return dict(iters=iters, r1=r1, r2=r2, err=err)
 
-    def sweeps(self, psi, f, alpha, sweeps, want_rms=False):
-        """Exactly `sweeps` sweeps, no stop rule.  Returns the RMS residual of the last sweep per solve (or None)."""
+    def sweeps(self, psi, f, alpha, sweeps, want_rms=False, check_step=100):
+        """Exactly `sweeps` sweeps, no stop rule.  Returns the RMS residual of the last sweep per solve (or None).
+        The BiCGStab methods run `sweeps` iterations with the residual replacements of a solve with `check_step` (the
+        returned field is then that of a solve stopping at iters = sweeps) and return the true residual after them."""
         nb = self.nbatch
         rms = np.zeros(nb) if want_rms else None
-        _lib.check(_lib.lib().xee_plan_sweeps_dev(
+        _lib.check(_lib.lib().xee_plan_sweeps_checked_dev(
             self._h, self._chk(psi, (nb, self.ny, self.nx)), self._chk(f, (nb, self.ny, self.nx)), C.c_double(alpha),
-            C.c_int(sweeps), rms.ctypes.data_as(C.c_void_p) if want_rms else None, self._stream()), "sweeps_dev")
+            C.c_int(sweeps), C.c_int(check_step), rms.ctypes.data_as(C.c_void_p) if want_rms else None, self._stream()),
+            "sweeps_dev")
         return rms
 
     def apply(self, psi):
