@@ -57,7 +57,7 @@ void xee_do_elliptic_f64(const double* psi, const double* coe, double* outdat, c
  * process like Fortran STOP (exit status 0), elliptic_tools.f90:126-129.
  * Environment: XEE_ARITH=strict|fast (default strict: no FMA contraction, true division,
  * iterates bit-identical to the reference's operation order); XEE_METHOD=jacobi|chebyshev|line_jacobi|line_chebyshev|
- * line2_jacobi|line2_chebyshev|line_bicgstab|line2_bicgstab (default jacobi, the reference's iteration). */
+ * line2_jacobi|line2_chebyshev|line_bicgstab|line2_bicgstab|line2_mixed (default jacobi, the reference's iteration). */
 void xee_solve_elliptic_f32(int* max_iter, const int* check_step, const int* converge_time, const int* lost_rate,
                             float* strategy_r1, float* strategy_r2, const float* alpha, float* dat,
                             const float* coe, const float* f, float* workspace, const int* nx, const int* ny,
@@ -132,6 +132,14 @@ void xee_cal_uw_f64(const double* rpsi, double* u, double* w, const double* ra, 
  * operator or one per solve, FAST arithmetic, sweep kernel 5; LINE2_BICGSTAB needs fp64 fields. */
 #define XEE_METHOD_LINE_BICGSTAB 6
 #define XEE_METHOD_LINE2_BICGSTAB 7
+/* Mixed-precision two-level method (not in the reference): fp64 iterative refinement around fp32 two-level block-line
+ * Chebyshev sweeps.  psi, f, the residual L psi - f and the stop rule stay fp64; each refinement step solves
+ * L e = r / s approximately with check_step fp32 sweeps (the operator rounded to fp32, fp64 coarse solve, fp64 spectral
+ * estimate, s a power of two per solve) and applies psi += s e in fp64.  iters and max_iter count fp32 sweeps, and
+ * check_step is the number of sweeps per refinement step: every step ends with one check of the fp64 residual.  A solve
+ * that reaches max_iter inside a step applies the partial correction.  fp64 plans only (an fp32 plan is refused), shared
+ * operator or one per solve, FAST arithmetic, sweep kernel 5, the grids of LINE2_CHEBYSHEV with nx % 4 == 0. */
+#define XEE_METHOD_LINE2_MIXED 8
 
 typedef struct xee_plan xee_plan;
 

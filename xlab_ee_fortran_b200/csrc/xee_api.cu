@@ -101,7 +101,8 @@ PlanBase* new_plan_or_die(int dtype, int nx, int ny, int nbatch, int shared) {
   d.method = !me ? XEE_METHOD_JACOBI : !strcmp(me, "chebyshev") ? XEE_METHOD_CHEBYSHEV : !strcmp(me, "line_jacobi") ? XEE_METHOD_LINE_JACOBI
              : !strcmp(me, "line_chebyshev") ? XEE_METHOD_LINE_CHEBYSHEV : !strcmp(me, "line2_jacobi") ? XEE_METHOD_LINE2_JACOBI
              : !strcmp(me, "line2_chebyshev") ? XEE_METHOD_LINE2_CHEBYSHEV : !strcmp(me, "line_bicgstab") ? XEE_METHOD_LINE_BICGSTAB
-             : !strcmp(me, "line2_bicgstab") ? XEE_METHOD_LINE2_BICGSTAB : XEE_METHOD_JACOBI;
+             : !strcmp(me, "line2_bicgstab") ? XEE_METHOD_LINE2_BICGSTAB : !strcmp(me, "line2_mixed") ? XEE_METHOD_LINE2_MIXED
+             : XEE_METHOD_JACOBI;
   PlanBase* p = nullptr;
   if (make_plan(&d, &p)) die("plan create");
   return p;

@@ -20,6 +20,7 @@
 #include "xee_twolevel.cuh"
 #include "xee_resident.cuh"
 #include "xee_krylov.cuh"
+#include "xee_mixed.cuh"
 
 namespace xee {
 
@@ -231,10 +232,10 @@ struct Plan : PlanBase {
   unsigned char* linepack = nullptr; // operator + factors in tile/thread order
   bool linefac_ready = false;
   int ln_tiles_x = 0, ln_tiles_y = 0, ln_chunk = 1, ln_nchunks = 1;
-  struct LineMap { const void* ptr; int nb; int kind; CUtensorMap map; };
+  struct LineMap { const void* ptr; int nb; int kind; int es; CUtensorMap map; };
   std::vector<LineMap> line_maps;    // kind 0: psi box (with halo), 1: f / psi_{k-1} box, 2: 4-D store view of the result
   bool ln_tstore = false;            // results leave through TMA stores (nx a multiple of the tile width)
-  bool method_is_cheb() const { return d.method == XEE_METHOD_CHEBYSHEV || d.method == XEE_METHOD_LINE_CHEBYSHEV || d.method == XEE_METHOD_LINE2_CHEBYSHEV; }
+  bool method_is_cheb() const { return d.method == XEE_METHOD_CHEBYSHEV || d.method == XEE_METHOD_LINE_CHEBYSHEV || d.method == XEE_METHOD_LINE2_CHEBYSHEV || d.method == XEE_METHOD_LINE2_MIXED; }
   // two-level block-line methods (XEE_METHOD_LINE2_*, xee_twolevel.cuh): coarse-grid data of the operator and of a batch
   bool use_two = false;
   tl::Dims tld{};
@@ -260,6 +261,13 @@ struct Plan : PlanBase {
   kr::Scal ksc{};
   double* kpart = nullptr;
   int kcheck = 100;                  // iterations between residual replacements in the current call (its check_step)
+  // line2_mixed (xee_mixed.cuh): the fp32 operator pack, r32 [nbatch][ny][nx], the per-solve scales [2][nbatch] and a float
+  // copy of the per-solve Chebyshev radii; the fp32 pair of the Chebyshev recurrence lives in x1
+  bool use_mixed = false;
+  unsigned char* linepack32 = nullptr;
+  float *mx_r32 = nullptr, *mx_rho = nullptr;
+  double* mx_scale = nullptr;
+  std::vector<float> mx_rho_h;
 
   int init() {
     TraceTimer tt("plan init");
@@ -319,9 +327,11 @@ struct Plan : PlanBase {
     }
     // v5: segment-line relaxation is a METHOD, not a variant of the reference iteration: explicit request only.
     use_krylov = d.method == XEE_METHOD_LINE_BICGSTAB || d.method == XEE_METHOD_LINE2_BICGSTAB;
-    use_two = d.method == XEE_METHOD_LINE2_JACOBI || d.method == XEE_METHOD_LINE2_CHEBYSHEV || d.method == XEE_METHOD_LINE2_BICGSTAB;
+    use_mixed = d.method == XEE_METHOD_LINE2_MIXED;
+    use_two = d.method == XEE_METHOD_LINE2_JACOBI || d.method == XEE_METHOD_LINE2_CHEBYSHEV || d.method == XEE_METHOD_LINE2_BICGSTAB || use_mixed;
     use_line = use_two || use_krylov || d.method == XEE_METHOD_LINE_JACOBI || d.method == XEE_METHOD_LINE_CHEBYSHEV;
-    if (d.method < 0 || d.method > XEE_METHOD_LINE2_BICGSTAB) return fail("xee: unknown method");
+    if (d.method < 0 || d.method > XEE_METHOD_LINE2_MIXED) return fail("xee: unknown method");
+    if (use_mixed && sizeof(T) != 8) return fail("xee: line2_mixed returns fp64 answers from fp32 sweeps: it needs an fp64 plan");
     if (use_line) {
       if (d.arith != XEE_ARITH_FAST || !tma_ok)
         return fail("xee: the line-relaxation methods need FAST arithmetic and nx*sizeof(real) % 16 == 0");
@@ -353,6 +363,14 @@ struct Plan : PlanBase {
         XEE_CHECK(cudaMemsetAsync(tl_rc, 0, sizeof(double) * (size_t)nb * tld.ncp, own_stream));                 // padding stays 0
         XEE_CHECK(cudaMemsetAsync(tl_cv, 0, sizeof(double) * 2 * (size_t)nb * tld.pz * tld.px, own_stream));     // rim stays 0
         if (encode_map(&map_cv, tl_cv, tld.px, tld.pz, 2 * nb, 8, 3)) return 1;
+      }
+      if (use_mixed) {
+        if (((size_t)d.nx * sizeof(float)) % 16) return fail("xee: line2_mixed needs nx % 4 == 0 (rows of its fp32 fields are 16-byte multiples)");
+        XEE_CHECK(pool_alloc(&linepack32, (size_t)nt * line_pack_tile_bytes<float>() * nsets));
+        XEE_CHECK(pool_alloc(&mx_r32, sizeof(float) * nn * nb));
+        XEE_CHECK(cudaMemsetAsync(mx_r32, 0, sizeof(float) * nn * nb, own_stream));   // the rim stays 0
+        XEE_CHECK(pool_alloc(&mx_scale, sizeof(double) * 2 * nb));
+        XEE_CHECK(pool_alloc(&mx_rho, sizeof(float) * nsets));
       }
       if (use_krylov) {
         T** vecs[7] = {&kv.r, &kv.r0, &kv.p, &kv.ph, &kv.s, &kv.v, &kv.t};
@@ -389,7 +407,7 @@ struct Plan : PlanBase {
   }
   int sweep_ntiles() const { return use_line ? ln_tiles_x * ln_tiles_y : use_tma ? tma_tiles_x * tma_tiles_y : ntiles; }
   int tb_ntiles() const { return tb_tiles_x * tb_tiles_y; }
-  int check_ntiles() const { return use_krylov ? ntiles : use_tb ? tb_ntiles() : sweep_ntiles(); }   // residual partials per solve
+  int check_ntiles() const { return use_krylov || use_mixed ? ntiles : use_tb ? tb_ntiles() : sweep_ntiles(); }   // residual partials per solve
 
   // Solves per work unit of a persistent kernel: the chunk in [chmin, chmax] that minimises the makespan
   // cost(rounds, chunk) of the static round-robin of the units over at most num_sms CTAs (ties: the largest chunk).
@@ -412,8 +430,10 @@ struct Plan : PlanBase {
     return 0;
   }
 
-  // cuTensorMapEncodeTiled through the runtime (no link-time dependency on libcuda): elements of type T, no interleave, no
-  // swizzle, 128-byte L2 promotion, no out-of-bounds fill.  dims and box have `rank` entries, byte_strides rank - 1.
+  // cuTensorMapEncodeTiled through the runtime (no link-time dependency on libcuda): elements of type E (the plan's T, or
+  // float for the fp32 fields of line2_mixed), no interleave, no swizzle, 128-byte L2 promotion, no out-of-bounds fill.
+  // dims and box have `rank` entries, byte_strides rank - 1.
+  template <class E = T>
   static int encode_tiled(CUtensorMap* m, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* byte_strides,
                           const cuuint32_t* box) {
     typedef CUresult (*Fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -427,18 +447,19 @@ struct Plan : PlanBase {
       fn = (Fn)p;
     }
     const cuuint32_t es[4] = {1, 1, 1, 1};
-    const CUresult r = fn(m, sizeof(T) == 8 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, rank,
+    const CUresult r = fn(m, sizeof(E) == 8 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, rank,
                           const_cast<void*>(base), dims, byte_strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
                           CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { char b[128]; snprintf(b, sizeof b, "xee: cuTensorMapEncodeTiled (rank %d) failed (%d)", rank, (int)r); return fail(b); }
     return 0;
   }
   // a batch of nb fields [nb][ny][nx] in boxes of box_w x box_h
+  template <class E = T>
   static int encode_map(CUtensorMap* m, const void* base, int nx, int ny, int nb, int box_w, int box_h) {
     const cuuint64_t dims[3] = {(cuuint64_t)nx, (cuuint64_t)ny, (cuuint64_t)nb};
-    const cuuint64_t strides[2] = {(cuuint64_t)nx * sizeof(T), (cuuint64_t)nx * ny * sizeof(T)};
+    const cuuint64_t strides[2] = {(cuuint64_t)nx * sizeof(E), (cuuint64_t)nx * ny * sizeof(E)};
     const cuuint32_t box[3] = {(cuuint32_t)box_w, (cuuint32_t)box_h, 1};
-    return encode_tiled(m, base, 3, dims, strides, box);
+    return encode_tiled<E>(m, base, 3, dims, strides, box);
   }
   // (Re)build the tensor maps when the buffers of this call differ from the cached ones.
   int prepare_maps(const T* x0, const T* x1buf, const T* f, int nb) {
@@ -465,6 +486,7 @@ struct Plan : PlanBase {
     // its buffers: apply / eta / uw return without synchronising) still touches them before they go back on the free list.
     cudaDeviceSynchronize();
     { TraceTimer t("  ~Plan: field buffers"); pool_free(coe); pool_free(linefac); pool_free(linepack); pool_free(tl_ainv); pool_free(tl_tmp); pool_free(tl_part); pool_free(tl_rc); pool_free(tl_ck); pool_free(tl_cv); pool_free(tl_scale); pool_free(tl_band); pool_free(x1); pool_free(x2); pool_free(x3); pool_free(io_psi); pool_free(io_f); pool_free(rho_dev);
+      pool_free(linepack32); pool_free(mx_r32); pool_free(mx_scale); pool_free(mx_rho);
       pool_free(res_omega); pool_free(res_final); pool_free(res_prev); pool_free(res_halo); pool_free(res_ints); pool_free(res_partial);
       T* const kvecs[7] = {kv.r, kv.r0, kv.p, kv.ph, kv.s, kv.v, kv.t};
       for (T* v : kvecs) pool_free(v); }
@@ -520,7 +542,24 @@ struct Plan : PlanBase {
     XEE_LAUNCH_OK();
     XEE_CHECK(cudaStreamSynchronize(own_stream));
     linefac_ready = true;
+    if (use_mixed && mixed_factors()) return 1;
     return use_two ? two_setup() : 0;
+  }
+  // line2_mixed, once per operator: the operator rounded to fp32, its block-line factors computed from it in fp32, packed
+  int mixed_factors() {
+    float *c32 = nullptr, *f32 = nullptr;
+    XEE_CHECK(pool_alloc(&c32, sizeof(float) * kPlanes * nn * nsets));
+    XEE_CHECK(pool_alloc(&f32, sizeof(float) * kLineFacPlanes * nn * nsets));
+    mx::to_f32_kernel<<<1024, 256, 0, own_stream>>>(reinterpret_cast<const double*>(coe), c32, kPlanes * nn * nsets);
+    XEE_LAUNCH_OK();
+    const int nblk = (d.nx + ln::SEG * ln::BLK - 1) / (ln::SEG * ln::BLK);
+    line_factor_kernel<float><<<dim3((nblk + 31) / 32, d.ny, nsets), 32, 0, own_stream>>>(c32, f32, d.nx, d.ny);
+    XEE_LAUNCH_OK();
+    line_pack_kernel<float><<<dim3(ln_tiles_x * ln_tiles_y, nsets), ln::NT, 0, own_stream>>>(c32, f32, linepack32, d.nx, d.ny, ln_tiles_x);
+    XEE_LAUNCH_OK();
+    XEE_CHECK(cudaStreamSynchronize(own_stream));
+    pool_free(c32); pool_free(f32);
+    return 0;
   }
   // Two-level methods, once per operator: Galerkin coarse operator Ac = P^T L P and its inverse (band LU on the device).
   int two_setup() {
@@ -554,7 +593,8 @@ struct Plan : PlanBase {
   // batch, scaled by `scale` = -omega gamma, written as the coarse correction c of the NEW iterate (slot `slot`).  The fields
   // are not touched: psi = y + P c is formed by whoever reads them (the next sweep; two_flush at the end).
   double* two_cv(int slot, int nb) const { return tl_cv + (size_t)slot * nb * tld.pz * tld.px; }
-  int two_coarse(int slot, int nb, double scale, const T* rho_ps_dev, int cheb_k, const int* done, cudaStream_t s) {
+  template <class E>
+  int two_coarse(int slot, int nb, double scale, const E* rho_ps_dev, int cheb_k, const int* done, cudaStream_t s) {
     const int nt = ln_tiles_x * ln_tiles_y;
     if (d.shared_coe && nb <= 4 && !rho_ps_dev && tld.nc <= tl::kMaxNcSmem) {   // single solves, probes: one launch instead of two
       tl::coarse_gather_matvec_kernel<<<dim3((tld.nc + 7) / 8, nb), 256, 0, s>>>(tl_ainv, tl_part, two_cv(slot, d.nbatch), done, scale, nt, ln_tiles_x,
@@ -568,7 +608,7 @@ struct Plan : PlanBase {
       // one coarse operator per solve (time series), or a handful of solves (spectral probes): a matrix-vector product per solve
       const double* sps = nullptr;
       if (rho_ps_dev) {
-        tl::coarse_scale_kernel<T><<<(nb + 127) / 128, 128, 0, s>>>(rho_ps_dev, cheb_k, tl_gamma, tl_scale, nb);
+        tl::coarse_scale_kernel<E><<<(nb + 127) / 128, 128, 0, s>>>(rho_ps_dev, cheb_k, tl_gamma, tl_scale, nb);
         XEE_LAUNCH_OK();
         sps = tl_scale;
       }
@@ -650,53 +690,63 @@ struct Plan : PlanBase {
     XEE_LAUNCH_OK();
     return 0;
   }
-  // ---- v5: segment-line relaxation
+  // ---- v5: segment-line relaxation.  E: element type of the fields (the plan's T; float for the fp32 sweeps of line2_mixed)
+  template <class E = T>
   int line_map(const void* ptr, int nb, int kind, CUtensorMap* out) {
-    for (auto& m : line_maps) if (m.ptr == ptr && m.nb == nb && m.kind == kind) { *out = m.map; return 0; }
+    for (auto& m : line_maps) if (m.ptr == ptr && m.nb == nb && m.kind == kind && m.es == (int)sizeof(E)) { *out = m.map; return 0; }
     if ((uintptr_t)ptr & 15) return fail("xee: TMA path needs 16-byte aligned field buffers");
     if (line_maps.size() >= 24) line_maps.erase(line_maps.begin());
-    LineMap lm{ptr, nb, kind, {}};
+    LineMap lm{ptr, nb, kind, (int)sizeof(E), {}};
     if (kind < 2) {
-      if (encode_map(&lm.map, ptr, d.nx, d.ny, nb, kind == 0 ? ln::Cfg<T>::XW : ln::Cfg<T>::FW, kind == 0 ? ln::TH + 2 : ln::TH)) return 1;
+      if (encode_map<E>(&lm.map, ptr, d.nx, d.ny, nb, kind == 0 ? ln::Cfg<E>::XW : ln::Cfg<E>::FW, kind == 0 ? ln::TH + 2 : ln::TH)) return 1;
     } else {   // (column within a TW-wide tile column, tile column, row, solve): a [TH][FW] staging box stored at column 0
                // loses its FW - TW pad columns as out-of-bounds elements
       const cuuint64_t dims[4] = {(cuuint64_t)ln::TW, (cuuint64_t)(d.nx / ln::TW), (cuuint64_t)d.ny, (cuuint64_t)nb};
-      const cuuint64_t strides[3] = {(cuuint64_t)ln::TW * sizeof(T), (cuuint64_t)d.nx * sizeof(T), (cuuint64_t)d.nx * d.ny * sizeof(T)};
-      const cuuint32_t box[4] = {(cuuint32_t)ln::Cfg<T>::FW, 1, (cuuint32_t)ln::TH, 1};
-      if (encode_tiled(&lm.map, ptr, 4, dims, strides, box)) return 1;
+      const cuuint64_t strides[3] = {(cuuint64_t)ln::TW * sizeof(E), (cuuint64_t)d.nx * sizeof(E), (cuuint64_t)d.nx * d.ny * sizeof(E)};
+      const cuuint32_t box[4] = {(cuuint32_t)ln::Cfg<E>::FW, 1, (cuuint32_t)ln::TH, 1};
+      if (encode_tiled<E>(&lm.map, ptr, 4, dims, strides, box)) return 1;
     }
     line_maps.push_back(lm);
     *out = lm.map;
     return 0;
   }
-  template <bool CHEB, bool CHECK, bool TWO>
-  int launch_line_inst(const LineArgs<T>& A, int grid, const CUtensorMap& mx, const CUtensorMap& mxm, const CUtensorMap& mf, const CUtensorMap& mo, cudaStream_t s) {
-    constexpr int smem = TWO ? ln::Cfg<T>::SMEM_BYTES_TWO : ln::Cfg<T>::SMEM_BYTES;
+  template <class E, bool CHEB, bool CHECK, bool TWO>
+  int launch_line_inst(const LineArgs<E>& A, int grid, const CUtensorMap& mx, const CUtensorMap& mxm, const CUtensorMap& mf, const CUtensorMap& mo, cudaStream_t s) {
+    constexpr int smem = TWO ? ln::Cfg<E>::SMEM_BYTES_TWO : ln::Cfg<E>::SMEM_BYTES;
     static std::atomic<unsigned long long> attr_done{0};
-    if (opt_in_smem(sweep_line_kernel<T, CHEB, CHECK, TWO>, smem, attr_done)) return 1;
-    sweep_line_kernel<T, CHEB, CHECK, TWO><<<grid, ln::NT, smem, s>>>(A, mx, mxm, mf, mo, TWO ? map_cv : mf);
+    if (opt_in_smem(sweep_line_kernel<E, CHEB, CHECK, TWO>, smem, attr_done)) return 1;
+    sweep_line_kernel<E, CHEB, CHECK, TWO><<<grid, ln::NT, smem, s>>>(A, mx, mxm, mf, mo, TWO ? map_cv : mf);
+    return 0;
+  }
+  // Kernel arguments and tensor maps of one sweep from src to dst (dst holds the previous iterate) with right-hand side f,
+  // the operator and factors from `pack`.  The caller fills in the per-sweep weights.
+  struct LineLaunch { CUtensorMap cx, cxm, cf, co; int grid; };
+  template <class E>
+  int line_setup(const E* src, E* dst, const E* f, int nbatch, int two_slot, const int* done, const unsigned char* pack, LineArgs<E>& A, LineLaunch& L) {
+    if (!linefac_ready) return fail("xee: line relaxation: the operator has not been set");
+    if (line_map<E>(src, nbatch, 0, &L.cx) || line_map<E>(f, nbatch, 1, &L.cf) || line_map<E>(dst, nbatch, 1, &L.cxm)) return 1;
+    if (ln_tstore) { if (line_map<E>(dst, nbatch, 2, &L.co)) return 1; } else L.co = L.cxm;
+    A = LineArgs<E>{};
+    A.pack = pack; A.pack_set_stride = d.shared_coe ? 0 : (long long)(ln_tiles_x * ln_tiles_y) * (long long)line_pack_tile_bytes<E>();
+    A.dst = dst; A.field_stride = (long long)nn; A.nx = d.nx; A.ny = d.ny; A.nbatch = nbatch;
+    A.done = done; A.partial = partial;
+    A.tiles_x = ln_tiles_x; A.tiles_y = ln_tiles_y;
+    A.chunk = std::min(ln_chunk, nbatch); A.nchunks = (nbatch + A.chunk - 1) / A.chunk;
+    A.tstore = ln_tstore ? 1 : 0;
+    A.gamma = (E)(use_two ? tl_gamma : 1.0); A.cpart = tl_part;
+    // the coarse correction of `src` sits in slot two_slot, the one of the previous iterate (held by `dst`) in the other
+    // slot, which the coarse solve after this sweep overwrites with the correction of the NEW iterate; the batch index of a
+    // launch over a sub-batch (spectral probes) still strides by the plan's nbatch
+    A.cv_cur_z = two_slot * d.nbatch; A.cv_prev_z = (1 - two_slot) * d.nbatch;
+    if (use_two && !tl_ready) return fail("xee: two-level method: the operator has not been set");
+    L.grid = (int)std::min<long long>((long long)num_sms * ln::CTAS_PER_SM, (long long)ln_tiles_x * ln_tiles_y * A.nchunks);
     return 0;
   }
   int launch_sweep_line(const SweepArgs<T>& a, int mode, bool check, cudaStream_t s) {
-    if (!linefac_ready) return fail("xee: line relaxation: the operator has not been set");
-    CUtensorMap cx, cxm, cf, co;
-    if (line_map(a.src, a.nbatch, 0, &cx) || line_map(a.f, a.nbatch, 1, &cf) || line_map(a.dst, a.nbatch, 1, &cxm)) return 1;
-    if (ln_tstore) { if (line_map(a.dst, a.nbatch, 2, &co)) return 1; } else co = cxm;
-    LineArgs<T> A{};
-    A.pack = linepack; A.pack_set_stride = d.shared_coe ? 0 : (long long)(ln_tiles_x * ln_tiles_y) * (long long)line_pack_tile_bytes<T>();
-    A.dst = a.dst; A.field_stride = (long long)nn; A.nx = d.nx; A.ny = d.ny; A.nbatch = a.nbatch;
-    A.alpha = a.alpha; A.omega = a.omega; A.rho_ps = a.rho_ps; A.cheb_k = a.cheb_k; A.done = a.done; A.partial = partial;
-    A.tiles_x = ln_tiles_x; A.tiles_y = ln_tiles_y;
-    A.chunk = std::min(ln_chunk, a.nbatch); A.nchunks = (a.nbatch + A.chunk - 1) / A.chunk;
-    A.tstore = ln_tstore ? 1 : 0;
-    A.gamma = (T)(use_two ? tl_gamma : 1.0); A.cpart = tl_part;
-    // the coarse correction of `src` sits in slot a.two_slot, the one of the previous iterate (held by `dst`) in the other
-    // slot, which the coarse solve after this sweep overwrites with the correction of the NEW iterate; the batch index of a
-    // launch over a sub-batch (spectral probes) still strides by the plan's nbatch
-    A.cv_cur_z = a.two_slot * d.nbatch; A.cv_prev_z = (1 - a.two_slot) * d.nbatch;
-    if (use_two && !tl_ready) return fail("xee: two-level method: the operator has not been set");
-    const int grid = (int)std::min<long long>((long long)num_sms * ln::CTAS_PER_SM, (long long)ln_tiles_x * ln_tiles_y * A.nchunks);
-    const int rc = dispatch([&](auto cheb, auto chk, auto two) { return launch_line_inst<cheb, chk, two>(A, grid, cx, cxm, cf, co, s); },
+    LineArgs<T> A; LineLaunch L;
+    if (line_setup<T>(a.src, a.dst, a.f, a.nbatch, a.two_slot, a.done, linepack, A, L)) return 1;
+    A.alpha = a.alpha; A.omega = a.omega; A.rho_ps = a.rho_ps; A.cheb_k = a.cheb_k;
+    const int rc = dispatch([&](auto cheb, auto chk, auto two) { return launch_line_inst<T, cheb, chk, two>(A, L.grid, L.cx, L.cxm, L.cf, L.co, s); },
                             mode == MODE_CHEBYSHEV, check, use_two);
     if (rc) return rc;
     XEE_LAUNCH_OK();
@@ -773,6 +823,12 @@ struct Plan : PlanBase {
   // kernels ping-pong: sweep c reads x0 when c is odd, x1 when it is even.
   int run_sweeps(T* x0, const T* f, T alpha, int mode, int cnt, int k, bool check, const int* done, int& tb_pass, cudaStream_t s) {
     const int end = cnt + k;
+    if (use_mixed) {    // fp32 sweeps; a refinement step ends with the fold and the residual pass (the check partials)
+      while (cnt < end)
+        if (mixed_sweep((cnt++ % kcheck) + 1, done, s) || (cnt % kcheck == 0 && mixed_check(x0, f, done, s))) return 1;
+      kernel_launches += k; sweep_launches += k;
+      return 0;
+    }
     if (use_krylov) {   // iterations, two preconditioner sweeps each; the residual replacements leave the check partials
       while (cnt < end)
         if (krylov_iteration(x0, f, ++cnt % kcheck == 0, done, s)) return 1;
@@ -800,6 +856,58 @@ struct Plan : PlanBase {
     }
     sweep_launches += k;
     return 0;
+  }
+
+  // ---- line2_mixed (xee_mixed.cuh)
+  float* mixed_e(int buf) const { return reinterpret_cast<float*>(x1) + (size_t)buf * nn * d.nbatch; }
+  // fp32 sweep number k (1 .. kcheck) of the current refinement step: buffer e(b) owns coarse slot b, sweep k reads e(k & 1)
+  int mixed_sweep(int k, const int* done, cudaStream_t s) {
+    LineArgs<float> A; LineLaunch L;
+    const int slot = k & 1;
+    if (line_setup<float>(mixed_e(slot), mixed_e(slot ^ 1), mx_r32, d.nbatch, slot, done, linepack32, A, L)) return 1;
+    A.alpha = 1.f; A.omega = (float)cheb_omega_host(k, cheb_rho); A.cheb_k = k;
+    A.rho_ps = d.shared_coe ? nullptr : mx_rho;
+    if (launch_line_inst<float, true, false, true>(A, L.grid, L.cx, L.cxm, L.cf, L.co, s)) return 1;
+    XEE_LAUNCH_OK();
+    return two_coarse(slot ^ 1, d.nbatch, -(double)A.omega * tl_gamma, A.rho_ps, k, done, s);
+  }
+  // psi += s (e + P c) with the iterate of the step's last sweep (k sweeps into the step: buffer and slot (k + 1) & 1), then
+  // e = c = 0 for the next step
+  int mixed_fold(T* x0, int k, const int* done, cudaStream_t s) {
+    const dim3 g((((d.nx + 7) / 8) * d.ny + 255) / 256, 1, d.nbatch);
+    const int last = (k + 1) & 1;
+    mx::mixed_fold_kernel<<<g, 256, 0, s>>>(reinterpret_cast<double*>(x0), mixed_e(last), mixed_e(0), two_cv(last, d.nbatch), mx_scale,
+                                            done, d.nx, d.ny, d.nbatch, tld.px, tld.pz * tld.px);
+    XEE_LAUNCH_OK();
+    return two_reset(s);
+  }
+  // r = f - L psi: Sum r^2 per tile into `partial`; write_r32: also r32 = r / s' and the scales move on
+  int mixed_residual(const T* x0, const T* f, bool write_r32, const int* done, cudaStream_t s) {
+    mx::mixed_residual_kernel<<<dim3(gx, gy, d.nbatch), dim3(mx::BX, mx::BY), 0, s>>>(
+        reinterpret_cast<const double*>(x0), reinterpret_cast<const double*>(f), reinterpret_cast<const double*>(coe),
+        d.shared_coe ? 0 : (long long)kPlanes * nn, d.nx, d.ny, mx_scale + d.nbatch, write_r32 ? mx_r32 : nullptr, partial, done);
+    XEE_LAUNCH_OK();
+    if (!write_r32) return 0;
+    mx::mixed_scale_kernel<<<d.nbatch, 128, 0, s>>>(partial, ntiles, (d.nx - 2) * (d.ny - 2), mx_scale, d.nbatch, 1, done);
+    XEE_LAUNCH_OK();
+    return 0;
+  }
+  // end of a refinement step: fold, then the residual of the new iterate (the check partials) and the next step's r32
+  int mixed_check(T* x0, const T* f, const int* done, cudaStream_t s) {
+    return mixed_fold(x0, kcheck, done, s) || mixed_residual(x0, f, true, done, s);
+  }
+  // Start of a solve or of sweeps(): e = c = 0, the scale from the first guess's residual, then the first r32.
+  int mixed_begin(const T* x0, const T* f, const int* done, cudaStream_t s) {
+    XEE_CHECK(cudaMemsetAsync(x1, 0, sizeof(T) * nn * d.nbatch, s));
+    if (two_reset(s) || mixed_residual(x0, f, false, done, s)) return 1;
+    mx::mixed_scale_kernel<<<d.nbatch, 128, 0, s>>>(partial, ntiles, (d.nx - 2) * (d.ny - 2), mx_scale, d.nbatch, 0, done);
+    XEE_LAUNCH_OK();
+    if (!d.shared_coe) {   // the per-solve Chebyshev radii as the fp32 sweeps and their coarse scaling read them
+      mx_rho_h.resize(nsets);
+      for (int n = 0; n < nsets; ++n) mx_rho_h[n] = (float)rho_ps[n];
+      XEE_CHECK(cudaMemcpyAsync(mx_rho, mx_rho_h.data(), sizeof(float) * nsets, cudaMemcpyHostToDevice, s));
+    }
+    return mixed_residual(x0, f, true, done, s);
   }
 
   // ---- BiCGStab (xee_krylov.cuh)
@@ -973,16 +1081,20 @@ struct Plan : PlanBase {
     kcheck = check_step > 0 ? check_step : 100;
     const int mode = method_is_cheb() ? MODE_CHEBYSHEV : MODE_JACOBI;
     if (mode == MODE_CHEBYSHEV && prepare_cheb(0.0, s)) return 1;   // before the start event: the spectral probe is not sweep time
-    if (seed_buffers(x0, (const T*)f, s)) return 1;
+    if (!use_mixed && seed_buffers(x0, (const T*)f, s)) return 1;
     cheb_rho_used = cheb_rho; cheb_gamma_used = use_two ? tl_gamma : 1.0;
     cudaEvent_t e0 = next_event(), e1 = next_event();
     XEE_CHECK(cudaEventRecord(e0, s));
     if (use_two && two_reset(s)) return 1;
     if (use_krylov && krylov_begin(x0, (const T*)f, nullptr, s)) return 1;
+    if (use_mixed && mixed_begin(x0, (const T*)f, nullptr, s)) return 1;
     int tb_pass = 0;
     if (run_sweeps(x0, (const T*)f, (T)alpha, mode, 0, nsw, rms != nullptr, nullptr, tb_pass, s)) return 1;
     variant_used = use_line ? 5 : use_tb ? 4 : use_tma ? 2 : 1; depth_used = use_tb ? tb_depth : 1;
-    if (use_krylov) {   // the iterate is x0 itself; rms: the true residual after the last iteration
+    if (use_mixed) {    // a partial last step is applied as a solve that reaches max_iter inside a step applies it
+      if (nsw % kcheck && (mixed_fold(x0, nsw % kcheck, nullptr, s) || (rms && mixed_residual(x0, (const T*)f, false, nullptr, s)))) return 1;
+      XEE_CHECK(cudaEventRecord(e1, s));
+    } else if (use_krylov) {   // the iterate is x0 itself; rms: the true residual after the last iteration
       if (rms && krylov_residual(x0, (const T*)f, nullptr, false, s)) return 1;
       XEE_CHECK(cudaEventRecord(e1, s));
     } else {
@@ -1426,10 +1538,11 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
     XEE_CHECK(cudaEventRecord(e1, s));
     return finish(true);
   }
-  if (seed_buffers(x0, fd, s)) return 1;
+  if (!use_mixed && seed_buffers(x0, fd, s)) return 1;
   if (use_two && two_reset(s)) return 1;
   kcheck = check_step;
   if (use_krylov && krylov_begin(x0, fd, st.done, s)) return 1;
+  if (use_mixed && mixed_begin(x0, fd, st.done, s)) return 1;
   int tb_pass = 0;
   variant_used = use_line ? 5 : use_tb ? 4 : use_tma ? 2 : 1; depth_used = use_tb ? tb_depth : 1;
   const int ninterior = (d.nx - 2) * (d.ny - 2);
@@ -1486,10 +1599,11 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
     if (ev_used > 4096) { XEE_CHECK(cudaStreamSynchronize(s)); harvest_events(); }
   }
   if (!all_done) {  // max_iter exhausted (possibly on a non-check sweep)
+    if (use_mixed && cnt % check_step && mixed_fold(x0, cnt % check_step, st.done, s)) return 1;   // the partial last step
     finalize_maxiter_kernel<T><<<(nb + 127) / 128, 128, 0, s>>>(st, nb, max_iter);
     XEE_LAUNCH_OK();
   }
-  if (use_krylov) {   // the result is x0 itself; `workspace` receives a copy of it
+  if (use_krylov || use_mixed) {   // the result is x0 itself; `workspace` receives a copy of it
     XEE_CHECK(cudaMemcpyAsync(x1, x0, fbytes, cudaMemcpyDeviceToDevice, s));
     return finish(false);
   }

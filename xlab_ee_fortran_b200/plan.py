@@ -15,10 +15,10 @@ from . import _lib
 F32, F64 = 0, 1
 ARITH_STRICT, ARITH_FAST = 0, 1
 JACOBI, CHEBYSHEV, LINE_JACOBI, LINE_CHEBYSHEV, LINE2_JACOBI, LINE2_CHEBYSHEV = 0, 1, 2, 3, 4, 5
-LINE_BICGSTAB, LINE2_BICGSTAB = 6, 7
+LINE_BICGSTAB, LINE2_BICGSTAB, LINE2_MIXED = 6, 7, 8
 METHODS = {"jacobi": JACOBI, "chebyshev": CHEBYSHEV, "line_jacobi": LINE_JACOBI, "line_chebyshev": LINE_CHEBYSHEV,
            "line2_jacobi": LINE2_JACOBI, "line2_chebyshev": LINE2_CHEBYSHEV, "line_bicgstab": LINE_BICGSTAB,
-           "line2_bicgstab": LINE2_BICGSTAB}
+           "line2_bicgstab": LINE2_BICGSTAB, "line2_mixed": LINE2_MIXED}
 
 
 class _PlanDesc(C.Structure):
@@ -150,7 +150,9 @@ class Plan:
     def sweeps(self, psi, f, alpha, sweeps, want_rms=False, check_step=100):
         """Exactly `sweeps` sweeps, no stop rule.  Returns the RMS residual of the last sweep per solve (or None).
         The BiCGStab methods run `sweeps` iterations with the residual replacements of a solve with `check_step` (the
-        returned field is then that of a solve stopping at iters = sweeps) and return the true residual after them."""
+        returned field is then that of a solve stopping at iters = sweeps) and return the true residual after them.
+        line2_mixed runs `sweeps` fp32 sweeps in refinement steps of `check_step` (a partial last step is applied), the
+        field and the residual are those of a solve stopping at iters = sweeps."""
         nb = self.nbatch
         rms = np.zeros(nb) if want_rms else None
         _lib.check(_lib.lib().xee_plan_sweeps_checked_dev(
