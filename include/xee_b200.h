@@ -194,8 +194,12 @@ int xee_plan_sweeps_checked_dev(xee_plan* p, void* psi_dev, const void* f_dev, d
                                 double* rms_out, void* stream);
 /* out = L psi (interior; boundary 0) for the whole batch. */
 int xee_plan_apply_dev(xee_plan* p, const void* psi_dev, void* out_dev, void* stream);
-/* The library keeps freed field buffers (>= 1 MiB) for reuse (cap: XEE_CACHE_MB, default 16 GiB); this returns them. */
+/* The library keeps freed device buffers of every size for reuse (cap: XEE_CACHE_MB, default 16 GiB); this returns them
+ * to the driver. */
 void xee_release_cached_memory(void);
+/* Bytes of the library's device-memory pool, over all devices: held by live plans, maps and series (live_bytes), and freed
+ * but kept for reuse (cached_bytes).  Either pointer may be NULL. */
+int xee_pool_stats(long long* live_bytes, long long* cached_bytes);
 /* Kernel-launch counter (bench.py's gpu_launches): launches issued by this library since reset. */
 long long xee_launch_count(int reset);
 /* Time (ms, CUDA events on the plan's stream) spent in the dominant sweep kernel and SWEEPS it performed since reset. */

@@ -18,11 +18,12 @@ int xee_device_count(void) { int n = 0; return cudaGetDeviceCount(&n) == cudaSuc
 const char* xee_build_info(void) { return "xee_b200 sm_100a " __DATE__ " " __TIME__; }
 long long xee_launch_count(int reset) { return reset ? g_launches.exchange(0) : g_launches.load(); }
 void xee_release_cached_memory(void) { DevPool::get().trim(0); }
+int xee_pool_stats(long long* live_bytes, long long* cached_bytes) { DevPool::get().stats(live_bytes, cached_bytes); return 0; }
 
 int xee_plan_create(const xee_plan_desc* desc, xee_plan** out) {
-  PlanBase* p = nullptr;
+  std::unique_ptr<PlanBase> p;
   if (make_plan(desc, &p)) return 1;
-  *out = new xee_plan{p};
+  *out = new xee_plan{p.release()};
   return 0;
 }
 // Every plan entry point runs with the plan's device current (and restores the caller's): a process may hold plans on
@@ -80,19 +81,18 @@ namespace {
 
 template <class T> constexpr int dtype_of() { return sizeof(T) == 4 ? XEE_F32 : XEE_F64; }
 
-// Small RAII device buffer with H2D upload.
+// Small device buffer with H2D upload.
 template <class T>
 struct DevBuf {
-  T* p = nullptr; size_t n = 0;
-  explicit DevBuf(size_t n_) : n(n_) { if (pool_alloc(&p, sizeof(T) * (n ? n : 1)) != cudaSuccess) { g_last_error = "cudaMalloc"; die("DevBuf"); } }
+  PoolBuf buf; T* p = nullptr; size_t n = 0;
+  explicit DevBuf(size_t n_) : n(n_) { if (buf.alloc(&p, sizeof(T) * (n ? n : 1)) != cudaSuccess) { g_last_error = "cudaMalloc"; die("DevBuf"); } }
   // a pageable H2D cudaMemcpy may return before the DMA has landed, and the plans work on non-blocking streams that the
   // legacy default stream does not order: synchronise the device before anyone reads the buffer
   DevBuf(const T* host, size_t n_) : DevBuf(n_) { if (cudaMemcpy(p, host, sizeof(T) * n, cudaMemcpyHostToDevice) != cudaSuccess || cudaDeviceSynchronize() != cudaSuccess) { g_last_error = "H2D"; die("DevBuf"); } }
-  ~DevBuf() { pool_free(p); }
   void to_host(T* host) const { if (cudaMemcpy(host, p, sizeof(T) * n, cudaMemcpyDeviceToHost) != cudaSuccess) { g_last_error = "D2H"; die("DevBuf"); } }
 };
 
-PlanBase* new_plan_or_die(int dtype, int nx, int ny, int nbatch, int shared) {
+std::unique_ptr<PlanBase> new_plan_or_die(int dtype, int nx, int ny, int nbatch, int shared) {
   xee_plan_desc d{};
   d.dtype = dtype; d.nx = nx; d.ny = ny; d.nbatch = nbatch; d.shared_coe = shared; d.device = -1;
   const char* ar = getenv("XEE_ARITH");
@@ -103,7 +103,7 @@ PlanBase* new_plan_or_die(int dtype, int nx, int ny, int nbatch, int shared) {
              : !strcmp(me, "line2_chebyshev") ? XEE_METHOD_LINE2_CHEBYSHEV : !strcmp(me, "line_bicgstab") ? XEE_METHOD_LINE_BICGSTAB
              : !strcmp(me, "line2_bicgstab") ? XEE_METHOD_LINE2_BICGSTAB : !strcmp(me, "line2_mixed") ? XEE_METHOD_LINE2_MIXED
              : XEE_METHOD_JACOBI;
-  PlanBase* p = nullptr;
+  std::unique_ptr<PlanBase> p;
   if (make_plan(&d, &p)) die("plan create");
   return p;
 }
@@ -112,11 +112,10 @@ template <class T>
 void cal_coe_impl(const T* a, const T* b, const T* c, T* coe, const T* dx, const T* dy, const int* nx, const int* ny, int* err) {
   *err = 1;                                                   // elliptic_tools.f90:33
   const int NX = *nx, NY = *ny;
-  PlanBase* p = new_plan_or_die(dtype_of<T>(), NX, NY, 1, 1);
+  std::unique_ptr<PlanBase> p = new_plan_or_die(dtype_of<T>(), NX, NY, 1, 1);
   DevBuf<T> da(a, (size_t)(NX - 1) * (NY - 2)), db(b, (size_t)(NX - 1) * (NY - 1)), dc(c, (size_t)(NX - 2) * (NY - 1));
   if (p->set_abc(da.p, db.p, dc.p, (double)*dx, (double)*dy)) die("cal_coe");
   if (p->coe_to_aos_host(coe)) die("cal_coe");
-  delete p;
   *err = 0;                                                   // :58
 }
 
@@ -125,7 +124,7 @@ void do_elliptic_impl(const T* psi, const T* coe, T* out, const int* nx, const i
   *err = 1;                                                   // :73 (never cleared by the reference)
   const int NX = *nx, NY = *ny;
   const size_t nn = (size_t)NX * NY;
-  PlanBase* p = new_plan_or_die(dtype_of<T>(), NX, NY, 1, 1);
+  std::unique_ptr<PlanBase> p = new_plan_or_die(dtype_of<T>(), NX, NY, 1, 1);
   if (p->set_coe_aos(coe, true)) die("do_elliptic");
   DevBuf<T> dpsi(psi, nn), dout(nn);
   if (p->apply(dpsi.p, dout.p, nullptr)) die("do_elliptic");
@@ -134,7 +133,6 @@ void do_elliptic_impl(const T* psi, const T* coe, T* out, const int* nx, const i
   dout.to_host(h.data());
   for (int j = 1; j < NY - 1; ++j)    // interior only; boundary of outdat untouched (:75-76)
     memcpy(out + (size_t)j * NX + 1, h.data() + (size_t)j * NX + 1, sizeof(T) * (NX - 2));
-  delete p;
 }
 
 template <class T>
@@ -166,7 +164,7 @@ void solve_elliptic_impl(int* max_iter, const int* check_step, const int* conver
   }
   *err = 0;                                                    // :164
   if (*max_iter <= 0) { memcpy(workspace, dat, sizeof(T) * (size_t)*nx * *ny); return; }  // loop body never runs
-  PlanBase* p = new_plan_or_die(dtype_of<T>(), *nx, *ny, 1, 1);
+  std::unique_ptr<PlanBase> p = new_plan_or_die(dtype_of<T>(), *nx, *ny, 1, 1);
   if (p->set_coe_aos(coe, true)) die("solve_elliptic");
   xee_solve_params prm{};
   prm.max_iter = *max_iter; prm.check_step = *check_step; prm.converge_time = *converge_time; prm.lost_rate = *lost_rate;
@@ -178,7 +176,6 @@ void solve_elliptic_impl(int* max_iter, const int* check_step, const int* conver
   prm.stall_checks = env_int("XEE_STALL_CHECKS", 0);
   int iters = 0, e = 0; double r1o = 0, r2o = 0;
   if (p->solve(dat, f, &prm, &iters, &r1o, &r2o, &e, nullptr, true, workspace, *debug)) die("solve_elliptic");
-  delete p;
   if ((e & XEE_ERR_STALLED) && check_abs && r1o < (double)*r1) e &= ~XEE_ERR_STALLED;
   *err = e;
   if (*debug == 2) {
@@ -204,7 +201,7 @@ void solve_elliptic_old_impl(const int* max_iter, int* strategy, T* strategy_r, 
   // 100 therefore falls out of the loop with err = 0, strategy / strategy_r untouched and judge_error not called.
   const int mi = *max_iter;
   if (mi <= 0) { memcpy(workspace, dat, sizeof(T) * (size_t)*nx * *ny); return; }
-  PlanBase* p = new_plan_or_die(dtype_of<T>(), *nx, *ny, 1, 1);
+  std::unique_ptr<PlanBase> p = new_plan_or_die(dtype_of<T>(), *nx, *ny, 1, 1);
   if (p->set_coe_aos(coe, true)) die("solve_elliptic(old)");
   if (maxnorm) {
     const int NX = *nx, NY = *ny;
@@ -221,7 +218,6 @@ void solve_elliptic_old_impl(const int* max_iter, int* strategy, T* strategy_r, 
   else { prm.r1 = 0.0; prm.r2 = (double)*strategy_r; prm.converge_time = 10; prm.lost_rate = 5; if (!(prm.r2 > 0)) prm.r2 = 1e-300; }
   int iters = 0, e = 0; double r1o = 0, r2o = 0;
   if (p->solve(dat, f, &prm, &iters, &r1o, &r2o, &e, nullptr, true, workspace, *debug == 1 ? 2 : 0)) die("solve_elliptic(old)");
-  delete p;
   if ((mi % 100) != 0 && iters == mi && (e & XEE_ERR_OVER_MAX_ITERATION)) {   // fell out of the loop between two checks
     *err = e & ~XEE_ERR_OVER_MAX_ITERATION;
     return;

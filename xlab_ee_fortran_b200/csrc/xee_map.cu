@@ -27,9 +27,9 @@ struct MapBase {
 };
 
 template <class T>
-struct Map : MapBase {
-  Plan<T>* pl = nullptr;      // batched solves (shared operator)
-  Plan<T>* pl1 = nullptr;     // the single adjoint (chi) solve
+struct Map : MapBase, PoolOwner {
+  std::unique_ptr<Plan<T>> pl;      // batched solves (shared operator)
+  std::unique_ptr<Plan<T>> pl1;     // the single adjoint (chi) solve
   T *A = nullptr, *B = nullptr, *C = nullptr, *ra = nullptr, *za = nullptr, *ex = nullptr, *rho = nullptr,
     *theta = nullptr, *eta = nullptr, *chi = nullptr, *fchi = nullptr, *psi = nullptr, *f = nullptr, *r1v = nullptr;
   Heat* heat_d = nullptr;
@@ -39,7 +39,7 @@ struct Map : MapBase {
   size_t nn = 0;
   PhysK<T> k;
 
-  PlanBase* plan() override { return pl; }
+  PlanBase* plan() override { return pl.get(); }
 
   int init(const float* hA, const float* hB, const float* hC) {
     TraceTimer tt("map init (total)");
@@ -58,23 +58,24 @@ struct Map : MapBase {
     xee_plan_desc pd{};
     pd.dtype = d.dtype; pd.nx = nr; pd.ny = nz; pd.nbatch = nb; pd.shared_coe = 1; pd.arith = d.arith; pd.method = d.method;
     pd.device = d.device;
-    pl = new Plan<T>(); pl->d = pd;
+    pl.reset(new Plan<T>()); pl->d = pd;
     if (pl->init()) return 1;
     cudaStream_t s = pl->own_stream;
-    XEE_CHECK(pool_alloc(&A, sizeof(T) * nn)); XEE_CHECK(pool_alloc(&B, sizeof(T) * nn)); XEE_CHECK(pool_alloc(&C, sizeof(T) * nn));
-    XEE_CHECK(pool_alloc(&ra, sizeof(T) * nr)); XEE_CHECK(pool_alloc(&za, sizeof(T) * nz));
-    XEE_CHECK(pool_alloc(&ex, sizeof(T) * nz)); XEE_CHECK(pool_alloc(&rho, sizeof(T) * nz));
-    XEE_CHECK(pool_alloc(&theta, sizeof(T) * (nr - 1) * (nz - 1)));
-    XEE_CHECK(pool_alloc(&psi, sizeof(T) * nn * nb)); XEE_CHECK(pool_alloc(&f, sizeof(T) * nn * nb));
-    XEE_CHECK(pool_alloc(&r1v, sizeof(T) * nb));
-    XEE_CHECK(pool_alloc(&heat_d, sizeof(Heat) * nb)); XEE_CHECK(pool_alloc(&integ, sizeof(double) * 3 * nb));
+    XEE_CHECK(own(&A, sizeof(T) * nn)); XEE_CHECK(own(&B, sizeof(T) * nn)); XEE_CHECK(own(&C, sizeof(T) * nn));
+    XEE_CHECK(own(&ra, sizeof(T) * nr)); XEE_CHECK(own(&za, sizeof(T) * nz));
+    XEE_CHECK(own(&ex, sizeof(T) * nz)); XEE_CHECK(own(&rho, sizeof(T) * nz));
+    XEE_CHECK(own(&theta, sizeof(T) * (nr - 1) * (nz - 1)));
+    XEE_CHECK(own(&psi, sizeof(T) * nn * nb)); XEE_CHECK(own(&f, sizeof(T) * nn * nb));
+    XEE_CHECK(own(&r1v, sizeof(T) * nb));
+    XEE_CHECK(own(&heat_d, sizeof(Heat) * nb)); XEE_CHECK(own(&integ, sizeof(double) * 3 * nb));
     XEE_CHECK(cudaMemcpyAsync(ra, h_ra.data(), sizeof(T) * nr, cudaMemcpyHostToDevice, s));
     XEE_CHECK(cudaMemcpyAsync(za, h_za.data(), sizeof(T) * nz, cudaMemcpyHostToDevice, s));
     XEE_CHECK(cudaMemcpyAsync(ex, h_ex.data(), sizeof(T) * nz, cudaMemcpyHostToDevice, s));
     XEE_CHECK(cudaMemcpyAsync(rho, h_rho.data(), sizeof(T) * nz, cudaMemcpyHostToDevice, s));
     // inputs arrive in the reference's file format: headerless float32, i fastest (field_tools.f90:30-52)
     float* stage = nullptr;
-    XEE_CHECK(pool_alloc(&stage, sizeof(float) * nn * 3));
+    PoolBuf stage_buf;
+    XEE_CHECK(stage_buf.alloc(&stage, sizeof(float) * nn * 3));
     XEE_CHECK(cudaMemcpyAsync(stage, hA, sizeof(float) * nn, cudaMemcpyHostToDevice, s));
     XEE_CHECK(cudaMemcpyAsync(stage + nn, hB, sizeof(float) * nn, cudaMemcpyHostToDevice, s));
     XEE_CHECK(cudaMemcpyAsync(stage + 2 * nn, hC, sizeof(float) * nn, cudaMemcpyHostToDevice, s));
@@ -84,8 +85,9 @@ struct Map : MapBase {
     f32_to_T_kernel<T><<<gb, 256, 0, s>>>(stage + 2 * nn, C, nn); XEE_LAUNCH_OK();
     // K1 + K2 (cylindrical: rcuva = ra)
     T *a = nullptr, *b = nullptr, *c = nullptr;
-    XEE_CHECK(pool_alloc(&a, sizeof(T) * (nr - 1) * (nz - 2))); XEE_CHECK(pool_alloc(&b, sizeof(T) * (nr - 1) * (nz - 1)));
-    XEE_CHECK(pool_alloc(&c, sizeof(T) * (nr - 2) * (nz - 1)));
+    PoolBuf a_buf, b_buf, c_buf;
+    XEE_CHECK(a_buf.alloc(&a, sizeof(T) * (nr - 1) * (nz - 2))); XEE_CHECK(b_buf.alloc(&b, sizeof(T) * (nr - 1) * (nz - 1)));
+    XEE_CHECK(c_buf.alloc(&c, sizeof(T) * (nr - 2) * (nz - 1)));
     dim3 blk(64, 4), g((nr + 63) / 64, (nz + 3) / 4);
     build_abc_kernel<T><<<g, blk, 0, s>>>(A, B, C, ra, rho, a, b, c, nr, nz); XEE_LAUNCH_OK();
     XEE_CHECK(cudaStreamSynchronize(s));
@@ -93,22 +95,19 @@ struct Map : MapBase {
     background_theta_kernel<T><<<1, 256, 0, s>>>(A, B, theta, ra, za, nr, nz, k.g0, k.theta0); XEE_LAUNCH_OK();
     if (d.adjoint_check) {
       pd.nbatch = 1;
-      pl1 = new Plan<T>(); pl1->d = pd;
+      pl1.reset(new Plan<T>()); pl1->d = pd;
       if (pl1->init()) return 1;
       XEE_CHECK(cudaStreamSynchronize(s));
       if (pl1->set_abc(a, b, c, (double)dr, (double)dz)) return 1;
-      XEE_CHECK(pool_alloc(&eta, sizeof(T) * (nr - 1) * nz)); XEE_CHECK(pool_alloc(&chi, sizeof(T) * nn));
-      XEE_CHECK(pool_alloc(&fchi, sizeof(T) * nn));
+      XEE_CHECK(own(&eta, sizeof(T) * (nr - 1) * nz)); XEE_CHECK(own(&chi, sizeof(T) * nn));
+      XEE_CHECK(own(&fchi, sizeof(T) * nn));
     }
     XEE_CHECK(cudaStreamSynchronize(s));
-    pool_free(a); pool_free(b); pool_free(c); pool_free(stage);
     return 0;
   }
   ~Map() override {
     TraceTimer tt("map destroy");
-    delete pl; delete pl1;
-    pool_free(A); pool_free(B); pool_free(C); pool_free(ra); pool_free(za); pool_free(ex); pool_free(rho); pool_free(theta);
-    pool_free(eta); pool_free(chi); pool_free(fchi); pool_free(psi); pool_free(f); pool_free(r1v); pool_free(heat_d); pool_free(integ);
+    cudaDeviceSynchronize();   // the device is done with the owned blocks before they go back to the pool (see ~Plan)
   }
 
   // table row: iters, r1, err, sum_Q, ke_gen=(g0/theta0) I[w theta], eff=ke_gen/sum_Q, sum_Qeta, eff_eta=sum_Qeta/sum_Q
@@ -138,15 +137,14 @@ struct Map : MapBase {
       XEE_CHECK(cudaMemsetAsync(chi, 0, sizeof(T) * nn, s));
       xee_solve_params p1 = *prm_in;
       T* r1c = nullptr;
+      PoolBuf r1c_buf;
       if (d.r1_rel_rms_f > 0) {
-        XEE_CHECK(pool_alloc(&r1c, sizeof(T)));
+        XEE_CHECK(r1c_buf.alloc(&r1c, sizeof(T)));
         rms_interior_kernel<T><<<1, 256, 0, s>>>(fchi, nr, nz, (T)d.r1_rel_rms_f, r1c); XEE_LAUNCH_OK();
         p1.r1 = 1.0; p1.r1_per_solve = r1c;
       }
       int it1, e1; double a1, a2;
-      const int rc = pl1->solve(chi, fchi, &p1, &it1, &a1, &a2, &e1, s, false, nullptr, 0);
-      if (r1c) pool_free(r1c);
-      if (rc) return 1;
+      if (pl1->solve(chi, fchi, &p1, &it1, &a1, &a2, &e1, s, false, nullptr, 0)) return 1;
       dim3 ge((nr - 1 + 127) / 128, nz, 1);
       eta_kernel<T><<<ge, 128, 0, s>>>(chi, eta, ra, ra, rho, ex, nr, nz, k.g0, k.Cp, k.theta0); XEE_LAUNCH_OK();
     }
@@ -195,12 +193,12 @@ int xee_map_create(const xee_map_desc* desc, const float* A, const float* B, con
   if (resolve_device(desc->device, &dev)) return 1;
   DeviceGuard guard(dev);
   if (desc->nr < 4 || desc->nz < 4 || desc->nheat < 1) return fail("xee_map: nr, nz >= 4 and nheat >= 1 required");
-  MapBase* m = nullptr; int rc;
-  if (desc->dtype == XEE_F32) { auto* q = new Map<float>(); q->d = *desc; q->d.device = dev; rc = q->init(A, B, C); m = q; }
-  else if (desc->dtype == XEE_F64) { auto* q = new Map<double>(); q->d = *desc; q->d.device = dev; rc = q->init(A, B, C); m = q; }
+  std::unique_ptr<MapBase> m; int rc;
+  if (desc->dtype == XEE_F32) { auto* q = new Map<float>(); m.reset(q); q->d = *desc; q->d.device = dev; rc = q->init(A, B, C); }
+  else if (desc->dtype == XEE_F64) { auto* q = new Map<double>(); m.reset(q); q->d = *desc; q->d.device = dev; rc = q->init(A, B, C); }
   else return fail("xee_map: dtype must be XEE_F32 or XEE_F64");
-  if (rc) { delete m; return 1; }
-  *out = new xee_map{m};
+  if (rc) return 1;
+  *out = new xee_map{m.release()};
   return 0;
 }
 int xee_map_destroy(xee_map* m) { if (m) { DeviceGuard g(m->impl->device()); delete m->impl; delete m; } return 0; }

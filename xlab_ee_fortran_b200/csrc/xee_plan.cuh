@@ -2,12 +2,14 @@
 // solve_elliptic (xtt-lib-fortran/elliptic_tools.f90:93-265).
 // No CPU compute path exists here: without a usable CUDA device every entry point fails loudly.
 #pragma once
+#include <algorithm>
 #include <atomic>
 #include <cmath>
 #include <ctime>
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <type_traits>
@@ -110,7 +112,7 @@ struct DevPool {
   typedef std::pair<int, size_t> Key;            // (device, bytes): blocks never migrate between devices
   std::multimap<Key, void*> free_blocks;
   std::map<void*, Key> live;
-  size_t cached = 0;
+  size_t cached = 0, live_bytes = 0;
   static DevPool& get() { static DevPool p; return p; }
   cudaError_t alloc(void** out, size_t bytes) {
     int dev = 0;
@@ -119,14 +121,17 @@ struct DevPool {
     {
       std::lock_guard<std::mutex> g(mu);
       auto it = free_blocks.find(key);
-      if (it != free_blocks.end()) { *out = it->second; cached -= bytes; free_blocks.erase(it); live[*out] = key; return cudaSuccess; }
+      if (it != free_blocks.end()) {
+        *out = it->second; cached -= bytes; free_blocks.erase(it); live[*out] = key; live_bytes += bytes;
+        return cudaSuccess;
+      }
     }
     cudaError_t e = cudaMalloc(out, bytes);
     if (e != cudaSuccess) {
       cudaGetLastError();   // clear the sticky-free allocation error: the retry below may succeed and the next launch check must not see it
       trim(0); e = cudaMalloc(out, bytes);
     }
-    if (e == cudaSuccess) { std::lock_guard<std::mutex> g(mu); live[*out] = key; }
+    if (e == cudaSuccess) { std::lock_guard<std::mutex> g(mu); live[*out] = key; live_bytes += bytes; }
     return e;
   }
   void release(void* p) {
@@ -135,7 +140,7 @@ struct DevPool {
       std::lock_guard<std::mutex> g(mu);
       auto it = live.find(p);
       if (it == live.end()) { cudaFree(p); return; }
-      const Key key = it->second; live.erase(it);
+      const Key key = it->second; live.erase(it); live_bytes -= key.second;
       const size_t cap = (size_t)env_int("XEE_CACHE_MB", 16384) << 20;
       if (cached + key.second <= cap) { free_blocks.emplace(key, p); cached += key.second; return; }
     }
@@ -148,9 +153,40 @@ struct DevPool {
       cudaFree(it->second); cached -= it->first.second; free_blocks.erase(it);
     }
   }
+  void stats(long long* live_out, long long* cached_out) {
+    std::lock_guard<std::mutex> g(mu);
+    if (live_out) *live_out = (long long)live_bytes;
+    if (cached_out) *cached_out = (long long)cached;
+  }
 };
-template <class P> inline cudaError_t pool_alloc(P** out, size_t bytes) { return DevPool::get().alloc((void**)out, bytes); }
 inline void pool_free(void* p) { DevPool::get().release(p); }
+
+// The one owner of a pool block: the block goes back to the pool when the handle is destroyed.  The pool does not track
+// streams, so whoever destroys a handle makes sure the device has finished with its block.
+class PoolBuf {
+  void* p_ = nullptr;
+ public:
+  PoolBuf() = default;
+  PoolBuf(PoolBuf&& o) noexcept : p_(o.p_) { o.p_ = nullptr; }
+  ~PoolBuf() { pool_free(p_); }
+  // allocates the block of an empty handle and points *view at it (nullptr on failure)
+  template <class P> cudaError_t alloc(P** view, size_t bytes) {
+    const cudaError_t e = DevPool::get().alloc(&p_, bytes);
+    if (e != cudaSuccess) p_ = nullptr;
+    *view = (P*)p_;
+    return e;
+  }
+};
+
+// The device memory of a plan, map or series: own() allocates a block, keeps its handle and sets the raw view the kernels
+// take.  The blocks go back to the pool when the owner is destroyed, after the body of its destructor.
+struct PoolOwner {
+  std::vector<PoolBuf> owned;
+  template <class P> cudaError_t own(P** view, size_t bytes) {
+    owned.emplace_back();
+    return owned.back().alloc(view, bytes);
+  }
+};
 
 // XEE_TRACE=1: wall-clock phase timings on stderr (host side, after a device sync).
 struct TraceTimer {
@@ -200,7 +236,7 @@ struct PlanBase {
 };
 
 template <class T>
-struct Plan : PlanBase {
+struct Plan : PlanBase, PoolOwner {
   size_t nn = 0;
   int nsets = 1;
   T* coe = nullptr;       // [nsets][10][ny][nx]
@@ -274,22 +310,22 @@ struct Plan : PlanBase {
     nn = (size_t)d.nx * d.ny;
     nsets = d.shared_coe ? 1 : d.nbatch;
     XEE_CHECK(cudaStreamCreateWithFlags(&own_stream, cudaStreamNonBlocking));
-    XEE_CHECK(pool_alloc(&coe, sizeof(T) * kPlanes * nn * nsets));
+    XEE_CHECK(own(&coe, sizeof(T) * kPlanes * nn * nsets));
     // on the plan's own (non-blocking) stream: a cudaMemset on the legacy default stream is asynchronous and NOT ordered with
     // it, and could land after the operator assembly (seen under multi-process timing: a zeroed operator, NaN factors)
     XEE_CHECK(cudaMemsetAsync(coe, 0, sizeof(T) * kPlanes * nn * nsets, own_stream));
-    XEE_CHECK(pool_alloc(&x1, sizeof(T) * nn * d.nbatch));
+    XEE_CHECK(own(&x1, sizeof(T) * nn * d.nbatch));
     const int nb = d.nbatch;
-    XEE_CHECK(pool_alloc(&st.done, sizeof(int) * nb)); XEE_CHECK(pool_alloc(&st.iters, sizeof(int) * nb));
-    XEE_CHECK(pool_alloc(&st.ccnt, sizeof(int) * nb)); XEE_CHECK(pool_alloc(&st.lcnt, sizeof(int) * nb));
-    XEE_CHECK(pool_alloc(&st.errb, sizeof(int) * nb));
-    XEE_CHECK(pool_alloc(&st.err_before, sizeof(T) * nb)); XEE_CHECK(pool_alloc(&st.err_now, sizeof(T) * nb));
-    XEE_CHECK(pool_alloc(&st.ratio, sizeof(T) * nb)); XEE_CHECK(pool_alloc(&st.r1, sizeof(T) * nb));
-    XEE_CHECK(pool_alloc(&st.r2, sizeof(T) * nb)); XEE_CHECK(pool_alloc(&st.active, sizeof(int)));
-    XEE_CHECK(pool_alloc(&st.best_err, sizeof(T) * nb)); XEE_CHECK(pool_alloc(&st.stall, sizeof(int) * nb));
+    XEE_CHECK(own(&st.done, sizeof(int) * nb)); XEE_CHECK(own(&st.iters, sizeof(int) * nb));
+    XEE_CHECK(own(&st.ccnt, sizeof(int) * nb)); XEE_CHECK(own(&st.lcnt, sizeof(int) * nb));
+    XEE_CHECK(own(&st.errb, sizeof(int) * nb));
+    XEE_CHECK(own(&st.err_before, sizeof(T) * nb)); XEE_CHECK(own(&st.err_now, sizeof(T) * nb));
+    XEE_CHECK(own(&st.ratio, sizeof(T) * nb)); XEE_CHECK(own(&st.r1, sizeof(T) * nb));
+    XEE_CHECK(own(&st.r2, sizeof(T) * nb)); XEE_CHECK(own(&st.active, sizeof(int)));
+    XEE_CHECK(own(&st.best_err, sizeof(T) * nb)); XEE_CHECK(own(&st.stall, sizeof(int) * nb));
     st.trace_cap = 4096;
-    XEE_CHECK(pool_alloc(&st.trace_err, sizeof(T) * st.trace_cap));
-    XEE_CHECK(pool_alloc(&st.trace_ratio, sizeof(T) * st.trace_cap));
+    XEE_CHECK(own(&st.trace_err, sizeof(T) * st.trace_cap));
+    XEE_CHECK(own(&st.trace_ratio, sizeof(T) * st.trace_cap));
     XEE_CHECK(cudaMallocHost(&h_active, sizeof(int) * 4));
     for (auto& e : poll_ev) XEE_CHECK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     // launch geometry of the direct kernel
@@ -303,7 +339,6 @@ struct Plan : PlanBase {
       while (spb > 1 && (long long)ntiles * ((d.nbatch + spb - 1) / spb) < 148LL * 8 * 4) spb /= 2;
     }
     gz = (d.nbatch + spb - 1) / spb;
-    XEE_CHECK(pool_alloc(&partial, sizeof(double) * (size_t)ntiles * nb));
     int dev = 0;
     XEE_CHECK(cudaGetDevice(&dev));
     XEE_CHECK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
@@ -323,7 +358,6 @@ struct Plan : PlanBase {
       tma_grid = (int)std::min<long long>(num_sms, (long long)nt * tma_nchunks);
       static_assert(tma::NSTAGE_MAX >= 6, "six pipeline stages for a shared operator");
       tma_nstage = d.shared_coe ? 6 : 2;   // one operator per solve: its tiles travel with every stage, 2 x ~110 KB (fp64)
-      if (nt > ntiles) return fail("xee: internal: partial buffer too small for the TMA tiling");
     }
     // v5: segment-line relaxation is a METHOD, not a variant of the reference iteration: explicit request only.
     use_krylov = d.method == XEE_METHOD_LINE_BICGSTAB || d.method == XEE_METHOD_LINE2_BICGSTAB;
@@ -343,9 +377,8 @@ struct Plan : PlanBase {
       ln_chunk = pick_chunk(nt, std::min(4, chmax), chmax, [](long long rounds, int ch) { return rounds * (ch + 1); });
       ln_nchunks = (d.nbatch + ln_chunk - 1) / ln_chunk;
       ln_tstore = d.nx % ln::TW == 0;
-      if (grow_partial(nt)) return 1;
-      XEE_CHECK(pool_alloc(&linefac, sizeof(T) * kLineFacPlanes * nn * nsets));
-      XEE_CHECK(pool_alloc(&linepack, (size_t)nt * line_pack_tile_bytes<T>() * nsets));
+      XEE_CHECK(own(&linefac, sizeof(T) * kLineFacPlanes * nn * nsets));
+      XEE_CHECK(own(&linepack, (size_t)nt * line_pack_tile_bytes<T>() * nsets));
       want = 5;
       if (use_two) {
         static_assert(ln::TH == tl::HZ && 2 * ln::SEG == tl::HR, "the two-level restriction assumes 16-row tiles and two 8-point segments per coarse cell");
@@ -353,32 +386,32 @@ struct Plan : PlanBase {
         tld = tl::dims(d.nx, d.ny);
         if (tld.ncx < 1 || tld.ncz < 1) return fail("xee: the two-level methods need at least 18 x 18 grid points (one coarse node)");
         const size_t ab = sizeof(double) * (size_t)tld.ncp * tld.ncp * nsets;     // one coarse operator per operator set
-        XEE_CHECK(pool_alloc(&tl_ainv, ab)); XEE_CHECK(pool_alloc(&tl_tmp, ab));
-        XEE_CHECK(pool_alloc(&tl_scale, sizeof(double) * nb));
-        XEE_CHECK(pool_alloc(&tl_band, sizeof(double) * 2 * (size_t)tld.nc * (tld.ncx + 2) * nsets));
-        XEE_CHECK(pool_alloc(&tl_part, sizeof(double) * (size_t)nb * nt * 32));
-        XEE_CHECK(pool_alloc(&tl_rc, sizeof(double) * (size_t)nb * tld.ncp));
-        XEE_CHECK(pool_alloc(&tl_ck, sizeof(double) * tl::GSPLIT * (size_t)nb * tld.ncp));
-        XEE_CHECK(pool_alloc(&tl_cv, sizeof(double) * 2 * (size_t)nb * tld.pz * tld.px));
+        XEE_CHECK(own(&tl_ainv, ab)); XEE_CHECK(own(&tl_tmp, ab));
+        XEE_CHECK(own(&tl_scale, sizeof(double) * nb));
+        XEE_CHECK(own(&tl_band, sizeof(double) * 2 * (size_t)tld.nc * (tld.ncx + 2) * nsets));
+        XEE_CHECK(own(&tl_part, sizeof(double) * (size_t)nb * nt * 32));
+        XEE_CHECK(own(&tl_rc, sizeof(double) * (size_t)nb * tld.ncp));
+        XEE_CHECK(own(&tl_ck, sizeof(double) * tl::GSPLIT * (size_t)nb * tld.ncp));
+        XEE_CHECK(own(&tl_cv, sizeof(double) * 2 * (size_t)nb * tld.pz * tld.px));
         XEE_CHECK(cudaMemsetAsync(tl_rc, 0, sizeof(double) * (size_t)nb * tld.ncp, own_stream));                 // padding stays 0
         XEE_CHECK(cudaMemsetAsync(tl_cv, 0, sizeof(double) * 2 * (size_t)nb * tld.pz * tld.px, own_stream));     // rim stays 0
         if (encode_map(&map_cv, tl_cv, tld.px, tld.pz, 2 * nb, 8, 3)) return 1;
       }
       if (use_mixed) {
         if (((size_t)d.nx * sizeof(float)) % 16) return fail("xee: line2_mixed needs nx % 4 == 0 (rows of its fp32 fields are 16-byte multiples)");
-        XEE_CHECK(pool_alloc(&linepack32, (size_t)nt * line_pack_tile_bytes<float>() * nsets));
-        XEE_CHECK(pool_alloc(&mx_r32, sizeof(float) * nn * nb));
+        XEE_CHECK(own(&linepack32, (size_t)nt * line_pack_tile_bytes<float>() * nsets));
+        XEE_CHECK(own(&mx_r32, sizeof(float) * nn * nb));
         XEE_CHECK(cudaMemsetAsync(mx_r32, 0, sizeof(float) * nn * nb, own_stream));   // the rim stays 0
-        XEE_CHECK(pool_alloc(&mx_scale, sizeof(double) * 2 * nb));
-        XEE_CHECK(pool_alloc(&mx_rho, sizeof(float) * nsets));
+        XEE_CHECK(own(&mx_scale, sizeof(double) * 2 * nb));
+        XEE_CHECK(own(&mx_rho, sizeof(float) * nsets));
       }
       if (use_krylov) {
         T** vecs[7] = {&kv.r, &kv.r0, &kv.p, &kv.ph, &kv.s, &kv.v, &kv.t};
-        for (T** v : vecs) XEE_CHECK(pool_alloc(v, sizeof(T) * nn * nb));
-        XEE_CHECK(pool_alloc(&kpart, sizeof(double) * kr::NP * (size_t)ntiles * nb));
+        for (T** v : vecs) XEE_CHECK(own(v, sizeof(T) * nn * nb));
+        XEE_CHECK(own(&kpart, sizeof(double) * kr::NP * (size_t)ntiles * nb));
         double** sc[5] = {&ksc.rho, &ksc.alpha, &ksc.omega, &ksc.beta, &ksc.r0n};
-        for (double** v : sc) XEE_CHECK(pool_alloc(v, sizeof(double) * nb));
-        XEE_CHECK(pool_alloc(&ksc.restart, sizeof(int) * nb));
+        for (double** v : sc) XEE_CHECK(own(v, sizeof(double) * nb));
+        XEE_CHECK(own(&ksc.restart, sizeof(int) * nb));
       }
     } else if (want == 5) return fail("xee: kernel=5 is the line-relaxation kernel: select it with method = XEE_METHOD_LINE_*");
     // v4: temporal blocking.  auto: large shared-operator batches in FAST arithmetic (STRICT is bound by its true
@@ -399,10 +432,12 @@ struct Plan : PlanBase {
       tb_chunk = pick_chunk(nt, std::min(8, chmax), chmax, [](long long rounds, int ch) { return rounds * (ch + 2); });
       tb_nchunks = (d.nbatch + tb_chunk - 1) / tb_chunk;
       tb_grid = (int)std::min<long long>(num_sms, (long long)nt * tb_nchunks);
-      if (grow_partial(nt)) return 1;
-      XEE_CHECK(pool_alloc(&x2, sizeof(T) * nn * d.nbatch));
-      XEE_CHECK(pool_alloc(&x3, sizeof(T) * nn * d.nbatch));
+      XEE_CHECK(own(&x2, sizeof(T) * nn * d.nbatch));
+      XEE_CHECK(own(&x3, sizeof(T) * nn * d.nbatch));
     }
+    // the residual partials are per (solve, tile): room for the tiling with the most tiles
+    const int ptiles = std::max({ntiles, use_tma ? tma_tiles_x * tma_tiles_y : 0, use_line ? ln_tiles_x * ln_tiles_y : 0, use_tb ? tb_ntiles() : 0});
+    XEE_CHECK(own(&partial, sizeof(double) * (size_t)ptiles * nb));
     return 0;
   }
   int sweep_ntiles() const { return use_line ? ln_tiles_x * ln_tiles_y : use_tma ? tma_tiles_x * tma_tiles_y : ntiles; }
@@ -421,13 +456,6 @@ struct Plan : PlanBase {
       if (best < 0 || makespan < best) { best = makespan; chunk = ch; }
     }
     return chunk;
-  }
-  // the residual partials are per (solve, tile): room for a tiling with more tiles than the direct kernel's
-  int grow_partial(int nt) {
-    if (nt <= ntiles) return 0;
-    pool_free(partial); partial = nullptr;
-    XEE_CHECK(pool_alloc(&partial, sizeof(double) * (size_t)nt * d.nbatch));
-    return 0;
   }
 
   // cuTensorMapEncodeTiled through the runtime (no link-time dependency on libcuda): elements of type E (the plan's T, or
@@ -482,33 +510,23 @@ struct Plan : PlanBase {
     return 0;
   }
   ~Plan() override {
-    // The pool recycles blocks without stream tracking: make sure no kernel of this plan (or of a caller's stream that used
-    // its buffers: apply / eta / uw return without synchronising) still touches them before they go back on the free list.
+    // The pool recycles blocks without stream tracking: before the owned blocks go back on the free list (after this body),
+    // no kernel of this plan, nor of a caller's stream that used its buffers (apply / eta / uw return without
+    // synchronising), may still touch them.  ~Map and ~Series keep the same rule for their own blocks.
     cudaDeviceSynchronize();
-    { TraceTimer t("  ~Plan: field buffers"); pool_free(coe); pool_free(linefac); pool_free(linepack); pool_free(tl_ainv); pool_free(tl_tmp); pool_free(tl_part); pool_free(tl_rc); pool_free(tl_ck); pool_free(tl_cv); pool_free(tl_scale); pool_free(tl_band); pool_free(x1); pool_free(x2); pool_free(x3); pool_free(io_psi); pool_free(io_f); pool_free(rho_dev);
-      pool_free(linepack32); pool_free(mx_r32); pool_free(mx_scale); pool_free(mx_rho);
-      pool_free(res_omega); pool_free(res_final); pool_free(res_prev); pool_free(res_halo); pool_free(res_ints); pool_free(res_partial);
-      T* const kvecs[7] = {kv.r, kv.r0, kv.p, kv.ph, kv.s, kv.v, kv.t};
-      for (T* v : kvecs) pool_free(v); }
-    { TraceTimer t("  ~Plan: small cudaFree");
-      pool_free(partial); pool_free(partial_max);
-      pool_free(st.done); pool_free(st.iters); pool_free(st.ccnt); pool_free(st.lcnt); pool_free(st.errb);
-      pool_free(st.err_before); pool_free(st.err_now); pool_free(st.ratio); pool_free(st.r1); pool_free(st.r2);
-      pool_free(st.active); pool_free(st.trace_err); pool_free(st.trace_ratio); pool_free(st.best_err); pool_free(st.stall);
-      pool_free(kpart); pool_free(ksc.rho); pool_free(ksc.alpha); pool_free(ksc.omega); pool_free(ksc.beta); pool_free(ksc.r0n); pool_free(ksc.restart); }
-    { TraceTimer t("  ~Plan: cudaFreeHost"); if (h_active) cudaFreeHost(h_active); }
-    { TraceTimer t("  ~Plan: events+stream");
-      for (auto& e : poll_ev) if (e) cudaEventDestroy(e);
-      for (auto& e : ev_pool) cudaEventDestroy(e);
-      if (own_stream) cudaStreamDestroy(own_stream); }
+    if (h_active) cudaFreeHost(h_active);
+    for (auto& e : poll_ev) if (e) cudaEventDestroy(e);
+    for (auto& e : ev_pool) cudaEventDestroy(e);
+    if (own_stream) cudaStreamDestroy(own_stream);
   }
 
   int set_coe_aos(const void* src, bool on_host) override {
     const size_t bytes = sizeof(T) * 9 * nn * nsets;
     const T* dev = (const T*)src;
-    T* tmp = nullptr;
+    PoolBuf stage;
     if (on_host) {
-      XEE_CHECK(pool_alloc(&tmp, bytes));
+      T* tmp = nullptr;
+      XEE_CHECK(stage.alloc(&tmp, bytes));
       XEE_CHECK(cudaMemcpyAsync(tmp, src, bytes, cudaMemcpyHostToDevice, own_stream));
       dev = tmp;
     }
@@ -516,7 +534,6 @@ struct Plan : PlanBase {
     aos_to_planar_kernel<T><<<g, 128, 0, own_stream>>>(dev, coe, d.nx, d.ny);
     XEE_LAUNCH_OK();
     XEE_CHECK(cudaStreamSynchronize(own_stream));
-    if (tmp) pool_free(tmp);
     cheb_rho = 0.0; rho_ps.clear(); est_rho_ps.clear();
     return line_factors();
   }
@@ -548,8 +565,9 @@ struct Plan : PlanBase {
   // line2_mixed, once per operator: the operator rounded to fp32, its block-line factors computed from it in fp32, packed
   int mixed_factors() {
     float *c32 = nullptr, *f32 = nullptr;
-    XEE_CHECK(pool_alloc(&c32, sizeof(float) * kPlanes * nn * nsets));
-    XEE_CHECK(pool_alloc(&f32, sizeof(float) * kLineFacPlanes * nn * nsets));
+    PoolBuf c32_buf, f32_buf;
+    XEE_CHECK(c32_buf.alloc(&c32, sizeof(float) * kPlanes * nn * nsets));
+    XEE_CHECK(f32_buf.alloc(&f32, sizeof(float) * kLineFacPlanes * nn * nsets));
     mx::to_f32_kernel<<<1024, 256, 0, own_stream>>>(reinterpret_cast<const double*>(coe), c32, kPlanes * nn * nsets);
     XEE_LAUNCH_OK();
     const int nblk = (d.nx + ln::SEG * ln::BLK - 1) / (ln::SEG * ln::BLK);
@@ -558,7 +576,6 @@ struct Plan : PlanBase {
     line_pack_kernel<float><<<dim3(ln_tiles_x * ln_tiles_y, nsets), ln::NT, 0, own_stream>>>(c32, f32, linepack32, d.nx, d.ny, ln_tiles_x);
     XEE_LAUNCH_OK();
     XEE_CHECK(cudaStreamSynchronize(own_stream));
-    pool_free(c32); pool_free(f32);
     return 0;
   }
   // Two-level methods, once per operator: Galerkin coarse operator Ac = P^T L P and its inverse (band LU on the device).
@@ -641,14 +658,14 @@ struct Plan : PlanBase {
   int coe_to_aos_host(void* coe_host) override {  // set 0 only (Fortran-facing cal_coe)
     T* tmp = nullptr;
     const size_t bytes = sizeof(T) * 9 * nn;
-    XEE_CHECK(pool_alloc(&tmp, bytes));
+    PoolBuf tmp_buf;
+    XEE_CHECK(tmp_buf.alloc(&tmp, bytes));
     dim3 g((d.nx + 127) / 128, d.ny, 1);
     planar_to_aos_kernel<T><<<g, 128, 0, own_stream>>>(coe, tmp, d.nx, d.ny);
     XEE_LAUNCH_OK();
     std::vector<T> stage(9 * nn);
     XEE_CHECK(cudaMemcpyAsync(stage.data(), tmp, bytes, cudaMemcpyDeviceToHost, own_stream));
     XEE_CHECK(cudaStreamSynchronize(own_stream));
-    pool_free(tmp);
     // interior only: the reference never writes coe's boundary entries (elliptic_tools.f90:35-36)
     T* out = (T*)coe_host;
     for (int j = 1; j < d.ny - 1; ++j)
@@ -1036,7 +1053,7 @@ struct Plan : PlanBase {
   std::vector<double> radius_ps;     // per-set spectral radius rho (rho_ps holds the focal distance the weights are computed from)
   // Per-set Chebyshev parameters to rho_dev; h receives them in T, the values the device computes with.
   int upload_rho(const std::vector<double>& v, std::vector<T>& h, cudaStream_t s) {
-    if (!rho_dev) XEE_CHECK(pool_alloc(&rho_dev, sizeof(T) * nsets));
+    if (!rho_dev) XEE_CHECK(own(&rho_dev, sizeof(T) * nsets));
     h.resize(nsets);
     for (int n = 0; n < nsets; ++n) h[n] = (T)v[n];
     XEE_CHECK(cudaMemcpyAsync(rho_dev, h.data(), sizeof(T) * nsets, cudaMemcpyHostToDevice, s));
@@ -1138,14 +1155,15 @@ int Plan<T>::estimate_rho(cudaStream_t s) {
   //            x1 = rho_1/rho_E, xE = 1/rho_E.  Repeated until the correction is below 2 % of 1 - rho.
   const int ns = nsets;
   T *e0 = nullptr, *e1 = nullptr, *zf = nullptr; double* nrm_d = nullptr;
-  // the probe changes the launch geometry (nbatch, gz, spb): restored, and the probe buffers freed, on every exit path
+  PoolBuf e0_buf, e1_buf, zf_buf, nrm_buf;
+  // the probe changes the launch geometry (nbatch, gz, spb): restored on every exit path
   struct Restore {
-    Plan<T>* p; int nb, gz, spb; T **e0, **e1, **zf; double** nrm;
-    ~Restore() { p->d.nbatch = nb; p->gz = gz; p->spb = spb; pool_free(*e0); pool_free(*e1); pool_free(*zf); pool_free(*nrm); }
-  } restore{this, d.nbatch, gz, spb, &e0, &e1, &zf, &nrm_d};
-  XEE_CHECK(pool_alloc(&e0, sizeof(T) * nn * ns)); XEE_CHECK(pool_alloc(&e1, sizeof(T) * nn * ns));
-  XEE_CHECK(pool_alloc(&zf, sizeof(T) * nn * ns)); XEE_CHECK(pool_alloc(&nrm_d, sizeof(double) * ns * kWnormParts));
-  if (!rho_dev) XEE_CHECK(pool_alloc(&rho_dev, sizeof(T) * ns));
+    Plan<T>* p; int nb, gz, spb;
+    ~Restore() { p->d.nbatch = nb; p->gz = gz; p->spb = spb; }
+  } restore{this, d.nbatch, gz, spb};
+  XEE_CHECK(e0_buf.alloc(&e0, sizeof(T) * nn * ns)); XEE_CHECK(e1_buf.alloc(&e1, sizeof(T) * nn * ns));
+  XEE_CHECK(zf_buf.alloc(&zf, sizeof(T) * nn * ns)); XEE_CHECK(nrm_buf.alloc(&nrm_d, sizeof(double) * ns * kWnormParts));
+  if (!rho_dev) XEE_CHECK(own(&rho_dev, sizeof(T) * ns));
   XEE_CHECK(cudaMemsetAsync(zf, 0, sizeof(T) * nn * ns, s));
   auto start_vector = [&](int kind) -> int {     // e0 = e1 = start vector of `kind` (probe_start_kernel) in every set
     probe_start_kernel<T><<<dim3((unsigned)((nn + 255) / 256), ns), 256, 0, s>>>(e0, d.nx, d.ny, (long long)nn, kind);
@@ -1419,10 +1437,10 @@ int Plan<T>::solve_resident(T* x0, const T* fd, const xee_solve_params* prm, int
   const int nb = d.nbatch, G = res_G;
   const size_t fbytes = sizeof(T) * nn * nb;
   if (!res_final) {
-    XEE_CHECK(pool_alloc(&res_final, fbytes)); XEE_CHECK(pool_alloc(&res_prev, fbytes));
-    XEE_CHECK(pool_alloc(&res_halo, sizeof(T) * (size_t)nb * 2 * G * 2 * d.nx));
-    XEE_CHECK(pool_alloc(&res_ints, sizeof(int) * ((size_t)nb * G * res::FLAG_PAD + 64 * nb + 64)));
-    XEE_CHECK(pool_alloc(&res_partial, sizeof(double) * (size_t)nb * 2 * G));
+    XEE_CHECK(own(&res_final, fbytes)); XEE_CHECK(own(&res_prev, fbytes));
+    XEE_CHECK(own(&res_halo, sizeof(T) * (size_t)nb * 2 * G * 2 * d.nx));
+    XEE_CHECK(own(&res_ints, sizeof(int) * ((size_t)nb * G * res::FLAG_PAD + 64 * nb + 64)));
+    XEE_CHECK(own(&res_partial, sizeof(double) * (size_t)nb * 2 * G));
   }
   XEE_CHECK(cudaMemsetAsync(res_ints, 0, sizeof(int) * ((size_t)nb * G * res::FLAG_PAD + 64 * nb + 64), s));
   XEE_CHECK(cudaMemcpyAsync(res_final, x0, fbytes, cudaMemcpyDeviceToDevice, s));   // boundary values in both outputs
@@ -1437,7 +1455,7 @@ int Plan<T>::solve_resident(T* x0, const T* fd, const xee_solve_params* prm, int
   ra.max_iter = prm->max_iter; ra.check_step = check_step; ra.converge_time = converge_time; ra.lost_rate = lost_rate;
   ra.alpha = (T)prm->alpha; ra.rho = cheb_rho;
   if (mode == MODE_CHEBYSHEV) {   // host-computed weights, the same values the per-launch kernels receive
-    if (!res_omega) XEE_CHECK(pool_alloc(&res_omega, sizeof(T) * kChebClamp));
+    if (!res_omega) XEE_CHECK(own(&res_omega, sizeof(T) * kChebClamp));
     std::vector<T> tab(kChebClamp);
     for (int k = 1; k <= kChebClamp; ++k) tab[k - 1] = (T)cheb_omega_host(k, cheb_rho);
     XEE_CHECK(cudaMemcpyAsync(res_omega, tab.data(), sizeof(T) * kChebClamp, cudaMemcpyHostToDevice, s));
@@ -1471,7 +1489,7 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   T* x0 = (T*)psi;
   const T* fd = (const T*)f;
   if (host_io) {
-    if (!io_psi) { XEE_CHECK(pool_alloc(&io_psi, fbytes)); XEE_CHECK(pool_alloc(&io_f, fbytes)); }
+    if (!io_psi) { XEE_CHECK(own(&io_psi, fbytes)); XEE_CHECK(own(&io_f, fbytes)); }
     XEE_CHECK(cudaMemcpyAsync(io_psi, psi, fbytes, cudaMemcpyHostToDevice, s));
     XEE_CHECK(cudaMemcpyAsync(io_f, f, fbytes, cudaMemcpyHostToDevice, s));
     x0 = io_psi; fd = io_f;
@@ -1492,7 +1510,7 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   // v3: the whole loop in one cooperative launch (single / few solves that fit on the chip)
   int want_kernel = d.kernel > 0 ? d.kernel : env_int("XEE_KERNEL", 0);
   if (norm_max && (use_line || use_tb)) return fail("xee: the max-abs residual norm (legacy strategies 3/4) is provided for the point methods only");
-  if (norm_max && !partial_max) XEE_CHECK(pool_alloc(&partial_max, sizeof(double) * nb * kResmaxBlocks));
+  if (norm_max && !partial_max) XEE_CHECK(own(&partial_max, sizeof(double) * nb * kResmaxBlocks));
   const bool resident_ok = !norm_max && !use_line && (d.shared_coe || nb == 1) && max_iter >= 1 && resident_fits();
   if (want_kernel == 3 && !resident_ok) return fail("xee: kernel=3 (resident) needs a problem that fits: nbatch*strips <= SMs, <= 1536 points per strip");
   // the results: fields back to the host (host entry points), iters, err, r1 and r2 of every solve
@@ -1615,18 +1633,18 @@ int Plan<T>::solve(void* psi, const void* f, const xee_solve_params* prm, int* i
   return finish(false);
 }
 
-inline int make_plan(const xee_plan_desc* desc, PlanBase** out) {
+inline int make_plan(const xee_plan_desc* desc, std::unique_ptr<PlanBase>* out) {
   int dev = 0;
   if (resolve_device(desc->device, &dev)) return 1;
   if (desc->nx < 3 || desc->ny < 3 || desc->nbatch < 1) return fail("xee: nx, ny >= 3 and nbatch >= 1 required");
   DeviceGuard guard(dev);
-  PlanBase* p = nullptr;
+  std::unique_ptr<PlanBase> p;
   int rc;
-  if (desc->dtype == XEE_F32) { auto* q = new Plan<float>(); q->d = *desc; q->d.device = dev; rc = q->init(); p = q; }
-  else if (desc->dtype == XEE_F64) { auto* q = new Plan<double>(); q->d = *desc; q->d.device = dev; rc = q->init(); p = q; }
+  if (desc->dtype == XEE_F32) { auto* q = new Plan<float>(); p.reset(q); q->d = *desc; q->d.device = dev; rc = q->init(); }
+  else if (desc->dtype == XEE_F64) { auto* q = new Plan<double>(); p.reset(q); q->d = *desc; q->d.device = dev; rc = q->init(); }
   else return fail("xee: dtype must be XEE_F32 or XEE_F64");
-  if (rc) { delete p; return 1; }
-  *out = p;
+  if (rc) return 1;
+  *out = std::move(p);
   return 0;
 }
 

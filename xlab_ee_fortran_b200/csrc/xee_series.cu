@@ -142,15 +142,15 @@ struct SeriesBase {
 };
 
 template <class T>
-struct Series : SeriesBase {
-  Plan<T>* pl = nullptr;
+struct Series : SeriesBase, PoolOwner {
+  std::unique_ptr<Plan<T>> pl;
   T *A = nullptr, *B = nullptr, *C = nullptr, *a = nullptr, *b = nullptr, *c = nullptr, *m2 = nullptr, *theta = nullptr,
     *psi = nullptr, *f = nullptr, *u = nullptr, *w = nullptr, *r1v = nullptr, *ra = nullptr, *za = nullptr, *ex = nullptr, *rho = nullptr;
   Snap* snaps = nullptr; Heat* heat = nullptr; double* integ = nullptr; double* mx = nullptr;
   size_t nn = 0;
   T dr = 0, dz = 0;
   PhysK<T> k;
-  PlanBase* plan() override { return pl; }
+  PlanBase* plan() override { return pl.get(); }
 
   int init() {
     const int nr = d.nr, nz = d.nz, nb = d.nsnap;
@@ -165,20 +165,20 @@ struct Series : SeriesBase {
     }
     xee_plan_desc pd{};
     pd.dtype = d.dtype; pd.nx = nr; pd.ny = nz; pd.nbatch = nb; pd.shared_coe = 0; pd.arith = d.arith; pd.method = d.method; pd.device = d.device;
-    pl = new Plan<T>(); pl->d = pd;
+    pl.reset(new Plan<T>()); pl->d = pd;
     if (pl->init()) return 1;
     const size_t nB = (size_t)(nr - 1) * (nz - 1);
-    XEE_CHECK(pool_alloc(&A, sizeof(T) * nn * nb)); XEE_CHECK(pool_alloc(&B, sizeof(T) * nn * nb)); XEE_CHECK(pool_alloc(&C, sizeof(T) * nn * nb));
-    XEE_CHECK(pool_alloc(&a, sizeof(T) * (nr - 1) * (nz - 2) * nb)); XEE_CHECK(pool_alloc(&b, sizeof(T) * nB * nb));
-    XEE_CHECK(pool_alloc(&c, sizeof(T) * (nr - 2) * (nz - 1) * nb));
-    XEE_CHECK(pool_alloc(&m2, sizeof(T) * nB * nb)); XEE_CHECK(pool_alloc(&theta, sizeof(T) * nB * nb));
-    XEE_CHECK(pool_alloc(&psi, sizeof(T) * nn * nb)); XEE_CHECK(pool_alloc(&f, sizeof(T) * nn * nb));
-    XEE_CHECK(pool_alloc(&u, sizeof(T) * (size_t)nr * (nz - 1) * nb)); XEE_CHECK(pool_alloc(&w, sizeof(T) * (size_t)(nr - 1) * nz * nb));
-    XEE_CHECK(pool_alloc(&r1v, sizeof(T) * nb));
-    XEE_CHECK(pool_alloc(&ra, sizeof(T) * nr)); XEE_CHECK(pool_alloc(&za, sizeof(T) * nz));
-    XEE_CHECK(pool_alloc(&ex, sizeof(T) * nz)); XEE_CHECK(pool_alloc(&rho, sizeof(T) * nz));
-    XEE_CHECK(pool_alloc(&snaps, sizeof(Snap) * nb)); XEE_CHECK(pool_alloc(&heat, sizeof(Heat) * nb));
-    XEE_CHECK(pool_alloc(&integ, sizeof(double) * 3 * nb)); XEE_CHECK(pool_alloc(&mx, sizeof(double) * 2 * nb));
+    XEE_CHECK(own(&A, sizeof(T) * nn * nb)); XEE_CHECK(own(&B, sizeof(T) * nn * nb)); XEE_CHECK(own(&C, sizeof(T) * nn * nb));
+    XEE_CHECK(own(&a, sizeof(T) * (nr - 1) * (nz - 2) * nb)); XEE_CHECK(own(&b, sizeof(T) * nB * nb));
+    XEE_CHECK(own(&c, sizeof(T) * (nr - 2) * (nz - 1) * nb));
+    XEE_CHECK(own(&m2, sizeof(T) * nB * nb)); XEE_CHECK(own(&theta, sizeof(T) * nB * nb));
+    XEE_CHECK(own(&psi, sizeof(T) * nn * nb)); XEE_CHECK(own(&f, sizeof(T) * nn * nb));
+    XEE_CHECK(own(&u, sizeof(T) * (size_t)nr * (nz - 1) * nb)); XEE_CHECK(own(&w, sizeof(T) * (size_t)(nr - 1) * nz * nb));
+    XEE_CHECK(own(&r1v, sizeof(T) * nb));
+    XEE_CHECK(own(&ra, sizeof(T) * nr)); XEE_CHECK(own(&za, sizeof(T) * nz));
+    XEE_CHECK(own(&ex, sizeof(T) * nz)); XEE_CHECK(own(&rho, sizeof(T) * nz));
+    XEE_CHECK(own(&snaps, sizeof(Snap) * nb)); XEE_CHECK(own(&heat, sizeof(Heat) * nb));
+    XEE_CHECK(own(&integ, sizeof(double) * 3 * nb)); XEE_CHECK(own(&mx, sizeof(double) * 2 * nb));
     cudaStream_t s = pl->own_stream;
     XEE_CHECK(cudaMemcpyAsync(ra, h_ra.data(), sizeof(T) * nr, cudaMemcpyHostToDevice, s));
     XEE_CHECK(cudaMemcpyAsync(za, h_za.data(), sizeof(T) * nz, cudaMemcpyHostToDevice, s));
@@ -188,9 +188,7 @@ struct Series : SeriesBase {
     return 0;
   }
   ~Series() override {
-    delete pl;
-    void* all[] = {A, B, C, a, b, c, m2, theta, psi, f, u, w, r1v, ra, za, ex, rho, snaps, heat, integ, mx};
-    for (void* p : all) pool_free(p);
+    cudaDeviceSynchronize();   // the device is done with the owned blocks before they go back to the pool (see ~Plan)
   }
 
   // table row: iters, r1, err, sum_Q, ke_gen, efficiency, max|w|, max|u|
@@ -286,12 +284,12 @@ int xee_series_create(const xee_series_desc* desc, xee_series** out) {
   if (resolve_device(desc->device, &dev)) return 1;
   DeviceGuard guard(dev);
   if (desc->nr < 4 || desc->nz < 5 || desc->nsnap < 1) return fail("xee_series: nr >= 4, nz >= 5 and nsnap >= 1 required");
-  SeriesBase* m = nullptr; int rc;
-  if (desc->dtype == XEE_F32) { auto* q = new Series<float>(); q->d = *desc; q->d.device = dev; rc = q->init(); m = q; }
-  else if (desc->dtype == XEE_F64) { auto* q = new Series<double>(); q->d = *desc; q->d.device = dev; rc = q->init(); m = q; }
+  std::unique_ptr<SeriesBase> m; int rc;
+  if (desc->dtype == XEE_F32) { auto* q = new Series<float>(); m.reset(q); q->d = *desc; q->d.device = dev; rc = q->init(); }
+  else if (desc->dtype == XEE_F64) { auto* q = new Series<double>(); m.reset(q); q->d = *desc; q->d.device = dev; rc = q->init(); }
   else return fail("xee_series: dtype must be XEE_F32 or XEE_F64");
-  if (rc) { delete m; return 1; }
-  *out = new xee_series{m};
+  if (rc) return 1;
+  *out = new xee_series{m.release()};
   return 0;
 }
 int xee_series_destroy(xee_series* m) { if (m) { DeviceGuard g(m->impl->device()); delete m->impl; delete m; } return 0; }

@@ -190,3 +190,11 @@ class Plan:
 
 def launch_count(reset=False) -> int:
     return int(_lib.lib().xee_launch_count(C.c_int(int(reset))))
+
+
+def pool_stats():
+    """(live_bytes, cached_bytes) of the library's device-memory pool: blocks held by live plans, maps and series, and
+    freed blocks kept for reuse."""
+    live = C.c_longlong(0); cached = C.c_longlong(0)
+    _lib.check(_lib.lib().xee_pool_stats(C.byref(live), C.byref(cached)), "pool_stats")
+    return live.value, cached.value
