@@ -245,8 +245,22 @@ int xee_map_destroy(xee_map* m);
 /* heat: [nheat][5] doubles {r_c, z_c, sigma_r, sigma_z, Q0}; table: [nheat][XEE_MAP_COLS] doubles. */
 int xee_map_run_host(xee_map* m, const double* heat_host, const xee_solve_params* prm, double* table_host);
 int xee_map_run_dev(xee_map* m, const double* heat_dev, const xee_solve_params* prm, double* table_dev, void* stream);
-/* which: 0 psi [nheat][nz][nr], 1 f, 2 theta_B [(nz-1)][(nr-1)], 3 eta [nz][nr-1], 4 chi.  Plan dtype, HOST out. */
+/* which: 0 psi [nheat][nz][nr], 1 f, 2 theta_B [(nz-1)][(nr-1)], 3 eta [nz][nr-1], 4 chi,
+ * 5 eta_d [(nz-1)][(nr-1)] and 6 lambda [nz][nr] of the last xee_map_adjoint_solve.  Plan dtype, HOST out. */
 int xee_map_get_field(xee_map* m, int which, void* host_out);
+/* Discrete adjoint.  ke_gen of a heating Q is <g, L^-1 H Q> = <mu, Q> with mu = H^T lambda and L^T lambda = g, g the
+ * gradient of ke_gen in psi and H the map Q -> f: one solve gives the exact discrete efficiency sum(mu Q) / sum(W Q) of any
+ * heating, equal to column 5 of the table to solver tolerance (efficiency_eta, column 7, is the continuous adjoint's, first
+ * order in the grid spacing).  eta_d = mu / W is the efficiency of heating concentrated in one B cell.
+ * adjoint_solve: L^T lambda = g from lambda = 0 with the map's dtype, arithmetic and method; r1 = r1_rel_rms_f * rms(g) when
+ * r1_rel_rms_f > 0, else prm->r1.  Leaves lambda, mu and eta_d on the device.
+ * adjoint_eval_host: heat [n][5] as for run, any n >= 1; table [n][XEE_ADJ_COLS] doubles.  Fails before an adjoint solve.
+ * adjoint_timings: host wall time of the first call's setup (plan, L^T, line factors, coarse operator), of the spectral
+ * probes and of the sweep kernels of the adjoint plan, in ms, summed over its calls. */
+#define XEE_ADJ_COLS 3 /* sum_Q, ke_gen (scaled by g0/theta0 like table column 4), efficiency */
+int xee_map_adjoint_solve(xee_map* m, const xee_solve_params* prm, int* iters, double* r1_out, int* err);
+int xee_map_adjoint_eval_host(xee_map* m, const double* heat_host, int n, double* table_host);
+int xee_map_adjoint_timings(xee_map* m, double* setup_ms, double* probe_ms, double* sweep_ms);
 int xee_map_sweep_kernel_stats(xee_map* m, double* ms_total, long long* sweeps, int reset);
 int xee_map_kernel_info(xee_map* m, int* variant, int* sweeps_per_pass, long long* kernel_launches);
 

@@ -9,10 +9,12 @@
 //   K3/K4 batched solve         elliptic_tools.f90:93-265
 //   K6 ke_generation_kernel     old-diagnose/diagnose.f90:915-941 (w), :1117-1127 (w theta), :1094-1113 (integral)
 //      sum_q_kernel             :1050-1071      qeta_kernel  :1073-1092 (adjoint check through eta)
+//   discrete adjoint            xee_adjoint_kernels.cuh: one solve of L^T lambda = g, then the exact efficiency of any
+//                               number of heating distributions as weighted sums (adjoint_solve, adjoint_eval)
 //
 // The legacy driver's latent bugs are not reproduced; the intended maths is (SURVEY section 7):
 // Q is a genuine B-grid (nr-1,nz-1) field, theta is the background state (testing_dt = 0).
-#include "xee_map_kernels.cuh"
+#include "xee_adjoint_kernels.cuh"
 
 namespace xee {
 
@@ -24,12 +26,19 @@ struct MapBase {
                   cudaStream_t s) = 0;
   virtual PlanBase* plan() = 0;
   virtual int get_field(int which, void* host_out) = 0;
+  virtual int adjoint_solve(const xee_solve_params* prm, int* iters, double* r1, int* err) = 0;
+  virtual int adjoint_eval(const double* heat_host, int n, double* table_host) = 0;
+  virtual int adjoint_timings(double* setup_ms, double* probe_ms, double* sweep_ms) = 0;
 };
 
 template <class T>
 struct Map : MapBase, PoolOwner {
   std::unique_ptr<Plan<T>> pl;      // batched solves (shared operator)
   std::unique_ptr<Plan<T>> pl1;     // the single adjoint (chi) solve
+  std::unique_ptr<Plan<T>> pla;     // the discrete adjoint: L^T, made by the first adjoint_solve
+  T *adj_g = nullptr, *adj_lam = nullptr, *adj_mu = nullptr, *adj_eta = nullptr, *adj_r1 = nullptr;
+  bool adj_ready = false;           // lambda, mu and eta_d hold the result of an adjoint solve
+  double adj_setup_ms = 0.0;
   T *A = nullptr, *B = nullptr, *C = nullptr, *ra = nullptr, *za = nullptr, *ex = nullptr, *rho = nullptr,
     *theta = nullptr, *eta = nullptr, *chi = nullptr, *fchi = nullptr, *psi = nullptr, *f = nullptr, *r1v = nullptr;
   Heat* heat_d = nullptr;
@@ -174,10 +183,90 @@ struct Map : MapBase, PoolOwner {
       case 2: src = theta; bytes = sizeof(T) * (nr - 1) * (nz - 1); break;
       case 3: src = eta; bytes = sizeof(T) * (nr - 1) * nz; break;
       case 4: src = chi; bytes = sizeof(T) * nn; break;
+      case 5: src = adj_ready ? adj_eta : nullptr; bytes = sizeof(T) * (nr - 1) * (nz - 1); break;
+      case 6: src = adj_ready ? adj_lam : nullptr; bytes = sizeof(T) * nn; break;
       default: return fail("xee_map_get_field: unknown field");
     }
-    if (!src) return fail("xee_map_get_field: field not computed (adjoint_check off?)");
+    if (!src) return fail(which >= 5 ? "xee_map_get_field: field not computed (no xee_map_adjoint_solve yet)"
+                                     : "xee_map_get_field: field not computed (adjoint_check off?)");
     XEE_CHECK(cudaMemcpy(out, src, bytes, cudaMemcpyDeviceToHost));
+    return 0;
+  }
+
+  // Discrete adjoint (xee_adjoint_kernels.cuh).  The first call makes a single-solve plan of the map's dtype, arithmetic and
+  // method and writes L^T into it; its line factors, coarse operator and spectral estimate are then those of L^T.
+  int adjoint_setup() {
+    const double t0 = TraceTimer::now();
+    const int nr = d.nr, nz = d.nz;
+    xee_plan_desc pd = pl->d;
+    pd.nbatch = 1;
+    std::unique_ptr<Plan<T>> p(new Plan<T>()); p->d = pd;
+    if (p->init()) return 1;
+    cudaStream_t s = p->own_stream;
+    XEE_CHECK(own(&adj_g, sizeof(T) * nn)); XEE_CHECK(own(&adj_lam, sizeof(T) * nn));
+    XEE_CHECK(own(&adj_mu, sizeof(T) * (nr - 1) * (nz - 1))); XEE_CHECK(own(&adj_eta, sizeof(T) * (nr - 1) * (nz - 1)));
+    XEE_CHECK(own(&adj_r1, sizeof(T)));
+    XEE_CHECK(cudaStreamSynchronize(pl->own_stream));   // L is complete
+    transpose_coe_kernel<T><<<dim3((nr + 127) / 128, nz), 128, 0, s>>>(pl->coe, p->coe, nr, nz); XEE_LAUNCH_OK();
+    if (p->operator_written()) return 1;
+    ke_functional_kernel<T><<<dim3((nr + 127) / 128, nz), 128, 0, s>>>(theta, ra, za, rho, nr, nz, k.g0, k.theta0, adj_g);
+    XEE_LAUNCH_OK();
+    XEE_CHECK(cudaStreamSynchronize(s));
+    pla = std::move(p);
+    adj_setup_ms = (TraceTimer::now() - t0) * 1e3;
+    return 0;
+  }
+  // L^T lambda = g from lambda = 0, with the tolerance rule of the chi solve; then mu = H^T lambda and eta_d = mu / W.
+  int adjoint_solve(const xee_solve_params* prm_in, int* iters, double* r1, int* err) override {
+    TraceTimer tt("map adjoint solve");
+    const int nr = d.nr, nz = d.nz;
+    if (!pla && adjoint_setup()) return 1;
+    cudaStream_t s = pla->own_stream;
+    adj_ready = false;
+    XEE_CHECK(cudaMemsetAsync(adj_lam, 0, sizeof(T) * nn, s));
+    xee_solve_params p = *prm_in;
+    if (d.r1_rel_rms_f > 0) {
+      rms_interior_kernel<T><<<1, 256, 0, s>>>(adj_g, nr, nz, (T)d.r1_rel_rms_f, adj_r1); XEE_LAUNCH_OK();
+      p.r1 = 1.0; p.r1_per_solve = adj_r1;
+    }
+    int it = 0, e = 0; double a1 = 0, a2 = 0;
+    if (pla->solve(adj_lam, adj_g, &p, &it, &a1, &a2, &e, s, false, nullptr, 0)) return 1;
+    heating_adjoint_kernel<T><<<dim3((nr - 1 + 127) / 128, nz - 1), 128, 0, s>>>(adj_lam, ra, za, ex, rho, nr, nz, k.g0, k.theta0,
+                                                                                k.Cp, adj_mu, adj_eta);
+    XEE_LAUNCH_OK();
+    XEE_CHECK(cudaStreamSynchronize(s));
+    adj_ready = true;
+    if (iters) *iters = it;
+    if (r1) *r1 = a1;
+    if (err) *err = e;
+    return 0;
+  }
+  // rows [n][XEE_ADJ_COLS]: sum_Q, ke_gen = sum mu Q (g0/theta0 is in mu), efficiency.  XEE_ADJ_FULL_SUM=1 sums over every
+  // cell instead of the cells a heating blob can reach (the same bits; the switch exists to show that).
+  int adjoint_eval(const double* heat_host, int n, double* table) override {
+    if (!adj_ready) return fail("xee_map_adjoint_eval: no adjoint field: call xee_map_adjoint_solve first");
+    if (n < 1) return fail("xee_map_adjoint_eval: n >= 1 heating rows required");
+    cudaStream_t s = pla->own_stream;
+    Heat* hd = nullptr; double* sums = nullptr;
+    PoolBuf hd_buf, sums_buf;
+    XEE_CHECK(hd_buf.alloc(&hd, sizeof(Heat) * (size_t)n)); XEE_CHECK(sums_buf.alloc(&sums, sizeof(double) * 2 * (size_t)n));
+    XEE_CHECK(cudaMemcpyAsync(hd, heat_host, sizeof(Heat) * (size_t)n, cudaMemcpyHostToDevice, s));
+    adjoint_eval_kernel<T><<<n, 256, 0, s>>>(hd, adj_mu, ra, za, rho, d.nr, d.nz, env_int("XEE_ADJ_FULL_SUM", 0) ? 0 : 1, sums);
+    XEE_LAUNCH_OK();
+    std::vector<double> h(2 * (size_t)n);
+    XEE_CHECK(cudaMemcpyAsync(h.data(), sums, sizeof(double) * h.size(), cudaMemcpyDeviceToHost, s));
+    XEE_CHECK(cudaStreamSynchronize(s));
+    for (size_t q = 0; q < (size_t)n; ++q) {
+      double* r = table + q * XEE_ADJ_COLS;
+      r[0] = h[2 * q]; r[1] = h[2 * q + 1]; r[2] = r[1] / r[0];
+    }
+    return 0;
+  }
+  int adjoint_timings(double* setup_ms, double* probe_ms, double* sweep_ms) override {
+    if (!pla) return fail("xee_map_adjoint_timings: no adjoint solve yet");
+    if (setup_ms) *setup_ms = adj_setup_ms;
+    if (probe_ms) *probe_ms = pla->probe_ms;
+    if (sweep_ms) *sweep_ms = pla->sweep_ms;
     return 0;
   }
 };
@@ -211,6 +300,17 @@ int xee_map_run_dev(xee_map* m, const double* heat_dev, const xee_solve_params* 
   return m->impl->run(heat_dev, false, prm, table_dev, false, (cudaStream_t)stream);
 }
 int xee_map_get_field(xee_map* m, int which, void* host_out) { DeviceGuard g(m->impl->device()); return m->impl->get_field(which, host_out); }
+int xee_map_adjoint_solve(xee_map* m, const xee_solve_params* prm, int* iters, double* r1_out, int* err) {
+  DeviceGuard g(m->impl->device());
+  return m->impl->adjoint_solve(prm, iters, r1_out, err);
+}
+int xee_map_adjoint_eval_host(xee_map* m, const double* heat_host, int n, double* table_host) {
+  DeviceGuard g(m->impl->device());
+  return m->impl->adjoint_eval(heat_host, n, table_host);
+}
+int xee_map_adjoint_timings(xee_map* m, double* setup_ms, double* probe_ms, double* sweep_ms) {
+  return m->impl->adjoint_timings(setup_ms, probe_ms, sweep_ms);
+}
 int xee_map_sweep_kernel_stats(xee_map* m, double* ms, long long* launches, int reset) { return m->impl->plan()->kernel_stats(ms, launches, reset); }
 int xee_map_kernel_info(xee_map* m, int* variant, int* sweeps_per_pass, long long* kernel_launches) {
   return m->impl->plan()->kernel_info(variant, sweeps_per_pass, kernel_launches);

@@ -533,9 +533,7 @@ struct Plan : PlanBase, PoolOwner {
     dim3 g((d.nx + 127) / 128, d.ny, nsets);
     aos_to_planar_kernel<T><<<g, 128, 0, own_stream>>>(dev, coe, d.nx, d.ny);
     XEE_LAUNCH_OK();
-    XEE_CHECK(cudaStreamSynchronize(own_stream));
-    cheb_rho = 0.0; rho_ps.clear(); est_rho_ps.clear();
-    return line_factors();
+    return operator_written();
   }
   int set_abc(const void* a, const void* b, const void* c, double dx, double dy) override {
     dim3 blk(64, 4), g((d.nx - 2 + 63) / 64, (d.ny - 2 + 3) / 4, nsets);
@@ -545,6 +543,11 @@ struct Plan : PlanBase, PoolOwner {
     cal_coe_kernel<T><<<g, blk, 0, own_stream>>>((const T*)a, (const T*)b, (const T*)c, coe, (T)dx, (T)dy, d.nx,
                                                  d.ny, sa, sb, sc, (long long)kPlanes * nn);
     XEE_LAUNCH_OK();
+    return operator_written();
+  }
+  // A new planar operator has been written into `coe` on own_stream (set_coe_aos, set_abc, or a kernel of the caller's, as
+  // the transposed operator of a map's adjoint): forget the spectral data of the old one, rebuild what derives from it.
+  int operator_written() {
     XEE_CHECK(cudaStreamSynchronize(own_stream));
     cheb_rho = 0.0; rho_ps.clear(); est_rho_ps.clear();
     return line_factors();

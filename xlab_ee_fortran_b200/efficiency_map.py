@@ -15,6 +15,8 @@ from . import _lib
 from .plan import ARITH_FAST, ARITH_STRICT, CHEBYSHEV, F32, F64, JACOBI, METHODS, SolveParams, _SolveParams
 
 COLS = ("iters", "r1", "err", "sum_Q", "ke_gen", "efficiency", "sum_Qeta", "efficiency_eta")
+ADJ_COLS = ("sum_Q", "ke_gen", "efficiency")     # rows of adjoint_eval
+FIELDS = {"psi": 0, "f": 1, "theta": 2, "eta": 3, "chi": 4, "eta_discrete": 5, "lambda": 6}
 
 
 class _MapDesc(C.Structure):
@@ -74,10 +76,35 @@ class EfficiencyMap:
                                               C.c_void_p(table_t.data_ptr()), s), "map_run_dev")
         return table_t
 
+    def adjoint_solve(self, p: SolveParams):
+        """Solves L^T lambda = g once (g: the gradient of ke_gen in psi) and forms mu = H^T lambda on the B cells, after which
+        adjoint_eval gives the exact discrete efficiency of any heating.  Returns (iters, r1, err) of the solve."""
+        q = _prm(p)
+        it = C.c_int(0); r1 = C.c_double(0); err = C.c_int(0)
+        _lib.check(_lib.lib().xee_map_adjoint_solve(self._h, C.byref(q), C.byref(it), C.byref(r1), C.byref(err)),
+                   "map_adjoint_solve")
+        return it.value, r1.value, err.value
+
+    def adjoint_eval(self, heat):
+        """heat [n,5] host doubles, any n >= 1 -> [n, 3] host doubles (columns ADJ_COLS) from the last adjoint_solve."""
+        heat = np.ascontiguousarray(heat, np.float64)
+        assert heat.ndim == 2 and heat.shape[1] == 5
+        table = np.zeros((heat.shape[0], len(ADJ_COLS)))
+        _lib.check(_lib.lib().xee_map_adjoint_eval_host(self._h, heat.ctypes.data_as(C.c_void_p), C.c_int(heat.shape[0]),
+                                                        table.ctypes.data_as(C.c_void_p)), "map_adjoint_eval_host")
+        return table
+
+    def adjoint_timings(self):
+        """Host wall time (ms) of the adjoint plan: setup (first solve only), spectral probes and sweep kernels."""
+        v = [C.c_double(0) for _ in range(3)]
+        _lib.check(_lib.lib().xee_map_adjoint_timings(self._h, *(C.byref(x) for x in v)), "map_adjoint_timings")
+        return dict(setup_ms=v[0].value, probe_ms=v[1].value, sweep_ms=v[2].value)
+
     def field(self, which):
-        idx = {"psi": 0, "f": 1, "theta": 2, "eta": 3, "chi": 4}[which]
+        """psi, f, theta, eta, chi as computed by run(); eta_discrete (eta_d on the B cells) and lambda by adjoint_solve()."""
+        idx = FIELDS[which]
         shape = {0: (self.nheat, self.nz, self.nr), 1: (self.nheat, self.nz, self.nr), 2: (self.nz - 1, self.nr - 1),
-                 3: (self.nz, self.nr - 1), 4: (self.nz, self.nr)}[idx]
+                 3: (self.nz, self.nr - 1), 4: (self.nz, self.nr), 5: (self.nz - 1, self.nr - 1), 6: (self.nz, self.nr)}[idx]
         out = np.zeros(shape, self.np_dtype)
         _lib.check(_lib.lib().xee_map_get_field(self._h, idx, out.ctypes.data_as(C.c_void_p)), "map_get_field")
         return out
