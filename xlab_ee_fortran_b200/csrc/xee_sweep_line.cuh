@@ -16,8 +16,8 @@
 //     in registers (z0 = M_t^-1 r), exchanges the two end values of z0 with the 3 other threads of the block by
 //     two butterfly shuffles, forms the true values of its neighbours' end points from 2 x 8 precomputed reduced-
 //     system coefficients, and subtracts the two precomputed spike vectors:  z = z0 - v b(t-1) - w a(t+1);
-//   * the 9 coefficients of its points (144 registers) and the 16 reduced coefficients stay in registers for the whole
-//     chunk of solves, the 4 x 8 factors (m, u, v, w) in thread-private shared-memory cells.  The coupling data (v, w
+//   * the 9 coefficients of its points (144 registers) stay in registers for the whole chunk of solves, the 4 x 8 factors
+//     (m, u, v, w) and the 16 reduced coefficients in thread-private shared-memory cells.  The coupling data (v, w
 //     and the reduced coefficients) are stored in FLOAT: the local Thomas solve is exact in working precision, the
 //     coupling correction carries a 6e-8 relative perturbation.  That only perturbs the (fixed, linear) approximate
 //     inverse that multiplies the residual — the fixed point L psi = f and the residual-based stop rule are untouched —
@@ -37,7 +37,8 @@
 //     per-unit reload of a thread's constants is fully coalesced 128-bit loads (2-3 us per unit instead of 10).
 // TWO = true is the two-level variant (xee_twolevel.cuh): the iterate is stored as (field y, coarse vector c) with
 // psi = y + P c; the 3 x 8 coarse patch of a tile arrives with its stage, the correction is added to the values as they are
-// read, and the restriction moments of the new residual leave as 32 doubles per (tile, solve).
+// read, and the restriction moments of the new residual leave as 32 doubles per (tile, solve).  The same reducer warp that
+// forms them also sums r^2 over the tile on check sweeps, so a check sweep adds no reduction before the CTA barrier.
 // Measured on B200 (512 solves, 512x256, fp64, Chebyshev, ncu, profiles/r02_*): one level 355 us per sweep = 6.05 TB/s
 // algorithmic (97 % of the measured copy peak) with a shared operator; two-level 585 us (instruction/latency bound).
 #pragma once
@@ -73,14 +74,15 @@ template <class T> struct Cfg {
   static constexpr int X_RAW = XP * (TH + 2), F_RAW = FP * TH;
   static constexpr int X_BYTES = (X_RAW + 127) / 128 * 128, F_BYTES = (F_RAW + 127) / 128 * 128;
   static constexpr int STAGE_BYTES = X_BYTES + 2 * F_BYTES;
-  // thread-private cells of the current tile's factor planes: m, u in working precision (pitch FP), the spikes v, w in
-  // float (8 floats = 2 chunks per thread, pitch AP = 17 chunks)
+  // thread-private cells of the current tile's factor planes: m, u in working precision (pitch FP), then four float planes
+  // (8 floats = 2 chunks per thread, pitch AP = 17 chunks): the spikes v, w and the reduced-system rows cB, cA
   static constexpr int AP = (TW + 4) * 4, A_BYTES = AP * TH;
-  static constexpr int FAC_BYTES = 2 * F_BYTES + 2 * A_BYTES;
+  static constexpr int FAC_BYTES = 2 * F_BYTES + 4 * A_BYTES;
   // result staging for the TMA store (two buffers, same [TH][FW] layout as the f box: odd chunk pitch, conflict-free STS.128)
   static constexpr int OUT_BYTES = F_BYTES, NOUT = 2;
-  // two-level method: per-thread restriction moments (S0, S1) of the residual, [2 buffers][TH rows][NSEG segments] double2
-  static constexpr int RES_BYTES = TH * NSEG * 16;
+  // two-level method: per-thread restriction moments (S0, S1) of the residual, [TH rows][NSEG segments] double2, then the
+  // thread's sum of r^2 (CHECK), [NT threads] double; two buffers
+  static constexpr int RES_BYTES = TH * NSEG * 16 + NT * 8;
   static constexpr int SMEM_BYTES = NSTAGE * STAGE_BYTES + FAC_BYTES + NOUT * OUT_BYTES;
   // two-level method: every stage also carries two 3 x 8 patches of coarse-correction values (current / previous iterate)
   static constexpr int CP_RAW = 3 * 8 * 8, CP_BYTES = 2 * 256;
@@ -302,7 +304,7 @@ __global__ void __launch_bounds__(ln::NT, ln::CTAS_PER_SM)
   constexpr int RES_OFS = AFTER + C::FAC_BYTES + C::NOUT * C::OUT_BYTES;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ uint64_t full_bar[NSTAGE];
-  __shared__ double red[2][NT / 32];          // per-warp sums of r^2 (CHECK), double-buffered by iteration parity
+  __shared__ double red[2][NT / 32];          // per-warp sums of r^2 (CHECK without TWO), double-buffered by iteration parity
   __shared__ uint32_t sdone[kDoneWords];   // stop flags of the batch as a bit mask: no global load per (tile, solve)
 
   const int tid = threadIdx.x;
@@ -406,10 +408,10 @@ __global__ void __launch_bounds__(ln::NT, ln::CTAS_PER_SM)
       const uint32_t full = n1 - n0 >= 32 ? 0xffffffffu : (1u << (n1 - n0)) - 1u;
       if ((umask & full) == full) continue;   // every solve of the unit has stopped: skip it before reloading the operator
     }
-    // the 9 coefficients of the thread's points and its 2 x 8 reduced-system coefficients (float) stay in registers for the
-    // whole chunk; the factors m, u, v, w go to thread-private cells of shared memory (read back by the same thread only)
+    // the 9 coefficients of the thread's points stay in registers for the whole chunk; the factors m, u, v, w and the
+    // reduced-system rows cB, cA go to thread-private cells of shared memory (read back by the same thread only).  cB and cA
+    // in registers made ptxas keep them as 16 doubles, 10 of which it spilled to local memory in the two-level variants.
     T cf[9][SEG];
-    float cB[SEG], cA[SEG];
     {
       // one operator per solve: the host makes every unit one solve (chunk = 1), so n0 names the operator set
       const unsigned char* pb = a.pack + (size_t)n0 * a.pack_set_stride + (size_t)tile * line_pack_tile_bytes<T>();
@@ -427,17 +429,12 @@ __global__ void __launch_bounds__(ln::NT, ln::CTAS_PER_SM)
           ldg16(pk + (size_t)((9 + k) * NV + q) * NT * V, t); sts16(faca + k * C::F_BYTES + 16u * q, t);
         }
 #pragma unroll
-      for (int k = 0; k < 2; ++k)
+      for (int k = 0; k < 4; ++k)
 #pragma unroll
         for (int q = 0; q < 2; ++q) {
           float t[4];
           ldg16(pa + (size_t)(k * 2 + q) * NT * 4, t); sts16(auxa + k * C::A_BYTES + 16u * q, t);
         }
-#pragma unroll
-      for (int q = 0; q < 2; ++q) {
-        ldg16(pa + (size_t)(4 + q) * NT * 4, &cB[q * 4]);
-        ldg16(pa + (size_t)(6 + q) * NT * 4, &cA[q * 4]);
-      }
     }
     for (int n = n0; n < n1; ++n) {
       if ((umask >> (n - n0)) & 1u) continue;
@@ -520,6 +517,8 @@ __global__ void __launch_bounds__(ln::NT, ln::CTAS_PER_SM)
           if ((inb >> e) & 1u) { s0 += (double)acc[e]; s1 = fma((double)e, (double)acc[e], s1); }
         const double mom[2] = {s0, s1};
         sts16(resa + (it & 1u) * C::RES_BYTES + (uint32_t)((r * NSEG + sg) * 16), mom);
+        if (CHECK)   // the tile's sum of r^2 is formed by the reducer warp too: no reduction before the barrier
+          asm volatile("st.shared.f64 [%0], %1;" ::"r"(resa + (it & 1u) * C::RES_BYTES + (uint32_t)(TH * NSEG * 16 + tid * 8)), "d"(rr));
       }
       // ---- Thomas solve of the segment: forward  y(i) = (r(i) - coe4(i) y(i-1)) m(i),  back  z(i) = y(i) - u(i) z(i+1)
       {
@@ -543,6 +542,9 @@ __global__ void __launch_bounds__(ln::NT, ln::CTAS_PER_SM)
         g[2] = shfl_xor(g[0], 8); g[3] = shfl_xor(g[1], 8);
 #pragma unroll
         for (int k = 0; k < 4; ++k) g[4 + k] = shfl_xor(g[k], 16);
+        float cB[SEG], cA[SEG];
+        lds16(auxa + 2 * C::A_BYTES, &cB[0]); lds16(auxa + 2 * C::A_BYTES + 16u, &cB[4]);
+        lds16(auxa + 3 * C::A_BYTES, &cA[0]); lds16(auxa + 3 * C::A_BYTES + 16u, &cA[4]);
         T bl = (T)cB[0] * g[0], ar = (T)cA[0] * g[0];
 #pragma unroll
         for (int k = 1; k < 2 * BLK; ++k) { bl = Rn<T>::fma((T)cB[k], g[k], bl); ar = Rn<T>::fma((T)cA[k], g[k], ar); }
@@ -590,7 +592,7 @@ __global__ void __launch_bounds__(ln::NT, ln::CTAS_PER_SM)
         fence_proxy_async_smem();
         if (tid == 0) tma_store_wait_read0();
       }
-      if (CHECK) {   // per-warp sum of r^2 into this iteration's buffer BEFORE the barrier: no barrier of its own
+      if (CHECK && !TWO) {   // per-warp sum of r^2 into this iteration's buffer BEFORE the barrier: no barrier of its own
 #pragma unroll
         for (int q = 16; q > 0; q >>= 1) rr += __shfl_down_sync(0xffffffffu, rr, q);
         if ((tid & 31) == 0) red[it & 1u][tid >> 5] = rr;
@@ -619,6 +621,25 @@ __global__ void __launch_bounds__(ln::NT, ln::CTAS_PER_SM)
         }
         const double t = (t4[0] + t4[1]) + (t4[2] + t4[3]);
         a.cpart[((size_t)n * ntiles + tile) * 32 + lane] = t;
+        if (CHECK) {
+          // sum of r^2 over the tile in the order of the per-warp reduction below (a shuffle-down tree over the 32 lanes of
+          // warp w, then w = 0..3 in turn), so the check partials keep their bits: lane 8 w + p starts from the tree's first
+          // two levels for lane p of warp w, (v_p + v_p+16) + (v_p+8 + v_p+24), and finishes it with three shuffles
+          const double* rv = reinterpret_cast<const double*>(smem_raw + RES_OFS + (it & 1u) * C::RES_BYTES + TH * NSEG * 16) +
+                             32 * (lane >> 3) + (lane & 7);
+          double b = (rv[0] + rv[16]) + (rv[8] + rv[24]);
+#pragma unroll
+          for (int q = 4; q > 0; q >>= 1) b += __shfl_down_sync(0xffffffffu, b, q);
+          double w4[NT / 32];
+#pragma unroll
+          for (int q = 0; q < NT / 32; ++q) w4[q] = __shfl_sync(0xffffffffu, b, 8 * q);
+          if (lane == 0) {
+            double s = 0.0;
+#pragma unroll
+            for (int q = 0; q < NT / 32; ++q) s += w4[q];
+            a.partial[(size_t)n * ntiles + tile] = s;
+          }
+        }
       }
       if (!tstore) {
         T* const o = a.dst + ((size_t)n * nn + gofs);
@@ -631,7 +652,7 @@ __global__ void __launch_bounds__(ln::NT, ln::CTAS_PER_SM)
             if (gi + e < a.nx) o[e] = out[e];
         }
       }
-      if (CHECK && tid == 0) {   // fixed order: deterministic.  (The buffer is rewritten two iterations on, after a barrier this thread has passed.)
+      if (CHECK && !TWO && tid == 0) {   // fixed order: deterministic.  (The buffer is rewritten two iterations on, after a barrier this thread has passed.)
         double t = 0.0;
         for (int q = 0; q < NT / 32; ++q) t += red[it & 1u][q];
         a.partial[(size_t)n * ntiles + tile] = t;
