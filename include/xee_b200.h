@@ -283,7 +283,22 @@ int xee_series_destroy(xee_series* s);
 /* params: HOST [nsnap][XEE_SERIES_PARAMS]; table: HOST [nsnap][XEE_MAP_COLS] =
  * iters, r1, err, sum_Q, ke_gen, efficiency, max|w|, max|u| */
 int xee_series_run_host(xee_series* s, const double* params_host, const xee_solve_params* prm, double* table_host);
-/* which: 0 psi, 1 f, 2 theta_B, 3 u (C grid), 4 w (A grid), 5 A, 6 B, 7 C, 8 m2 (B grid); all [nsnap][...], plan dtype */
+/* The same series on caller-supplied snapshots (e.g. the reference's A.bin, B.bin, C.bin, Q and F files), arrays of the
+ * plan dtype with i (r) fastest:
+ *   A, B, C  [nsnap][nz][nr] on the O grid; required.
+ *   Q        [nsnap][nz-1][nr-1] heating on the B cells; required.  sum_Q = 0 gives a non-finite efficiency.
+ *   F        [nsnap][nz-1][nr-1] momentum forcing on the B cells; NULL: no momentum term (the bits of F = 0).
+ *   psi_bc   [nsnap][nz][nr]; only its rim is read, as Dirichlet values of r*psi; NULL: 0.  The first guess is 0 inside,
+ *            so r1_rel_rms_f keeps its meaning (relative to the initial residual).
+ * Every operator gets its own spectral probe (the parametric run may subsample a smooth series).  table as for run_host.
+ * _host: host pointers.  _dev: device pointers, read after the work already queued on `stream` (a cudaStream_t, NULL =
+ * the legacy default stream); the call returns after the table is on the host. */
+int xee_series_run_fields_host(xee_series* s, const void* A, const void* B, const void* C, const void* Q, const void* F,
+                               const void* psi_bc, const xee_solve_params* prm, double* table_host);
+int xee_series_run_fields_dev(xee_series* s, const void* A, const void* B, const void* C, const void* Q, const void* F,
+                              const void* psi_bc, const xee_solve_params* prm, double* table_host, void* stream);
+/* which: 0 psi, 1 f, 2 theta_B, 3 u (C grid), 4 w (A grid), 5 A, 6 B, 7 C, 8 m2 (B grid), 9 Q (B grid), 10 F (B grid; fails
+ * after a field run without F); all [nsnap][...], plan dtype */
 int xee_series_get_field(xee_series* s, int which, void* host_out);
 int xee_series_sweep_kernel_stats(xee_series* s, double* ms_total, long long* sweeps, int reset);
 int xee_series_kernel_info(xee_series* s, int* variant, int* sweeps_per_pass, long long* kernel_launches);

@@ -126,7 +126,7 @@ struct Map : MapBase, PoolOwner {
     const int nr = d.nr, nz = d.nz, nb = d.nheat;
     if (!s) s = pl->own_stream;
     XEE_CHECK(cudaMemcpyAsync(heat_d, heat, sizeof(Heat) * nb, heat_on_host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, s));
-    heating_rhs_kernel<T><<<heating_rhs_grid(nr, nz, nb), dim3(kHeatBX, kHeatBY), 0, s>>>(heat_d, f, ra, za, ex, nr, nz, k.g0, k.theta0, k.Cp); XEE_LAUNCH_OK();
+    heating_rhs_kernel<T><<<heating_rhs_grid(nr, nz, nb), dim3(kHeatBX, kHeatBY), 0, s>>>(BlobQ<T>{heat_d}, f, ra, za, ex, nr, nz, k.g0, k.theta0, k.Cp); XEE_LAUNCH_OK();
     XEE_CHECK(cudaMemsetAsync(psi, 0, sizeof(T) * nn * nb, s));     // rpsi = 0: boundary condition and first guess
     xee_solve_params prm = *prm_in;
     if (d.r1_rel_rms_f > 0) {   // tolerance relative to each location's own forcing: r1_n = r1_rel * rms(f_n)
@@ -157,7 +157,7 @@ struct Map : MapBase, PoolOwner {
       dim3 ge((nr - 1 + 127) / 128, nz, 1);
       eta_kernel<T><<<ge, 128, 0, s>>>(chi, eta, ra, ra, rho, ex, nr, nz, k.g0, k.Cp, k.theta0); XEE_LAUNCH_OK();
     }
-    map_integrals_kernel<T><<<nb, 256, 0, s>>>(heat_d, psi, theta, d.adjoint_check ? eta : nullptr, ra, ra, za, rho, nr, nz, integ);
+    map_integrals_kernel<T><<<nb, 256, 0, s>>>(BlobQ<T>{heat_d}, psi, theta, d.adjoint_check ? eta : nullptr, ra, ra, za, rho, nr, nz, integ);
     XEE_LAUNCH_OK();
     std::vector<double> hi(3 * (size_t)nb);
     XEE_CHECK(cudaMemcpyAsync(hi.data(), integ, sizeof(double) * 3 * nb, cudaMemcpyDeviceToHost, s));

@@ -19,6 +19,37 @@ __device__ __forceinline__ T heat_q(const Heat& h, T r, T z) {
   return (T)(h.q0 * exp(-dr * dr - dz * dz));
 }
 
+// Where the kernels below take the heating Q on B cell (ci, cj) of solve n from.  at(n) gives the solve's evaluator once;
+// calling it gives Q of one cell.
+// BlobQ: the Gaussian blob heat[n] at the cell centre ((ra(ci)+ra(ci+1))/2, (za(cj)+za(cj+1))/2), evaluated in T.
+template <class T>
+struct BlobQ {
+  const Heat* heat;
+  struct At {
+    Heat h;
+    __device__ __forceinline__ T operator()(int ci, int cj, const T* ra, const T* za) const {
+      using R = Rn<T>;
+      const T rm = R::div(R::add(ra[ci], ra[ci + 1]), T(2)), zm = R::div(R::add(za[cj], za[cj + 1]), T(2));
+      return heat_q<T>(h, rm, zm);
+    }
+  };
+  __device__ __forceinline__ At at(int n) const {
+    const Heat* h = heat + n;
+    return At{Heat{__ldg(&h->rc), __ldg(&h->zc), __ldg(&h->sr), __ldg(&h->sz), __ldg(&h->q0)}};
+  }
+};
+// FieldQ: a caller's field, [n][nz-1][nr-1] with i fastest.
+template <class T>
+struct FieldQ {
+  const T* Q;
+  int nr, nz;
+  struct At {
+    const T* q; int ld;
+    __device__ __forceinline__ T operator()(int ci, int cj, const T*, const T*) const { return __ldg(q + (size_t)cj * ld + ci); }
+  };
+  __device__ __forceinline__ At at(int n) const { return At{Q + (size_t)n * (nr - 1) * (nz - 1), nr - 1}; }
+};
+
 // K7: f(i,j) = g0/theta0 * ( dJ(i,j) + dJ(i,j-1) )/2 on the O interior, 0 on the boundary,
 //     dJ(i,j) = (J(i,j)-J(i-1,j)) / ((ra(i+1)-ra(i-1))/2),  J(i,j) = Q(i,j)/(Cp*exner(j))   [B grid]
 // A block of kHeatBX x kHeatBY points first forms J on the (kHeatBX+1) x (kHeatBY+1) B cells it touches (an exp and a division
@@ -27,23 +58,22 @@ __device__ __forceinline__ T heat_q(const Heat& h, T r, T z) {
 // the operations, in the order, of the reference: the values are bit for bit the same.
 constexpr int kHeatBX = 64, kHeatBY = 4;
 inline dim3 heating_rhs_grid(int nr, int nz, int nb) { return dim3((nr + kHeatBX - 1) / kHeatBX, (nz + kHeatBY - 1) / kHeatBY, nb); }
-template <class T>
-__global__ void __launch_bounds__(kHeatBX* kHeatBY) heating_rhs_kernel(const Heat* __restrict__ heat, T* __restrict__ f,
+template <class T, class QSrc>
+__global__ void __launch_bounds__(kHeatBX* kHeatBY) heating_rhs_kernel(QSrc src, T* __restrict__ f,
                                                                       const T* __restrict__ ra, const T* __restrict__ za,
                                                                       const T* __restrict__ ex, int nr, int nz, T g0, T theta0, T Cp) {
   using R = Rn<T>;
   __shared__ T Jc[kHeatBY + 1][kHeatBX + 1];     // cell (ci, cj) = (i0 - 1 + x, j0 - 1 + y)
   const int i0 = blockIdx.x * kHeatBX, j0 = blockIdx.y * kHeatBY, n = blockIdx.z;
   const int tid = threadIdx.y * kHeatBX + threadIdx.x;
-  const Heat h = heat[n];
+  const auto Qn = src.at(n);
   for (int q = tid; q < (kHeatBX + 1) * (kHeatBY + 1); q += kHeatBX * kHeatBY) {
     const int x = q % (kHeatBX + 1), y = q / (kHeatBX + 1);
     const int ci = i0 - 1 + x, cj = j0 - 1 + y;
     T v = T(0);
     if (ci >= 0 && ci <= nr - 2 && cj >= 0 && cj <= nz - 2) {
-      // Fortran (I,J) = (ci+1,cj+1).  B cell centre = ((ra(I)+ra(I+1))/2, (za(J)+za(J+1))/2); J(.,J) uses exner(J)
-      const T rm = R::div(R::add(ra[ci], ra[ci + 1]), T(2)), zm = R::div(R::add(za[cj], za[cj + 1]), T(2));
-      v = R::div(heat_q<T>(h, rm, zm), R::mul(Cp, ex[cj]));
+      // Fortran (I,J) = (ci+1,cj+1); J(.,J) uses exner(J)
+      v = R::div(Qn(ci, cj, ra, za), R::mul(Cp, ex[cj]));
     }
     Jc[y][x] = v;
   }
@@ -75,8 +105,8 @@ __device__ __forceinline__ T weighted(T v, const T* ra, const T* rc, const T* za
 
 // One block per heating location: sum_Q, (g0/theta0) * I[w theta], optional I[Q (eta(i,j)+eta(i,j+1))/2].
 // Deterministic tree reduction in double (the reference sums sequentially in real(4)).
-template <class T>
-__global__ void __launch_bounds__(256) map_integrals_kernel(const Heat* __restrict__ heat, const T* __restrict__ psi,
+template <class T, class QSrc>
+__global__ void __launch_bounds__(256) map_integrals_kernel(QSrc src, const T* __restrict__ psi,
                                                             const T* __restrict__ theta, const T* __restrict__ eta,
                                                             const T* __restrict__ ra, const T* __restrict__ rc,
                                                             const T* __restrict__ za, const T* __restrict__ rho,
@@ -85,15 +115,14 @@ __global__ void __launch_bounds__(256) map_integrals_kernel(const Heat* __restri
   using R = Rn<T>;
   __shared__ double red[32];
   const int n = blockIdx.x;
-  const Heat h = heat[n];
+  const auto Qn = src.at(n);
   const T* p = psi + (size_t)n * nr * nz;
   theta += (size_t)n * theta_stride;
   const int ncell = (nr - 1) * (nz - 1);
   double sq = 0, swt = 0, sqe = 0;
   for (int q = threadIdx.x; q < ncell; q += 256) {
     const int i = q % (nr - 1), j = q / (nr - 1);
-    const T rm = R::div(R::add(ra[i], ra[i + 1]), T(2)), zm = R::div(R::add(za[j], za[j + 1]), T(2));
-    const T Q = heat_q<T>(h, rm, zm);
+    const T Q = Qn(i, j, ra, za);
     sq += (double)weighted<T>(Q, ra, rc, za, rho, i, j);
     // w(i,j) = d_rcuvdr_O2A(rpsi)/rho(j)  (rpsiToUW, old-diagnose/diagnose.f90:921-927)
     const T den_r = R::sub(ra[i + 1], ra[i]), rcm = R::div(R::add(rc[i], rc[i + 1]), T(2));

@@ -10,6 +10,8 @@
 //   dynamical RHS       src/old-diagnose/diagnose.f90:350-354 (rhoC_C), 359-367 (m^2, intended maths), 412-436
 //   solve               elliptic_tools.f90:93-265, Chebyshev weights per solve (one spectral radius per operator)
 //   u, w, integrals     old-diagnose/diagnose.f90:915-941, 1117-1127, 1029-1113
+// The builders above are one producer of the fields A, B, C, Q, F and the rim of psi; run_fields takes the same fields from
+// the caller (old-diagnose/diagnose.f90:211-212, 241-242 read them from files).  Both end in the same tail.
 // Deviations from the legacy driver's latent bugs are listed in DESIGN.md section 3.
 #include "xee_map_kernels.cuh"
 
@@ -95,22 +97,33 @@ __global__ void series_m2_kernel(const T* __restrict__ C, T* __restrict__ m2, co
   }
 }
 
-// f += RHS_mom(i,j) = -(wA(i,j)+wA(i-1,j))/rcuva(i)^2, wA = d_dz_B2A(sqrt(m2)*F) on rows 2..nz-2 (0 elsewhere),
-// F(i,j) = -k v(r_{i+1/2}) exp(-z_{j+1/2}/h) on B.                      old-diagnose/diagnose.f90:412-436
+// The parametric sources on the B cells of snapshot blockIdx.z: the heating Q = heat_q of the snapshot's blob at the cell
+// centre (as heating_rhs_kernel and map_integrals_kernel evaluate it for a map) and the momentum forcing
+// F(i,j) = -k v(r_{i+1/2}) exp(-z_{j+1/2}/h), evaluated in double and rounded to T.
 template <class T>
-__global__ void series_mom_rhs_kernel(const Snap* __restrict__ snaps, const T* __restrict__ m2, T* __restrict__ f,
-                                      const T* __restrict__ ra, const T* __restrict__ rc, const T* __restrict__ za,
-                                      int nr, int nz) {
+__global__ void series_sources_kernel(const Snap* __restrict__ snaps, const Heat* __restrict__ heat, T* __restrict__ Q,
+                                      T* __restrict__ F, const T* __restrict__ ra, const T* __restrict__ za, int nr, int nz) {
+  const int ib = blockIdx.x * blockDim.x + threadIdx.x, jb = blockIdx.y, n = blockIdx.z;   // 0-based B cell
+  if (ib >= nr - 1) return;
+  const Snap s = snaps[n];
+  const size_t o = (size_t)n * (nr - 1) * (nz - 1) + (size_t)jb * (nr - 1) + ib;
+  Q[o] = BlobQ<T>{heat}.at(n)(ib, jb, ra, za);
+  const double rm = 0.5 * ((double)ra[ib] + (double)ra[ib + 1]), zm = 0.5 * ((double)za[jb] + (double)za[jb + 1]);
+  F[o] = (T)(-s.fk * wind_v(s, rm) * exp(-zm / s.fh));
+}
+
+// f += RHS_mom(i,j) = -(wA(i,j)+wA(i-1,j))/rcuva(i)^2, wA = d_dz_B2A(sqrt(m2)*F) on rows 2..nz-2 (0 elsewhere), F on B.
+//                                                                        old-diagnose/diagnose.f90:412-436
+template <class T>
+__global__ void series_mom_rhs_kernel(const T* __restrict__ F, const T* __restrict__ m2, T* __restrict__ f,
+                                      const T* __restrict__ rc, const T* __restrict__ za, int nr, int nz) {
   using R = Rn<T>;
   const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y, n = blockIdx.z;   // 0-based O point
   if (i < 1 || i >= nr - 1 || j < 1 || j >= nz - 1) return;
-  const Snap s = snaps[n];
-  const T* m = m2 + (size_t)n * (nr - 1) * (nz - 1);
-  auto Fb = [&](int ib, int jb) {   // B cell (0-based)
-    const double rm = 0.5 * ((double)ra[ib] + (double)ra[ib + 1]), zm = 0.5 * ((double)za[jb] + (double)za[jb + 1]);
-    return (T)(-s.fk * wind_v(s, rm) * exp(-zm / s.fh));
-  };
-  auto wB = [&](int ib, int jb) { return R::mul(R::sqrt(m[(size_t)jb * (nr - 1) + ib]), Fb(ib, jb)); };
+  const size_t nB = (size_t)(nr - 1) * (nz - 1);
+  const T* m = m2 + (size_t)n * nB;
+  const T* Fn = F + (size_t)n * nB;
+  auto wB = [&](int ib, int jb) { const size_t o = (size_t)jb * (nr - 1) + ib; return R::mul(R::sqrt(m[o]), Fn[o]); };
   auto wA = [&](int ia) {           // A point (ia, j), Fortran J = j+1 in 2..nz-2  <=>  1 <= j <= nz-3
     if (j < 1 || j > nz - 3) return T(0);
     return R::div(R::sub(wB(ia, j), wB(ia, j - 1)), R::div(R::sub(za[j + 1], za[j - 1]), T(2)));
@@ -118,6 +131,14 @@ __global__ void series_mom_rhs_kernel(const Snap* __restrict__ snaps, const T* _
   const T mom = -R::div(R::add(wA(i), wA(i - 1)), R::mul(rc[i], rc[i]));
   const size_t o = (size_t)n * nr * nz + (size_t)j * nr + i;
   f[o] = R::add(f[o], mom);
+}
+
+// Dirichlet data of a caller's psi_bc: keep the rim, zero the interior (the first guess).
+template <class T>
+__global__ void zero_interior_kernel(T* __restrict__ psi, int nr, int nz) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y;
+  if (i < 1 || i >= nr - 1 || j < 1 || j >= nz - 1) return;
+  psi[(size_t)blockIdx.z * nr * nz + (size_t)j * nr + i] = T(0);
 }
 
 template <class T>
@@ -137,16 +158,22 @@ struct SeriesBase {
   int device() const { return d.device; }
   virtual ~SeriesBase() {}
   virtual int run(const double* params_host, const xee_solve_params* prm, double* table_host) = 0;
+  virtual int run_fields(const void* A, const void* B, const void* C, const void* Q, const void* F, const void* psi_bc,
+                         bool on_host, const xee_solve_params* prm, double* table_host, cudaStream_t stream) = 0;
   virtual int get_field(int which, void* host_out) = 0;
   virtual PlanBase* plan() = 0;
 };
 
+// A run is a producer that fills A, B, C, Q, F and the rim of psi, followed by one shared tail from those fields to the table.
+// The parametric producer builds them from XEE_SERIES_PARAMS per snapshot; the field producer copies a caller's arrays.
 template <class T>
 struct Series : SeriesBase, PoolOwner {
   std::unique_ptr<Plan<T>> pl;
-  T *A = nullptr, *B = nullptr, *C = nullptr, *a = nullptr, *b = nullptr, *c = nullptr, *m2 = nullptr, *theta = nullptr,
-    *psi = nullptr, *f = nullptr, *u = nullptr, *w = nullptr, *r1v = nullptr, *ra = nullptr, *za = nullptr, *ex = nullptr, *rho = nullptr;
+  T *A = nullptr, *B = nullptr, *C = nullptr, *Q = nullptr, *F = nullptr, *a = nullptr, *b = nullptr, *c = nullptr, *m2 = nullptr,
+    *theta = nullptr, *psi = nullptr, *f = nullptr, *u = nullptr, *w = nullptr, *r1v = nullptr, *ra = nullptr, *za = nullptr,
+    *ex = nullptr, *rho = nullptr;
   Snap* snaps = nullptr; Heat* heat = nullptr; double* integ = nullptr; double* mx = nullptr;
+  bool has_F = false;   // F holds the last run's momentum forcing (a field run without F has none)
   size_t nn = 0;
   T dr = 0, dz = 0;
   PhysK<T> k;
@@ -169,6 +196,7 @@ struct Series : SeriesBase, PoolOwner {
     if (pl->init()) return 1;
     const size_t nB = (size_t)(nr - 1) * (nz - 1);
     XEE_CHECK(own(&A, sizeof(T) * nn * nb)); XEE_CHECK(own(&B, sizeof(T) * nn * nb)); XEE_CHECK(own(&C, sizeof(T) * nn * nb));
+    XEE_CHECK(own(&Q, sizeof(T) * nB * nb)); XEE_CHECK(own(&F, sizeof(T) * nB * nb));
     XEE_CHECK(own(&a, sizeof(T) * (nr - 1) * (nz - 2) * nb)); XEE_CHECK(own(&b, sizeof(T) * nB * nb));
     XEE_CHECK(own(&c, sizeof(T) * (nr - 2) * (nz - 1) * nb));
     XEE_CHECK(own(&m2, sizeof(T) * nB * nb)); XEE_CHECK(own(&theta, sizeof(T) * nB * nb));
@@ -191,8 +219,8 @@ struct Series : SeriesBase, PoolOwner {
     cudaDeviceSynchronize();   // the device is done with the owned blocks before they go back to the pool (see ~Plan)
   }
 
-  // table row: iters, r1, err, sum_Q, ke_gen, efficiency, max|w|, max|u|
-  int run(const double* params, const xee_solve_params* prm_in, double* table) override {
+  // Parametric producer: the vortex, the blob heating, the friction and the pumping rim of every snapshot.
+  int run(const double* params, const xee_solve_params* prm, double* table) override {
     TraceTimer tt("series run (total)");
     const int nr = d.nr, nz = d.nz, nb = d.nsnap;
     cudaStream_t s = pl->own_stream;
@@ -200,30 +228,76 @@ struct Series : SeriesBase, PoolOwner {
     std::vector<Heat> hh(nb);
     for (int n = 0; n < nb; ++n) { const double* p = params + (size_t)n * kSeriesCols; hh[n] = Heat{p[14], p[15], p[16], p[17], p[18]}; }
     XEE_CHECK(cudaMemcpyAsync(heat, hh.data(), sizeof(Heat) * nb, cudaMemcpyHostToDevice, s));
-    dim3 gO((nr + 127) / 128, nz, nb);
+    dim3 gO((nr + 127) / 128, nz, nb), gB((nr - 1 + 127) / 128, nz - 1, nb);
     series_vortex_kernel<T><<<gO, 128, 0, s>>>(snaps, A, B, C, nr, nz, d.Lr[0], d.Lr[1], d.Lz[0], d.Lz[1]); XEE_LAUNCH_OK();
+    series_sources_kernel<T><<<gB, 128, 0, s>>>(snaps, heat, Q, F, ra, za, nr, nz); XEE_LAUNCH_OK();
+    series_bc_kernel<T><<<gO, 128, 0, s>>>(snaps, psi, ra, nr, nz); XEE_LAUNCH_OK();
+    has_F = true;
+    // Spectral probes of the accelerated methods: when the snapshots form a smooth series (every vortex parameter changes by
+    // less than 5 % from one snapshot to the next) only every 8th operator is probed and the rest interpolated.
+    double worst = 0.0;
+    for (int n = 1; n < nb; ++n)
+      for (int q = 0; q < 14; ++q) {
+        const double a0 = params[(size_t)(n - 1) * kSeriesCols + q], a1 = params[(size_t)n * kSeriesCols + q];
+        const double sc = std::max(std::fabs(a0), std::fabs(a1));
+        if (sc > 0) worst = std::max(worst, std::fabs(a1 - a0) / sc);
+      }
+    return tail((nb >= 32 && worst < 0.05) ? env_int("XEE_RHO_SUBSAMPLE", 8) : 0, prm, table);
+  }
+
+  // Field producer: the caller's arrays of T (host, or device read on `in` after the work queued there).  F == nullptr: no
+  // momentum term; psi_bc == nullptr: a zero rim.  Only the rim of psi_bc is read; the first guess is 0 inside.
+  int run_fields(const void* A_in, const void* B_in, const void* C_in, const void* Q_in, const void* F_in, const void* bc_in,
+                 bool on_host, const xee_solve_params* prm, double* table, cudaStream_t in) override {
+    if (!A_in || !B_in || !C_in || !Q_in) return fail("xee_series_run_fields: A, B, C and Q must not be NULL");
+    TraceTimer tt("series run_fields (total)");
+    const int nr = d.nr, nz = d.nz, nb = d.nsnap;
+    cudaStream_t s = pl->own_stream;
+    if (on_host) in = s;
+    else {   // device arrays must live on the series' device: a copy from another device would depend on peer access
+      for (const void* p : {A_in, B_in, C_in, Q_in, F_in, bc_in}) {
+        if (!p) continue;
+        cudaPointerAttributes pa{};
+        if (cudaPointerGetAttributes(&pa, p) != cudaSuccess || (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) ||
+            pa.device != d.device) {
+          cudaGetLastError();
+          return fail("xee_series_run_fields_dev: every array must be device memory on the series' device");
+        }
+      }
+    }
+    // a run that failed part-way may have left work on the own stream that still reads these buffers
+    XEE_CHECK(cudaStreamSynchronize(s));
+    const cudaMemcpyKind kind = on_host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+    const size_t bO = sizeof(T) * nn * nb, bB = sizeof(T) * (size_t)(nr - 1) * (nz - 1) * nb;
+    XEE_CHECK(cudaMemcpyAsync(A, A_in, bO, kind, in)); XEE_CHECK(cudaMemcpyAsync(B, B_in, bO, kind, in));
+    XEE_CHECK(cudaMemcpyAsync(C, C_in, bO, kind, in)); XEE_CHECK(cudaMemcpyAsync(Q, Q_in, bB, kind, in));
+    has_F = F_in != nullptr;
+    if (has_F) XEE_CHECK(cudaMemcpyAsync(F, F_in, bB, kind, in));
+    if (bc_in) XEE_CHECK(cudaMemcpyAsync(psi, bc_in, bO, kind, in));
+    else XEE_CHECK(cudaMemsetAsync(psi, 0, bO, in));
+    XEE_CHECK(cudaStreamSynchronize(in));   // the caller's arrays are consumed; the rest runs on the series' own stream
+    if (bc_in) { zero_interior_kernel<T><<<dim3((nr + 127) / 128, nz, nb), 128, 0, s>>>(psi, nr, nz); XEE_LAUNCH_OK(); }
+    // Probe every operator: no smoothness rule for arbitrary fields has been calibrated.
+    return tail(0, prm, table);
+  }
+
+  // Shared tail: operators, theta, right-hand sides, the batched solve and the table from the fields of the producer.
+  // table row: iters, r1, err, sum_Q, ke_gen, efficiency, max|w|, max|u|
+  int tail(int rho_subsample, const xee_solve_params* prm_in, double* table) {
+    const int nr = d.nr, nz = d.nz, nb = d.nsnap;
+    cudaStream_t s = pl->own_stream;
+    dim3 gO((nr + 127) / 128, nz, nb);
     dim3 blk(64, 4), g2((nr + 63) / 64, (nz + 3) / 4, nb);
     build_abc_kernel<T><<<g2, blk, 0, s>>>(A, B, C, ra, rho, a, b, c, nr, nz); XEE_LAUNCH_OK();
     XEE_CHECK(cudaStreamSynchronize(s));
     if (pl->set_abc(a, b, c, (double)dr, (double)dz)) return 1;
+    const FieldQ<T> qsrc{Q, nr, nz};
     background_theta_kernel<T><<<nb, 256, 0, s>>>(A, B, theta, ra, za, nr, nz, k.g0, k.theta0); XEE_LAUNCH_OK();
-    heating_rhs_kernel<T><<<heating_rhs_grid(nr, nz, nb), dim3(kHeatBX, kHeatBY), 0, s>>>(heat, f, ra, za, ex, nr, nz, k.g0, k.theta0, k.Cp); XEE_LAUNCH_OK();
+    heating_rhs_kernel<T><<<heating_rhs_grid(nr, nz, nb), dim3(kHeatBX, kHeatBY), 0, s>>>(qsrc, f, ra, za, ex, nr, nz, k.g0, k.theta0, k.Cp); XEE_LAUNCH_OK();
     dim3 gm((nz - 1 + 63) / 64, nb);
     series_m2_kernel<T><<<gm, 64, 0, s>>>(C, m2, ra, ra, nr, nz, nb); XEE_LAUNCH_OK();
-    series_mom_rhs_kernel<T><<<gO, 128, 0, s>>>(snaps, m2, f, ra, ra, za, nr, nz); XEE_LAUNCH_OK();
-    series_bc_kernel<T><<<gO, 128, 0, s>>>(snaps, psi, ra, nr, nz); XEE_LAUNCH_OK();
-    // Spectral probes of the accelerated methods: when the snapshots form a smooth series (every vortex parameter changes by
-    // less than 5 % from one snapshot to the next) only every 8th operator is probed and the rest interpolated.
-    {
-      double worst = 0.0;
-      for (int n = 1; n < nb; ++n)
-        for (int q = 0; q < 14; ++q) {
-          const double a0 = params[(size_t)(n - 1) * kSeriesCols + q], a1 = params[(size_t)n * kSeriesCols + q];
-          const double sc = std::max(std::fabs(a0), std::fabs(a1));
-          if (sc > 0) worst = std::max(worst, std::fabs(a1 - a0) / sc);
-        }
-      pl->rho_subsample = (nb >= 32 && worst < 0.05) ? env_int("XEE_RHO_SUBSAMPLE", 8) : 0;
-    }
+    if (has_F) { series_mom_rhs_kernel<T><<<gO, 128, 0, s>>>(F, m2, f, ra, za, nr, nz); XEE_LAUNCH_OK(); }
+    pl->rho_subsample = rho_subsample;
     xee_solve_params prm = *prm_in;
     if (d.r1_rel_rms_f > 0) {
       // tolerance relative to the INITIAL residual L psi0 - f: with the pumping boundary condition the boundary data,
@@ -236,7 +310,7 @@ struct Series : SeriesBase, PoolOwner {
     std::vector<double> r1o(nb), r2o(nb);
     if (pl->solve(psi, f, &prm, iters.data(), r1o.data(), r2o.data(), err.data(), s, false, nullptr, 0)) return 1;
     uw_kernel<T><<<gO, 128, 0, s>>>(psi, u, w, ra, ra, za, rho, nr, nz); XEE_LAUNCH_OK();
-    map_integrals_kernel<T><<<nb, 256, 0, s>>>(heat, psi, theta, nullptr, ra, ra, za, rho, nr, nz, integ, (long long)(nr - 1) * (nz - 1));
+    map_integrals_kernel<T><<<nb, 256, 0, s>>>(qsrc, psi, theta, nullptr, ra, ra, za, rho, nr, nz, integ, (long long)(nr - 1) * (nz - 1));
     XEE_LAUNCH_OK();
     absmax_kernel<T><<<nb, 256, 0, s>>>(w, (long long)(nr - 1) * nz, mx); XEE_LAUNCH_OK();
     absmax_kernel<T><<<nb, 256, 0, s>>>(u, (long long)nr * (nz - 1), mx + nb); XEE_LAUNCH_OK();
@@ -266,6 +340,10 @@ struct Series : SeriesBase, PoolOwner {
       case 6: src = B; bytes = sizeof(T) * nn * nb; break;
       case 7: src = C; bytes = sizeof(T) * nn * nb; break;
       case 8: src = m2; bytes = sizeof(T) * nB * nb; break;
+      case 9: src = Q; bytes = sizeof(T) * nB * nb; break;
+      case 10:
+        if (!has_F) return fail("xee_series_get_field: the last run had no momentum forcing F");
+        src = F; bytes = sizeof(T) * nB * nb; break;
       default: return fail("xee_series_get_field: unknown field");
     }
     XEE_CHECK(cudaMemcpy(out, src, bytes, cudaMemcpyDeviceToHost));
@@ -294,6 +372,16 @@ int xee_series_create(const xee_series_desc* desc, xee_series** out) {
 }
 int xee_series_destroy(xee_series* m) { if (m) { DeviceGuard g(m->impl->device()); delete m->impl; delete m; } return 0; }
 int xee_series_run_host(xee_series* m, const double* params, const xee_solve_params* prm, double* table) { DeviceGuard g(m->impl->device()); return m->impl->run(params, prm, table); }
+int xee_series_run_fields_host(xee_series* m, const void* A, const void* B, const void* C, const void* Q, const void* F,
+                               const void* psi_bc, const xee_solve_params* prm, double* table) {
+  DeviceGuard g(m->impl->device());
+  return m->impl->run_fields(A, B, C, Q, F, psi_bc, true, prm, table, nullptr);
+}
+int xee_series_run_fields_dev(xee_series* m, const void* A, const void* B, const void* C, const void* Q, const void* F,
+                              const void* psi_bc, const xee_solve_params* prm, double* table, void* stream) {
+  DeviceGuard g(m->impl->device());
+  return m->impl->run_fields(A, B, C, Q, F, psi_bc, false, prm, table, (cudaStream_t)stream);
+}
 int xee_series_get_field(xee_series* m, int which, void* out) { DeviceGuard g(m->impl->device()); return m->impl->get_field(which, out); }
 int xee_series_sweep_kernel_stats(xee_series* m, double* ms, long long* launches, int reset) { return m->impl->plan()->kernel_stats(ms, launches, reset); }
 int xee_series_probe_stats(xee_series* m, double* ms, int reset) {

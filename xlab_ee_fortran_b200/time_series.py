@@ -46,11 +46,49 @@ class TimeSeries:
                                                   table.ctypes.data_as(C.c_void_p)), "series_run_host")
         return table
 
+    def run_fields(self, A, B, Cf, Q, p: SolveParams, F=None, psi_bc=None):
+        """The series on caller-supplied snapshots: A, B, C and psi_bc [nsnap, nz, nr] on the O grid, the heating Q and the
+        momentum forcing F [nsnap, nz-1, nr-1] on the B cells, i (r) fastest.  F=None: no momentum term; psi_bc=None: a zero
+        rim, else only its rim is read (Dirichlet values of r*psi).  Host arrays (numpy, CPU tensors) are converted to the
+        plan dtype and go through the host entry.  CUDA tensors must all be of the plan dtype and on the series' device,
+        and are read on the current stream; a mix of host and CUDA inputs is refused.  Returns the table
+        [nsnap, 8] (columns COLS); a heating whose integral is 0 gives a non-finite efficiency."""
+        n, nz, nr = self.nsnap, self.nz, self.nr
+        shapes = dict(A=(n, nz, nr), B=(n, nz, nr), C=(n, nz, nr), Q=(n, nz - 1, nr - 1), F=(n, nz - 1, nr - 1), psi_bc=(n, nz, nr))
+        given = dict(A=A, B=B, C=Cf, Q=Q, F=F, psi_bc=psi_bc)
+        on_dev = any(getattr(v, "is_cuda", False) for v in given.values())
+        if not on_dev:
+            given = {k: None if v is None else np.asarray(v) for k, v in given.items()}
+        for k, v in given.items():
+            if v is not None and tuple(v.shape) != shapes[k]:
+                raise ValueError(f"run_fields: {k} has shape {tuple(v.shape)}, expected {shapes[k]}")
+        if on_dev:
+            import torch
+            tdt = torch.float64 if self.np_dtype == np.float64 else torch.float32
+            for k, v in given.items():
+                if v is not None and not (isinstance(v, torch.Tensor) and v.is_cuda and v.dtype == tdt):
+                    raise TypeError(f"run_fields: {k} must be a CUDA tensor of {tdt} like the other device inputs")
+            arrs = {k: None if v is None else v.contiguous() for k, v in given.items()}
+            ptr = lambda v: None if v is None else C.c_void_p(v.data_ptr())
+            extra = (C.c_void_p(torch.cuda.current_stream(arrs["A"].device).cuda_stream),)
+            fn, what = _lib.lib().xee_series_run_fields_dev, "series_run_fields_dev"
+        else:
+            arrs = {k: None if v is None else np.ascontiguousarray(v, self.np_dtype) for k, v in given.items()}
+            ptr = lambda v: None if v is None else v.ctypes.data_as(C.c_void_p)
+            extra = ()
+            fn, what = _lib.lib().xee_series_run_fields_host, "series_run_fields_host"
+        table = np.zeros((n, len(COLS)))
+        q = _prm(p)
+        _lib.check(fn(self._h, *(ptr(arrs[k]) for k in ("A", "B", "C", "Q", "F", "psi_bc")), C.byref(q),
+                      table.ctypes.data_as(C.c_void_p), *extra), what)
+        return table
+
     def field(self, which):
+        """psi, f, theta, u, w, A, B, C, m2, Q and F of the last run (F fails after a run_fields without F)."""
         nr, nz, n = self.nr, self.nz, self.nsnap
         idx, shape = {"psi": (0, (n, nz, nr)), "f": (1, (n, nz, nr)), "theta": (2, (n, nz - 1, nr - 1)), "u": (3, (n, nz - 1, nr)),
                       "w": (4, (n, nz, nr - 1)), "A": (5, (n, nz, nr)), "B": (6, (n, nz, nr)), "C": (7, (n, nz, nr)),
-                      "m2": (8, (n, nz - 1, nr - 1))}[which]
+                      "m2": (8, (n, nz - 1, nr - 1)), "Q": (9, (n, nz - 1, nr - 1)), "F": (10, (n, nz - 1, nr - 1))}[which]
         out = np.zeros(shape, self.np_dtype)
         _lib.check(_lib.lib().xee_series_get_field(self._h, idx, out.ctypes.data_as(C.c_void_p)), "series_get_field")
         return out
@@ -85,5 +123,19 @@ def run_sharded(nr, nz, Lr, Lz, total, p: SolveParams, world=1, rank=0, device=-
     ts = TimeSeries(nr, nz, Lr, Lz, b - a, device=device, **kw)
     try:
         return a, b, ts.run(W.series_params(b - a, total=total, first=a), p)
+    finally:
+        ts.close()
+
+
+def run_fields_sharded(nr, nz, Lr, Lz, A, B, Cf, Q, p: SolveParams, F=None, psi_bc=None, world=1, rank=0, device=-1, **kw):
+    """The field counterpart of run_sharded: snapshots [a, b) of the caller's whole series (static contiguous chunks of
+    efficiency_map.partition) on this rank.  A, B, C, Q, F, psi_bc are the whole series' arrays as for TimeSeries.run_fields;
+    only rows [a, b) are read.  Returns (a, b, table [b-a, 8])."""
+    from .efficiency_map import partition
+    a, b = partition(int(A.shape[0]), world, rank)
+    ts = TimeSeries(nr, nz, Lr, Lz, b - a, device=device, **kw)
+    try:
+        rows = lambda x: None if x is None else x[a:b]
+        return a, b, ts.run_fields(A[a:b], B[a:b], Cf[a:b], Q[a:b], p, F=rows(F), psi_bc=rows(psi_bc))
     finally:
         ts.close()
