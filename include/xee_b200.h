@@ -300,6 +300,39 @@ int xee_series_run_fields_dev(xee_series* s, const void* A, const void* B, const
 /* which: 0 psi, 1 f, 2 theta_B, 3 u (C grid), 4 w (A grid), 5 A, 6 B, 7 C, 8 m2 (B grid), 9 Q (B grid), 10 F (B grid; fails
  * after a field run without F); all [nsnap][...], plan dtype */
 int xee_series_get_field(xee_series* s, int which, void* host_out);
+/* The legacy efficiency decomposition (src/old-diagnose/diagnose.f90, the chain behind efficiency.txt) of every snapshot, on
+ * the inputs of xee_series_run_fields_* plus chi_bc [nsnap][nz][nr] (only its rim is read, as Dirichlet values of r*chi;
+ * NULL: no boundary-condition chi solves and no exchange conversion).  CYLINDRICAL geometry, the series' density mode.
+ *   tendency 1 (TENDENCY): stage I solves L(B0) psi = f, stage II forms dtheta/dt, the anomaly over testing_dt (finite),
+ *            theta_after and the operator B0 + dB.  tendency 0 (INSTANT): no stage I, dB = 0, theta_after = the background.
+ *   baro     0 BAROTROPIC (operator tag 0: B = 0), 1 BAROCLINIC (tag B0dB: B = B0 + dB), 2 BARO_ALL (both).
+ * Per tag: the chi solves L chi = 0 (chi_bc rim), = f_anomaly, = f_basic; sum(Q eta) of each; the integral-check solve
+ * L psi = f and its w theta integral with theta_after; with chi_bc the exchange conversion, methods 1 and 2 ([D5] of the
+ * re-host: real r, dr, dz, from the working-precision fields).  prm_psi governs the psi solves, prm_chi the chi solves,
+ * tolerances as for run_fields.  Deviations from the legacy driver: every solve starts from its rim with a zero interior
+ * (the legacy driver carries chi from one chi solve into the next and starts psi from the whole psi_bc); the solves use this
+ * library's stop rule, not legacy strategies 1-4; converged answers agree to the tolerance.  A solve whose initial residual
+ * is exactly 0 (zero right-hand side and rim: f_anomaly in INSTANT mode) is not run: its field is its first guess, iters 0.
+ * table [nsnap][XEE_DECOMP_COLS], raw sums (an efficiency.txt line is "value , value / sum_Q"); NaN = not computed (a tag
+ * baro excludes, the chi_bc terms without chi_bc, the tendency terms in INSTANT mode):
+ *   0 sum_Q, 1 sum_dtheta_dt, 2 local heat response sum_dtheta_dt / sum_Q,
+ *   3..9 tag 0 and 10..16 tag B0dB: eta_bc, eta_dB, eta_B0, bndconv, bndconv2, etaQ (decomposition sum), wtheta.
+ * iters, err: HOST [nsnap][XEE_DECOMP_SOLVES] or NULL, in the order psi_before, chi 0_0, chi B0dB_0, chi 0_dB, chi B0dB_dB,
+ * chi 0_B0, chi B0dB_B0, psi_after 0, psi_after B0dB; iters -1 for a solve not run.  _host / _dev as for run_fields. */
+typedef struct xee_decomp_desc { int tendency; double testing_dt; int baro; } xee_decomp_desc;
+#define XEE_DECOMP_COLS 17
+#define XEE_DECOMP_SOLVES 9
+int xee_series_decompose_host(xee_series* s, const xee_decomp_desc* desc, const void* A, const void* B, const void* C,
+                              const void* Q, const void* F, const void* psi_bc, const void* chi_bc,
+                              const xee_solve_params* prm_psi, const xee_solve_params* prm_chi, double* table, int* iters,
+                              int* err);
+int xee_series_decompose_dev(xee_series* s, const xee_decomp_desc* desc, const void* A, const void* B, const void* C,
+                             const void* Q, const void* F, const void* psi_bc, const void* chi_bc,
+                             const xee_solve_params* prm_psi, const xee_solve_params* prm_chi, double* table, int* iters,
+                             int* err, void* stream);
+/* which: 0 dtheta_dt, 1 theta_after (B grid [nsnap][nz-1][nr-1]); 2 + k: the field of solve k in the iters order (O grid
+ * [nsnap][nz][nr]).  Fails for a field the last decomposition did not make.  Plan dtype, HOST out. */
+int xee_series_get_decomp_field(xee_series* s, int which, void* host_out);
 int xee_series_sweep_kernel_stats(xee_series* s, double* ms_total, long long* sweeps, int reset);
 int xee_series_kernel_info(xee_series* s, int* variant, int* sweeps_per_pass, long long* kernel_launches);
 /* Host wall time (ms) the spectral-radius probes of the accelerated methods have taken since the last reset (with one

@@ -101,7 +101,7 @@ struct Map : MapBase, PoolOwner {
     build_abc_kernel<T><<<g, blk, 0, s>>>(A, B, C, ra, rho, a, b, c, nr, nz); XEE_LAUNCH_OK();
     XEE_CHECK(cudaStreamSynchronize(s));
     if (pl->set_abc(a, b, c, (double)dr, (double)dz)) return 1;
-    background_theta_kernel<T><<<1, 256, 0, s>>>(A, B, theta, ra, za, nr, nz, k.g0, k.theta0); XEE_LAUNCH_OK();
+    relative_theta_kernel<T><<<1, 256, 0, s>>>(BasicState<T>{A, B, nr, nz}, theta, ra, za, nr, nz, k.g0, k.theta0); XEE_LAUNCH_OK();
     if (d.adjoint_check) {
       pd.nbatch = 1;
       pl1.reset(new Plan<T>()); pl1->d = pd;
@@ -142,7 +142,7 @@ struct Map : MapBase, PoolOwner {
     if (d.adjoint_check) {
       TraceTimer t2("  map: adjoint chi solve + eta");
       dim3 g1((nr + 127) / 128, nz, 1);
-      rhs_from_B_kernel<T><<<g1, 128, 0, s>>>(B, fchi, nr, nz); XEE_LAUNCH_OK();
+      rhs_from_B_kernel<T><<<g1, 128, 0, s>>>(OGridB<T>{B, nr, nz}, fchi, nr, nz); XEE_LAUNCH_OK();
       XEE_CHECK(cudaMemsetAsync(chi, 0, sizeof(T) * nn, s));
       xee_solve_params p1 = *prm_in;
       T* r1c = nullptr;

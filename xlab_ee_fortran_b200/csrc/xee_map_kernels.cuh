@@ -111,13 +111,14 @@ __global__ void __launch_bounds__(256) map_integrals_kernel(QSrc src, const T* _
                                                             const T* __restrict__ ra, const T* __restrict__ rc,
                                                             const T* __restrict__ za, const T* __restrict__ rho,
                                                             int nr, int nz, double* __restrict__ out /*[n][3]*/,
-                                                            long long theta_stride = 0) {
+                                                            long long theta_stride = 0, long long eta_stride = 0) {
   using R = Rn<T>;
   __shared__ double red[32];
   const int n = blockIdx.x;
   const auto Qn = src.at(n);
   const T* p = psi + (size_t)n * nr * nz;
   theta += (size_t)n * theta_stride;
+  if (eta != nullptr) eta += (size_t)n * eta_stride;
   const int ncell = (nr - 1) * (nz - 1);
   double sq = 0, swt = 0, sqe = 0;
   for (int q = threadIdx.x; q < ncell; q += 256) {
@@ -141,55 +142,93 @@ __global__ void __launch_bounds__(256) map_integrals_kernel(QSrc src, const T* _
   if (threadIdx.x == 0) { out[3 * n + 0] = a; out[3 * n + 1] = b; out[3 * n + 2] = c; }
 }
 
-// Background potential temperature on B from the basic state (testing_dt = 0):
-//   rhoA_A = (A(i,j)+A(i+1,j))/2, rhoB_B = 4-point average of B, rhoB_C(i,j) = (rhoB_B(i-1,j)+rhoB_B(i,j))/2 (i=2..nr-1)
+// rhoB_B(i,j) = 4-point average of an O-grid B on B cell (i, j), 0-based   old-diagnose/diagnose.f90:335-336
+template <class T>
+__device__ __forceinline__ T rhoB_B_of(const T* B, int nr, int i, int j) {
+  using R = Rn<T>;
+  const size_t o = (size_t)j * nr + i;
+  return R::div(R::add(R::add(R::add(B[o], B[o + 1]), B[o + nr]), B[o + nr + 1]), T(4));
+}
+
+// The state relative_theta_kernel integrates, per field set n: at(n) gives rhoB_C(i) on the bottom row (0-based C index
+// i = 1..nr-2) and rhoA_A(i, j) (0-based A index, j = 1..nz-2).
+// BasicState: the basic state of A and B, rhoA_A = (A(i,j)+A(i+1,j))/2, rhoB_C(i,j) = (rhoB_B(i-1,j)+rhoB_B(i,j))/2
+// (old-diagnose/diagnose.f90:329-354, 503-509); the state after a tendency step is another (xee_series.cu).
+template <class T>
+struct BasicState {
+  const T* A; const T* B; int nr, nz;
+  struct At {
+    const T* A; const T* B; int nr;
+    __device__ __forceinline__ T rhoB_C(int i) const {
+      using R = Rn<T>;
+      return R::div(R::add(rhoB_B_of(B, nr, i - 1, 0), rhoB_B_of(B, nr, i, 0)), T(2));
+    }
+    __device__ __forceinline__ T rhoA_A(int i, int j) const {
+      using R = Rn<T>;
+      return R::div(R::add(A[(size_t)j * nr + i], A[(size_t)j * nr + i + 1]), T(2));
+    }
+  };
+  __device__ __forceinline__ At at(int n) const { return At{A + (size_t)n * nr * nz, B + (size_t)n * nr * nz, nr}; }
+};
+
+// Potential temperature on B of a state S (blockIdx.x = field set):
 //   theta = relativeTheta(theta, rhoA_A*theta0/g0, rhoB_C*(-theta0/g0))          old-diagnose/diagnose.f90:893-912
 // One block; thread 0 integrates the bottom row in r, then one thread per column integrates in z.
-template <class T>
-__global__ void background_theta_kernel(const T* __restrict__ A, const T* __restrict__ B, T* __restrict__ theta,
-                                        const T* __restrict__ ra, const T* __restrict__ za, int nr, int nz, T g0,
-                                        T theta0) {
+template <class T, class S>
+__global__ void relative_theta_kernel(S st, T* __restrict__ theta, const T* __restrict__ ra, const T* __restrict__ za,
+                                      int nr, int nz, T g0, T theta0) {
   using R = Rn<T>;
-  A += (size_t)blockIdx.x * nr * nz; B += (size_t)blockIdx.x * nr * nz;      // blockIdx.x = field set
+  const auto sn = st.at(blockIdx.x);
   theta += (size_t)blockIdx.x * (nr - 1) * (nz - 1);
   const T k = R::div(theta0, g0);
-  auto rhoB_B = [&](int i, int j) {  // 0-based B cell
-    const size_t o = (size_t)j * nr + i;
-    return R::div(R::add(R::add(R::add(B[o], B[o + 1]), B[o + nr]), B[o + nr + 1]), T(4));
-  };
   if (threadIdx.x == 0) {
     theta[0] = theta0;
     for (int i = 1; i < nr - 1; ++i) {   // Fortran i = 2..nr-1
       const T dist = R::div(R::sub(ra[i + 1], ra[i - 1]), T(2));
-      const T rhoB_C = R::div(R::add(rhoB_B(i - 1, 0), rhoB_B(i, 0)), T(2));
-      theta[i] = R::add(theta[i - 1], R::mul(dist, R::mul(rhoB_C, -k)));
+      theta[i] = R::add(theta[i - 1], R::mul(dist, R::mul(sn.rhoB_C(i), -k)));
     }
   }
   __syncthreads();
   for (int i = threadIdx.x; i < nr - 1; i += blockDim.x) {
     for (int j = 1; j < nz - 1; ++j) {   // Fortran j = 2..nz-1
       const T dist = R::div(R::sub(za[j + 1], za[j - 1]), T(2));
-      const T rhoA_A = R::div(R::add(A[(size_t)j * nr + i], A[(size_t)j * nr + i + 1]), T(2));
-      theta[(size_t)j * (nr - 1) + i] = R::add(theta[(size_t)(j - 1) * (nr - 1) + i], R::mul(dist, R::mul(rhoA_A, k)));
+      theta[(size_t)j * (nr - 1) + i] = R::add(theta[(size_t)(j - 1) * (nr - 1) + i], R::mul(dist, R::mul(sn.rhoA_A(i, j), k)));
     }
   }
 }
 
-// f_basic = -(4-point average of rhoB_B) on the O interior   old-diagnose/diagnose.f90:524-530
+// Where rhs_from_B_kernel takes the B-cell field b of set n from.  OGridB: rhoB_B of an O-grid B [n][nz][nr] (f_basic);
+// BGridB: a B-cell field [n][nz-1][nr-1] (f_anomaly of the time series' decomposition).
 template <class T>
-__global__ void rhs_from_B_kernel(const T* __restrict__ B, T* __restrict__ f, int nr, int nz) {
+struct OGridB {
+  const T* B; int nr, nz;
+  struct At {
+    const T* B; int nr;
+    __device__ __forceinline__ T operator()(int i, int j) const { return rhoB_B_of(B, nr, i, j); }
+  };
+  __device__ __forceinline__ At at(int n) const { return At{B + (size_t)n * nr * nz, nr}; }
+};
+template <class T>
+struct BGridB {
+  const T* b; int nr, nz;
+  struct At {
+    const T* b; int ld;
+    __device__ __forceinline__ T operator()(int i, int j) const { return b[(size_t)j * ld + i]; }
+  };
+  __device__ __forceinline__ At at(int n) const { return At{b + (size_t)n * (nr - 1) * (nz - 1), nr - 1}; }
+};
+
+// f = -(4-point average of b) on the O interior, 0 on the rim; blockIdx.z = field set   old-diagnose/diagnose.f90:524-530
+template <class T, class BSrc>
+__global__ void rhs_from_B_kernel(BSrc src, T* __restrict__ f, int nr, int nz) {
   using R = Rn<T>;
   const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y;
   if (i >= nr) return;
+  const auto bb = src.at(blockIdx.z);
   T out = T(0);
-  if (i > 0 && i < nr - 1 && j > 0 && j < nz - 1) {
-    auto bb = [&](int ii, int jj) {
-      const size_t o = (size_t)jj * nr + ii;
-      return R::div(R::add(R::add(R::add(B[o], B[o + 1]), B[o + nr]), B[o + nr + 1]), T(4));
-    };
+  if (i > 0 && i < nr - 1 && j > 0 && j < nz - 1)
     out = -R::div(R::add(R::add(R::add(bb(i - 1, j - 1), bb(i - 1, j)), bb(i, j)), bb(i, j - 1)), T(4));
-  }
-  f[(size_t)j * nr + i] = out;
+  f[(size_t)blockIdx.z * nr * nz + (size_t)j * nr + i] = out;
 }
 
 template <class T>

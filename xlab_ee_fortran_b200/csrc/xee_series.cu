@@ -12,7 +12,11 @@
 //   u, w, integrals     old-diagnose/diagnose.f90:915-941, 1117-1127, 1029-1113
 // The builders above are one producer of the fields A, B, C, Q, F and the rim of psi; run_fields takes the same fields from
 // the caller (old-diagnose/diagnose.f90:211-212, 241-242 read them from files).  Both end in the same tail.
+// decompose is a second tail on the field producer's buffers: the legacy efficiency decomposition (old-diagnose/diagnose.f90:
+// 447-841, xee_old_diagnose.cpp) of every snapshot, each of its up to nine solves batched over the snapshots.
 // Deviations from the legacy driver's latent bugs are listed in DESIGN.md section 3.
+#include <limits>
+
 #include "xee_map_kernels.cuh"
 
 namespace xee {
@@ -141,6 +145,138 @@ __global__ void zero_interior_kernel(T* __restrict__ psi, int nr, int nz) {
   psi[(size_t)blockIdx.z * nr * nz + (size_t)j * nr + i] = T(0);
 }
 
+// ---- the legacy efficiency decomposition (old-diagnose/diagnose.f90:468-772), one block or one thread per cell per snapshot
+
+// Stage II tendency on the B cells of snapshot blockIdx.x (:488-493) and its integral integrate_weight_B (:496):
+//   dtheta_dt = J - theta0/g0 (rhoA_A w)avg_z + theta0/g0 (rhoB_C u)avg_r,  J = Q/(Cp exner),
+// rhoA_A = (A(i,j)+A(i+1,j))/2 and rhoB_C = (B(i,j)+B(i,j+1))/2 of the basic state.  out[n] = the weighted sum in double,
+// in the fixed order of map_integrals_kernel.
+template <class T>
+__global__ void __launch_bounds__(256) tendency_kernel(FieldQ<T> src, const T* __restrict__ A, const T* __restrict__ B,
+                                                       const T* __restrict__ u, const T* __restrict__ w, T* __restrict__ dth,
+                                                       const T* __restrict__ ra, const T* __restrict__ za,
+                                                       const T* __restrict__ ex, const T* __restrict__ rho, int nr, int nz,
+                                                       T g0, T theta0, T Cp, double* __restrict__ out) {
+  using R = Rn<T>;
+  __shared__ double red[32];
+  const int n = blockIdx.x;
+  const auto Qn = src.at(n);
+  A += (size_t)n * nr * nz; B += (size_t)n * nr * nz;
+  u += (size_t)n * nr * (nz - 1); w += (size_t)n * (nr - 1) * nz; dth += (size_t)n * (nr - 1) * (nz - 1);
+  const T k = R::div(theta0, g0);
+  const int ncell = (nr - 1) * (nz - 1);
+  double s = 0;
+  for (int q = threadIdx.x; q < ncell; q += 256) {
+    const int i = q % (nr - 1), j = q / (nr - 1);
+    const size_t o = (size_t)j * nr + i, oa = (size_t)j * (nr - 1) + i;
+    const T J = R::div(Qn(i, j, ra, za), R::mul(Cp, ex[j]));
+    const T rA0 = R::div(R::add(A[o], A[o + 1]), T(2)), rA1 = R::div(R::add(A[o + nr], A[o + nr + 1]), T(2));
+    const T rC0 = R::div(R::add(B[o], B[o + nr]), T(2)), rC1 = R::div(R::add(B[o + 1], B[o + nr + 1]), T(2));
+    const T tw = R::div(R::mul(k, R::add(R::mul(rA0, w[oa]), R::mul(rA1, w[oa + nr - 1]))), T(2));
+    const T tu = R::div(R::mul(k, R::add(R::mul(rC0, u[o]), R::mul(rC1, u[o + 1]))), T(2));
+    const T v = R::add(R::sub(J, tw), tu);
+    dth[oa] = v;
+    s += (double)weighted<T>(v, ra, ra, za, rho, i, j);
+  }
+  const double t = block_sum(s, red, threadIdx.x, 8);
+  if (threadIdx.x == 0) out[n] = t;
+}
+
+// The anomaly of a tendency step of length dt on B cell (i, j) of snapshot blockIdx.z (:497-500, 513-514):
+//   b_anom = -g0/theta0 d_dr_B2B(dtheta_dt dt)                 (one-sided in the first and last column, :975-990)
+//   b_op   = b_basic + b_anom / rcuv / rho_                    the b of L(A, B0+dB, C) in set_abc's normalisation
+template <class T>
+__global__ void anomaly_kernel(const T* __restrict__ dth, const T* __restrict__ b_basic, T* __restrict__ b_anom,
+                               T* __restrict__ b_op, const T* __restrict__ ra, const T* __restrict__ rho, int nr, int nz,
+                               T dt, T g0, T theta0) {
+  using R = Rn<T>;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y;
+  if (i >= nr - 1) return;
+  const size_t o = (size_t)blockIdx.z * (nr - 1) * (nz - 1) + (size_t)j * (nr - 1) + i;
+  const T* row = dth + (o - i);
+  const int m = i == 0 ? 0 : -1, p = i == nr - 2 ? 0 : 1;
+  const T d = R::div(R::sub(R::mul(row[i + m], dt), R::mul(row[i + p], dt)), R::sub(ra[i + m], ra[i + p]));
+  const T ba = R::mul(R::div(-g0, theta0), d);
+  const T sb = R::div(R::div(ba, R::div(R::add(ra[i], ra[i + 1]), T(2))), R::div(R::add(rho[j], rho[j + 1]), T(2)));
+  b_anom[o] = ba;
+  b_op[o] = R::add(b_basic[o], sb);
+}
+
+// The state after the tendency step, for relative_theta_kernel (:497-509): rhoB_B + b_anom, its rhoB_C, and
+// rhoA_A + g0/theta0 d_dz_B2A(dtheta_dt dt) (0 on the rows d_dz_B2A does not write, [D3] of xee_old_diagnose.cpp).
+template <class T>
+struct TendencyState {
+  const T* A; const T* B; const T* dth; const T* b_anom; const T* za; T dt, g0, theta0; int nr, nz;
+  struct At {
+    const T* A; const T* B; const T* dth; const T* b_anom; const T* za; T dt, g0, theta0; int nr, nz;
+    __device__ __forceinline__ T rhoB_C(int i) const {
+      using R = Rn<T>;
+      return R::div(R::add(R::add(rhoB_B_of(B, nr, i - 1, 0), b_anom[i - 1]), R::add(rhoB_B_of(B, nr, i, 0), b_anom[i])), T(2));
+    }
+    __device__ __forceinline__ T rhoA_A(int i, int j) const {
+      using R = Rn<T>;
+      const T rA = R::div(R::add(A[(size_t)j * nr + i], A[(size_t)j * nr + i + 1]), T(2));
+      T dA = T(0);
+      if (j <= nz - 3) {
+        const T t1 = R::mul(dth[(size_t)j * (nr - 1) + i], dt), t0 = R::mul(dth[(size_t)(j - 1) * (nr - 1) + i], dt);
+        dA = R::div(R::sub(t1, t0), R::div(R::sub(za[j + 1], za[j - 1]), T(2)));
+      }
+      return R::add(rA, R::mul(R::div(g0, theta0), dA));
+    }
+  };
+  __device__ __forceinline__ At at(int n) const {
+    const size_t nO = (size_t)nr * nz, nB = (size_t)(nr - 1) * (nz - 1);
+    return At{A + n * nO, B + n * nO, dth + n * nB, b_anom + n * nB, za, dt, g0, theta0, nr, nz};
+  }
+};
+
+// One boundary term of cal_exchange_conversion (:1152-1166) at mid-point i+1/2: values at columns i, i+1 of the boundary row
+// (b), and of the rows hi > lo of the one-sided z difference;  (C/rho) ((psi)avg dchi/dz - (chi)avg dpsi/dz) / r^2.
+template <class T>
+__device__ __forceinline__ T exchange_term(T C0, T C1, T rho_b, T p0, T p1, T ph0, T ph1, T pl0, T pl1, T c0, T c1, T ch0, T ch1,
+                                           T cl0, T cl1, T dz2, T r) {
+  using R = Rn<T>;
+  const T dchi = R::div(R::sub(R::sub(R::add(ch0, ch1), cl0), cl1), dz2);
+  const T dpsi = R::div(R::sub(R::sub(R::add(ph0, ph1), pl0), pl1), dz2);
+  const T fac = R::div(R::add(C0, C1), R::mul(T(2), rho_b));
+  const T x = R::sub(R::mul(R::div(R::add(p0, p1), T(2)), dchi), R::mul(R::div(R::add(c0, c1), T(2)), dpsi));
+  return R::div(R::mul(fac, x), R::mul(r, r));
+}
+
+// cal_exchange_conversion (:730-772, :1143-1174, [D5]: real r, dr, dz) of snapshot blockIdx.x, both methods in one pass:
+// chi = chi_bc + chi_dB + chi_B0 (method 1) and chi_dB + chi_B0 (method 2), summed in working precision as the legacy
+// driver adds the fields;  out[n][m] = -sum_i (bnd_top - bnd_bottom) r dr, in double in a fixed order.
+template <class T>
+__global__ void __launch_bounds__(256) exchange_conversion_kernel(const T* __restrict__ psi, const T* __restrict__ chi_bc,
+                                                                  const T* __restrict__ chi_dB, const T* __restrict__ chi_B0,
+                                                                  const T* __restrict__ C, const T* __restrict__ ra,
+                                                                  const T* __restrict__ za, const T* __restrict__ rho,
+                                                                  int nr, int nz, double* __restrict__ out /*[n][2]*/) {
+  using R = Rn<T>;
+  __shared__ double red[32];
+  const size_t off = (size_t)blockIdx.x * nr * nz;
+  psi += off; chi_bc += off; chi_dB += off; chi_B0 += off; C += off;
+  const T dz2 = R::mul(T(2), R::sub(za[1], za[0])), ddr = R::sub(ra[1], ra[0]);
+  const size_t top = (size_t)(nz - 1) * nr, below = (size_t)(nz - 2) * nr;
+  double s[2] = {0, 0};
+  for (int i = threadIdx.x; i < nr - 1; i += 256) {
+    const T r = R::div(R::add(ra[i], ra[i + 1]), T(2));
+#pragma unroll
+    for (int m = 0; m < 2; ++m) {
+      auto chi = [&](size_t o) { const T c = R::add(chi_dB[o], chi_B0[o]); return m == 0 ? R::add(R::add(chi_bc[o], chi_dB[o]), chi_B0[o]) : c; };
+      const size_t b0 = i, b1 = (size_t)nr + i, t1 = top + i, t0 = below + i;
+      const T bot = exchange_term(C[b0], C[b0 + 1], rho[0], psi[b0], psi[b0 + 1], psi[b1], psi[b1 + 1], psi[b0], psi[b0 + 1],
+                                  chi(b0), chi(b0 + 1), chi(b1), chi(b1 + 1), chi(b0), chi(b0 + 1), dz2, r);
+      const T tp = exchange_term(C[t1], C[t1 + 1], rho[nz - 1], psi[t1], psi[t1 + 1], psi[t1], psi[t1 + 1], psi[t0], psi[t0 + 1],
+                                 chi(t1), chi(t1 + 1), chi(t1), chi(t1 + 1), chi(t0), chi(t0 + 1), dz2, r);
+      s[m] -= (double)R::mul(R::mul(R::sub(tp, bot), r), ddr);
+    }
+  }
+  const double a = block_sum(s[0], red, threadIdx.x, 8);
+  const double b = block_sum(s[1], red, threadIdx.x, 8);
+  if (threadIdx.x == 0) { out[2 * blockIdx.x] = a; out[2 * blockIdx.x + 1] = b; }
+}
+
 template <class T>
 __global__ void __launch_bounds__(256) absmax_kernel(const T* __restrict__ x, long long count, double* __restrict__ out) {
   __shared__ double red[32];
@@ -161,6 +297,10 @@ struct SeriesBase {
   virtual int run_fields(const void* A, const void* B, const void* C, const void* Q, const void* F, const void* psi_bc,
                          bool on_host, const xee_solve_params* prm, double* table_host, cudaStream_t stream) = 0;
   virtual int get_field(int which, void* host_out) = 0;
+  virtual int decompose(const xee_decomp_desc* dd, const void* A, const void* B, const void* C, const void* Q, const void* F,
+                        const void* psi_bc, const void* chi_bc, bool on_host, const xee_solve_params* prm_psi,
+                        const xee_solve_params* prm_chi, double* table, int* iters, int* err, cudaStream_t stream) = 0;
+  virtual int get_decomp_field(int which, void* host_out) = 0;
   virtual PlanBase* plan() = 0;
 };
 
@@ -174,6 +314,14 @@ struct Series : SeriesBase, PoolOwner {
     *ex = nullptr, *rho = nullptr;
   Snap* snaps = nullptr; Heat* heat = nullptr; double* integ = nullptr; double* mx = nullptr;
   bool has_F = false;   // F holds the last run's momentum forcing (a field run without F has none)
+  // The decomposition's buffers, allocated by its first call: dfield[2 + slot] = the field of solve slot (XEE_DECOMP_SOLVES
+  // order), dfield[0] = dtheta_dt, dfield[1] = theta_after; dmade[w]: the last decomposition made dfield[w].
+  static constexpr int kDecompFields = 2 + XEE_DECOMP_SOLVES;
+  T* dfield[kDecompFields] = {};
+  bool dmade[kDecompFields] = {};
+  T *eta = nullptr, *b_anom = nullptr, *b_op = nullptr, *zero = nullptr, *f_basic = nullptr, *f_anom = nullptr,
+    *chi_rim = nullptr, *r0v = nullptr;
+  double *dsum = nullptr /*[slot][n][3]*/, *sdt = nullptr /*[n]*/, *exch = nullptr /*[tag][n][2]*/;
   size_t nn = 0;
   T dr = 0, dz = 0;
   PhysK<T> k;
@@ -249,19 +397,30 @@ struct Series : SeriesBase, PoolOwner {
   // momentum term; psi_bc == nullptr: a zero rim.  Only the rim of psi_bc is read; the first guess is 0 inside.
   int run_fields(const void* A_in, const void* B_in, const void* C_in, const void* Q_in, const void* F_in, const void* bc_in,
                  bool on_host, const xee_solve_params* prm, double* table, cudaStream_t in) override {
-    if (!A_in || !B_in || !C_in || !Q_in) return fail("xee_series_run_fields: A, B, C and Q must not be NULL");
     TraceTimer tt("series run_fields (total)");
+    if (load_fields("xee_series_run_fields", A_in, B_in, C_in, Q_in, F_in, bc_in,
+                    nullptr, nullptr, on_host, in))
+      return 1;
+    // Probe every operator: no smoothness rule for arbitrary fields has been calibrated.
+    return tail(0, prm, table);
+  }
+
+  // Field producer: copies the caller's A, B, C, Q, F and the rim of psi_bc (and of chi_bc into chi_rim) into the series.
+  // `who` names the entry point in messages (its _dev form for device arrays).
+  int load_fields(const char* who, const void* A_in, const void* B_in, const void* C_in, const void* Q_in, const void* F_in,
+                  const void* bc_in, const void* chi_in, T* chi_rim, bool on_host, cudaStream_t in) {
+    if (!A_in || !B_in || !C_in || !Q_in) return fail((std::string(who) + ": A, B, C and Q must not be NULL").c_str());
     const int nr = d.nr, nz = d.nz, nb = d.nsnap;
     cudaStream_t s = pl->own_stream;
     if (on_host) in = s;
     else {   // device arrays must live on the series' device: a copy from another device would depend on peer access
-      for (const void* p : {A_in, B_in, C_in, Q_in, F_in, bc_in}) {
+      for (const void* p : {A_in, B_in, C_in, Q_in, F_in, bc_in, chi_in}) {
         if (!p) continue;
         cudaPointerAttributes pa{};
         if (cudaPointerGetAttributes(&pa, p) != cudaSuccess || (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) ||
             pa.device != d.device) {
           cudaGetLastError();
-          return fail("xee_series_run_fields_dev: every array must be device memory on the series' device");
+          return fail((std::string(who) + "_dev: every array must be device memory on the series' device").c_str());
         }
       }
     }
@@ -275,29 +434,43 @@ struct Series : SeriesBase, PoolOwner {
     if (has_F) XEE_CHECK(cudaMemcpyAsync(F, F_in, bB, kind, in));
     if (bc_in) XEE_CHECK(cudaMemcpyAsync(psi, bc_in, bO, kind, in));
     else XEE_CHECK(cudaMemsetAsync(psi, 0, bO, in));
+    if (chi_in) XEE_CHECK(cudaMemcpyAsync(chi_rim, chi_in, bO, kind, in));
     XEE_CHECK(cudaStreamSynchronize(in));   // the caller's arrays are consumed; the rest runs on the series' own stream
     if (bc_in) { zero_interior_kernel<T><<<dim3((nr + 127) / 128, nz, nb), 128, 0, s>>>(psi, nr, nz); XEE_LAUNCH_OK(); }
-    // Probe every operator: no smoothness rule for arbitrary fields has been calibrated.
-    return tail(0, prm, table);
+    if (chi_in) { zero_interior_kernel<T><<<dim3((nr + 127) / 128, nz, nb), 128, 0, s>>>(chi_rim, nr, nz); XEE_LAUNCH_OK(); }
+    return 0;
   }
 
   // Shared tail: operators, theta, right-hand sides, the batched solve and the table from the fields of the producer.
-  // table row: iters, r1, err, sum_Q, ke_gen, efficiency, max|w|, max|u|
   int tail(int rho_subsample, const xee_solve_params* prm_in, double* table) {
+    if (prepare(true)) return 1;
+    pl->rho_subsample = rho_subsample;
+    return solve_psi(prm_in, table);
+  }
+  // a, b, c, (with set_op) the operator L(A, B, C) of every snapshot, the background theta, the forcing f and m2
+  int prepare(bool set_op) {
     const int nr = d.nr, nz = d.nz, nb = d.nsnap;
     cudaStream_t s = pl->own_stream;
     dim3 gO((nr + 127) / 128, nz, nb);
     dim3 blk(64, 4), g2((nr + 63) / 64, (nz + 3) / 4, nb);
     build_abc_kernel<T><<<g2, blk, 0, s>>>(A, B, C, ra, rho, a, b, c, nr, nz); XEE_LAUNCH_OK();
     XEE_CHECK(cudaStreamSynchronize(s));
-    if (pl->set_abc(a, b, c, (double)dr, (double)dz)) return 1;
+    if (set_op && pl->set_abc(a, b, c, (double)dr, (double)dz)) return 1;
     const FieldQ<T> qsrc{Q, nr, nz};
-    background_theta_kernel<T><<<nb, 256, 0, s>>>(A, B, theta, ra, za, nr, nz, k.g0, k.theta0); XEE_LAUNCH_OK();
+    relative_theta_kernel<T><<<nb, 256, 0, s>>>(BasicState<T>{A, B, nr, nz}, theta, ra, za, nr, nz, k.g0, k.theta0); XEE_LAUNCH_OK();
     heating_rhs_kernel<T><<<heating_rhs_grid(nr, nz, nb), dim3(kHeatBX, kHeatBY), 0, s>>>(qsrc, f, ra, za, ex, nr, nz, k.g0, k.theta0, k.Cp); XEE_LAUNCH_OK();
     dim3 gm((nz - 1 + 63) / 64, nb);
     series_m2_kernel<T><<<gm, 64, 0, s>>>(C, m2, ra, ra, nr, nz, nb); XEE_LAUNCH_OK();
     if (has_F) { series_mom_rhs_kernel<T><<<gO, 128, 0, s>>>(F, m2, f, ra, za, nr, nz); XEE_LAUNCH_OK(); }
-    pl->rho_subsample = rho_subsample;
+    return 0;
+  }
+  // The batched solve L psi = f on the current operator, u, w and the table.
+  // table row: iters, r1, err, sum_Q, ke_gen, efficiency, max|w|, max|u|
+  int solve_psi(const xee_solve_params* prm_in, double* table) {
+    const int nr = d.nr, nz = d.nz, nb = d.nsnap;
+    cudaStream_t s = pl->own_stream;
+    dim3 gO((nr + 127) / 128, nz, nb);
+    const FieldQ<T> qsrc{Q, nr, nz};
     xee_solve_params prm = *prm_in;
     if (d.r1_rel_rms_f > 0) {
       // tolerance relative to the INITIAL residual L psi0 - f: with the pumping boundary condition the boundary data,
@@ -324,6 +497,181 @@ struct Series : SeriesBase, PoolOwner {
       r[0] = iters[n]; r[1] = r1o[n]; r[2] = err[n]; r[3] = hi[3 * n]; r[4] = hi[3 * n + 1] * gth; r[5] = r[4] / r[3];
       r[6] = hm[n]; r[7] = hm[nb + n];
     }
+    return 0;
+  }
+  // ---- The legacy efficiency decomposition (old-diagnose/diagnose.f90:447-841) on the field producer's snapshots.
+  int decomp_alloc() {   // once per series, on the first decomposition
+    if (zero) return 0;
+    const int nr = d.nr, nz = d.nz, nb = d.nsnap;
+    const size_t bO = sizeof(T) * nn * nb, bB = sizeof(T) * (size_t)(nr - 1) * (nz - 1) * nb;
+    XEE_CHECK(own(&dfield[0], bB)); XEE_CHECK(own(&dfield[1], bB));
+    for (int w = 2; w < kDecompFields; ++w) XEE_CHECK(own(&dfield[w], bO));
+    XEE_CHECK(own(&eta, sizeof(T) * (size_t)(nr - 1) * nz * nb));
+    XEE_CHECK(own(&b_anom, bB)); XEE_CHECK(own(&b_op, bB));
+    XEE_CHECK(own(&f_basic, bO)); XEE_CHECK(own(&f_anom, bO)); XEE_CHECK(own(&chi_rim, bO));
+    XEE_CHECK(own(&r0v, sizeof(T) * nb));
+    XEE_CHECK(own(&dsum, sizeof(double) * 3 * nb * XEE_DECOMP_SOLVES)); XEE_CHECK(own(&sdt, sizeof(double) * nb));
+    XEE_CHECK(own(&exch, sizeof(double) * 4 * nb));
+    T* z = nullptr;
+    XEE_CHECK(own(&z, bO));
+    XEE_CHECK(cudaMemsetAsync(z, 0, bO, pl->own_stream));
+    zero = z;   // set last: a call that failed above allocates again
+    return 0;
+  }
+
+  // The batched solve of decomposition slot `slot` on the current operator, from the first guess in x (the Dirichlet rim,
+  // 0 inside); tolerance as in the tail, r1_rel_rms_f * rms of the initial residual.  A snapshot whose initial residual is
+  // exactly 0 (a right-hand side and rim of zeros) keeps its first guess with iters 0 and err 0: its tolerance would be 0,
+  // which disables the stop rule.  When no snapshot has a residual nothing is solved.
+  int solve_slot(T* x, const T* rhs, const xee_solve_params* prm_in, int slot, std::vector<int>& its, std::vector<int>& errs) {
+    const int nr = d.nr, nz = d.nz, nb = d.nsnap;
+    cudaStream_t s = pl->own_stream;
+    if (pl->apply(x, pl->x1, s)) return 1;
+    rms_diff_interior_kernel<T><<<nb, 256, 0, s>>>(pl->x1, rhs, nr, nz, T(1), r0v); XEE_LAUNCH_OK();
+    std::vector<T> h0(nb);
+    XEE_CHECK(cudaMemcpyAsync(h0.data(), r0v, sizeof(T) * nb, cudaMemcpyDeviceToHost, s));
+    XEE_CHECK(cudaStreamSynchronize(s));
+    std::vector<int> it(nb, 0), er(nb, 0);
+    std::vector<double> r1o(nb), r2o(nb);
+    bool any = false;
+    for (int n = 0; n < nb; ++n) any |= !(h0[n] == T(0));
+    if (any) {
+      xee_solve_params prm = *prm_in;
+      if (d.r1_rel_rms_f > 0) {
+        rms_diff_interior_kernel<T><<<nb, 256, 0, s>>>(pl->x1, rhs, nr, nz, (T)d.r1_rel_rms_f, r1v); XEE_LAUNCH_OK();
+        prm.r1 = 1.0; prm.r1_per_solve = r1v;
+      }
+      if (pl->solve(x, rhs, &prm, it.data(), r1o.data(), r2o.data(), er.data(), s, false, nullptr, 0)) return 1;
+      for (int n = 0; n < nb; ++n)
+        if (h0[n] == T(0)) {
+          zero_interior_kernel<T><<<dim3((nr + 127) / 128, nz, 1), 128, 0, s>>>(x + (size_t)n * nn, nr, nz); XEE_LAUNCH_OK();
+          it[n] = 0; er[n] = 0;
+        }
+    }
+    for (int n = 0; n < nb; ++n) { its[(size_t)n * XEE_DECOMP_SOLVES + slot] = it[n]; errs[(size_t)n * XEE_DECOMP_SOLVES + slot] = er[n]; }
+    return 0;
+  }
+
+  // Stage I (TENDENCY): the tail's solve L(B0) psi = f.  Stage II: the tendency, the anomaly, theta_after, f_anomaly.
+  // Then per operator L(A, B=0, C) (tag 0) and L(A, B=B0+dB, C) (tag B0dB): the chi solves, eta and sum(Q eta), the
+  // integral-check psi solve and its w theta integral, and with chi_bc the exchange conversion.  Every solve starts from a
+  // zero interior; each operator is set (and probed) once.
+  int decompose(const xee_decomp_desc* dd, const void* A_in, const void* B_in, const void* C_in, const void* Q_in,
+                const void* F_in, const void* bc_in, const void* chi_in, bool on_host, const xee_solve_params* prm_psi,
+                const xee_solve_params* prm_chi, double* table, int* iters_out, int* err_out, cudaStream_t in) override {
+    if (!dd || !prm_psi || !prm_chi || !table) return fail("xee_series_decompose: desc, prm_psi, prm_chi and table must not be NULL");
+    if (dd->baro < 0 || dd->baro > 2) return fail("xee_series_decompose: baro must be 0 (BAROTROPIC), 1 (BAROCLINIC) or 2 (BARO_ALL)");
+    const bool tend = dd->tendency != 0;
+    if (tend && !std::isfinite(dd->testing_dt)) return fail("xee_series_decompose: testing_dt must be finite in TENDENCY mode");
+    TraceTimer tt("series decompose (total)");
+    if (decomp_alloc()) return 1;
+    for (bool& m : dmade) m = false;
+    if (load_fields("xee_series_decompose", A_in, B_in, C_in, Q_in, F_in, bc_in, chi_in, chi_rim, on_host, in)) return 1;
+    const int nr = d.nr, nz = d.nz, nb = d.nsnap;
+    const size_t nB = (size_t)(nr - 1) * (nz - 1), bO = sizeof(T) * nn * nb, bB = sizeof(T) * nB * nb;
+    cudaStream_t s = pl->own_stream;
+    const bool bc = chi_in != nullptr, use[2] = {dd->baro != 1, dd->baro != 0};
+    const T dt = (T)dd->testing_dt;
+    std::vector<int> its((size_t)nb * XEE_DECOMP_SOLVES, -1), errs(its.size(), 0);
+    if (prepare(tend)) return 1;
+    pl->rho_subsample = 0;   // every operator probed, as in run_fields
+    for (int t = 0; t < 2; ++t)   // first guesses of the integral checks: the rim of psi_bc, 0 inside
+      if (use[t]) XEE_CHECK(cudaMemcpyAsync(dfield[9 + t], psi, bO, cudaMemcpyDeviceToDevice, s));
+    const FieldQ<T> qsrc{Q, nr, nz};
+    const dim3 gO((nr + 127) / 128, nz, nb), gB((nr - 1 + 127) / 128, nz - 1, nb);
+    if (tend) {
+      std::vector<double> t8((size_t)nb * XEE_MAP_COLS);
+      {
+        TraceTimer t1("  decompose: stage I solve");
+        if (solve_psi(prm_psi, t8.data())) return 1;
+      }
+      TraceTimer t2("  decompose: stage II");
+      for (int n = 0; n < nb; ++n) { its[(size_t)n * XEE_DECOMP_SOLVES] = (int)t8[(size_t)n * XEE_MAP_COLS]; errs[(size_t)n * XEE_DECOMP_SOLVES] = (int)t8[(size_t)n * XEE_MAP_COLS + 2]; }
+      XEE_CHECK(cudaMemcpyAsync(dfield[2], psi, bO, cudaMemcpyDeviceToDevice, s));
+      dmade[2] = true;
+      tendency_kernel<T><<<nb, 256, 0, s>>>(qsrc, A, B, u, w, dfield[0], ra, za, ex, rho, nr, nz, k.g0, k.theta0, k.Cp, sdt); XEE_LAUNCH_OK();
+      anomaly_kernel<T><<<gB, 128, 0, s>>>(dfield[0], b, b_anom, b_op, ra, rho, nr, nz, dt, k.g0, k.theta0); XEE_LAUNCH_OK();
+      relative_theta_kernel<T><<<nb, 256, 0, s>>>(TendencyState<T>{A, B, dfield[0], b_anom, za, dt, k.g0, k.theta0, nr, nz}, dfield[1],
+                                                  ra, za, nr, nz, k.g0, k.theta0); XEE_LAUNCH_OK();
+      rhs_from_B_kernel<T><<<gO, 128, 0, s>>>(BGridB<T>{b_anom, nr, nz}, f_anom, nr, nz); XEE_LAUNCH_OK();
+      dmade[0] = true;
+    } else {   // INSTANT ([D4] of xee_old_diagnose.cpp): b_anom = 0, theta_after = the background state
+      XEE_CHECK(cudaMemcpyAsync(dfield[1], theta, bB, cudaMemcpyDeviceToDevice, s));
+      XEE_CHECK(cudaMemsetAsync(f_anom, 0, bO, s));
+    }
+    dmade[1] = true;
+    rhs_from_B_kernel<T><<<gO, 128, 0, s>>>(OGridB<T>{B, nr, nz}, f_basic, nr, nz); XEE_LAUNCH_OK();
+    const T* bop[2] = {zero, tend ? b_op : b};
+    const T* chi_rhs[3] = {zero, f_anom, f_basic};
+    const dim3 ge((nr - 1 + 127) / 128, nz, nb);
+    for (int t = 0; t < 2; ++t) {
+      if (!use[t]) continue;
+      XEE_CHECK(cudaStreamSynchronize(s));
+      {
+        TraceTimer t3("  decompose: operator set");
+        if (pl->set_abc(a, bop[t], c, (double)dr, (double)dz)) return 1;
+      }
+      {
+        TraceTimer t4("  decompose: chi solves");
+        for (int kind = bc ? 0 : 1; kind < 3; ++kind) {   // chi with the chi_bc rim and rhs 0, then -dB, then -B0
+          const int slot = 1 + 2 * kind + t;
+          T* x = dfield[2 + slot];
+          if (kind == 0) XEE_CHECK(cudaMemcpyAsync(x, chi_rim, bO, cudaMemcpyDeviceToDevice, s));
+          else XEE_CHECK(cudaMemsetAsync(x, 0, bO, s));
+          if (solve_slot(x, chi_rhs[kind], prm_chi, slot, its, errs)) return 1;
+          eta_kernel<T><<<ge, 128, 0, s>>>(x, eta, ra, ra, rho, ex, nr, nz, k.g0, k.Cp, k.theta0); XEE_LAUNCH_OK();
+          map_integrals_kernel<T><<<nb, 256, 0, s>>>(qsrc, x, dfield[1], eta, ra, ra, za, rho, nr, nz, dsum + (size_t)3 * nb * slot,
+                                                     (long long)nB, (long long)(nr - 1) * nz);
+          XEE_LAUNCH_OK();
+          dmade[2 + slot] = true;
+        }
+      }
+      TraceTimer t5("  decompose: check solve");
+      const int slot = 7 + t;   // the integral check L psi = f with theta_after
+      T* x = dfield[2 + slot];
+      if (solve_slot(x, f, prm_psi, slot, its, errs)) return 1;
+      map_integrals_kernel<T><<<nb, 256, 0, s>>>(qsrc, x, dfield[1], nullptr, ra, ra, za, rho, nr, nz, dsum + (size_t)3 * nb * slot, (long long)nB);
+      XEE_LAUNCH_OK();
+      dmade[2 + slot] = true;
+      if (bc) {
+        exchange_conversion_kernel<T><<<nb, 256, 0, s>>>(x, dfield[3 + t], dfield[5 + t], dfield[7 + t], C, ra, za, rho, nr, nz, exch + (size_t)2 * nb * t);
+        XEE_LAUNCH_OK();
+      }
+    }
+    std::vector<double> hs((size_t)3 * nb * XEE_DECOMP_SOLVES), ht(nb), hx((size_t)4 * nb);
+    XEE_CHECK(cudaMemcpyAsync(hs.data(), dsum, sizeof(double) * hs.size(), cudaMemcpyDeviceToHost, s));
+    if (tend) XEE_CHECK(cudaMemcpyAsync(ht.data(), sdt, sizeof(double) * nb, cudaMemcpyDeviceToHost, s));
+    if (bc) XEE_CHECK(cudaMemcpyAsync(hx.data(), exch, sizeof(double) * hx.size(), cudaMemcpyDeviceToHost, s));
+    XEE_CHECK(cudaStreamSynchronize(s));
+    const double gth = (double)k.g0 / (double)k.theta0, nan = std::numeric_limits<double>::quiet_NaN();
+    auto sums = [&](int slot, int n) { return &hs[((size_t)slot * nb + n) * 3]; };
+    for (int n = 0; n < nb; ++n) {
+      double* r = table + (size_t)n * XEE_DECOMP_COLS;
+      r[0] = sums(use[0] ? 7 : 8, n)[0];
+      r[1] = tend ? ht[n] : nan;
+      r[2] = r[1] / r[0];
+      for (int t = 0; t < 2; ++t) {
+        double* q = r + 3 + 7 * t;
+        if (!use[t]) { for (int m = 0; m < 7; ++m) q[m] = nan; continue; }
+        q[0] = bc ? sums(1 + t, n)[2] : nan;
+        q[1] = sums(3 + t, n)[2];
+        q[2] = sums(5 + t, n)[2];
+        q[3] = bc ? hx[((size_t)t * nb + n) * 2] : nan;
+        q[4] = bc ? hx[((size_t)t * nb + n) * 2 + 1] : nan;
+        q[5] = ((bc ? q[0] : 0.0) + q[1]) + q[2];   // the decomposition sum, in the legacy driver's order
+        if (bc) q[5] += q[3];
+        q[6] = sums(7 + t, n)[1] * gth;
+      }
+    }
+    if (iters_out) std::copy(its.begin(), its.end(), iters_out);
+    if (err_out) std::copy(errs.begin(), errs.end(), err_out);
+    return 0;
+  }
+  int get_decomp_field(int which, void* out) override {
+    if (which < 0 || which >= kDecompFields) return fail("xee_series_get_decomp_field: unknown field");
+    if (!dmade[which]) return fail("xee_series_get_decomp_field: the last decomposition did not make this field");
+    const size_t bytes = sizeof(T) * (which < 2 ? (size_t)(d.nr - 1) * (d.nz - 1) : nn) * d.nsnap;
+    XEE_CHECK(cudaMemcpy(out, dfield[which], bytes, cudaMemcpyDeviceToHost));
     return 0;
   }
   int get_field(int which, void* out) override {
@@ -383,6 +731,19 @@ int xee_series_run_fields_dev(xee_series* m, const void* A, const void* B, const
   return m->impl->run_fields(A, B, C, Q, F, psi_bc, false, prm, table, (cudaStream_t)stream);
 }
 int xee_series_get_field(xee_series* m, int which, void* out) { DeviceGuard g(m->impl->device()); return m->impl->get_field(which, out); }
+int xee_series_decompose_host(xee_series* m, const xee_decomp_desc* dd, const void* A, const void* B, const void* C, const void* Q,
+                              const void* F, const void* psi_bc, const void* chi_bc, const xee_solve_params* prm_psi,
+                              const xee_solve_params* prm_chi, double* table, int* iters, int* err) {
+  DeviceGuard g(m->impl->device());
+  return m->impl->decompose(dd, A, B, C, Q, F, psi_bc, chi_bc, true, prm_psi, prm_chi, table, iters, err, nullptr);
+}
+int xee_series_decompose_dev(xee_series* m, const xee_decomp_desc* dd, const void* A, const void* B, const void* C, const void* Q,
+                             const void* F, const void* psi_bc, const void* chi_bc, const xee_solve_params* prm_psi,
+                             const xee_solve_params* prm_chi, double* table, int* iters, int* err, void* stream) {
+  DeviceGuard g(m->impl->device());
+  return m->impl->decompose(dd, A, B, C, Q, F, psi_bc, chi_bc, false, prm_psi, prm_chi, table, iters, err, (cudaStream_t)stream);
+}
+int xee_series_get_decomp_field(xee_series* m, int which, void* out) { DeviceGuard g(m->impl->device()); return m->impl->get_decomp_field(which, out); }
 int xee_series_sweep_kernel_stats(xee_series* m, double* ms, long long* launches, int reset) { return m->impl->plan()->kernel_stats(ms, launches, reset); }
 int xee_series_probe_stats(xee_series* m, double* ms, int reset) {
   PlanBase* p = m->impl->plan();
